@@ -318,6 +318,7 @@ class Engine:
             L.fq_comm_destroy.restype = None
             L.fq_allreduce_stats.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
             L.fq_merge_stats.argtypes = [C.c_void_p, C.c_void_p]
+            L.fq_kmer_end_pass_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
             L.fq_last_allreduce_ms.argtypes = [C.c_void_p]
             L.fq_last_allreduce_ms.restype = C.c_float
             L.fq_device_outputs.argtypes = [C.c_void_p, C.POINTER(C.c_void_p * NUM_STREAM)]

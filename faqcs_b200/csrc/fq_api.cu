@@ -122,12 +122,15 @@ struct fq_ctx {
         uint64_t total_reads = 0;                  // TOTAL_NUMBER
         std::vector<fq_rarefaction> samples;       // finished points
         std::map<uint64_t, uint64_t> freq;         // kmer_frequency_histogram
-        // current pass
-        uint32_t pass_calls = 0;                   // trim() calls of this pass so far
-        uint32_t pass_counted = 0;                 // calls [0, pass_counted) fed the table
-        std::vector<std::pair<uint32_t, uint64_t>> pass_points;   // (call, TOTAL_NUMBER): distinct / total filled in at the end of the pass
+        // current pass: what this context's batches covered (call numbers follow from first_record_index)
+        std::vector<uint64_t> call_reads;          // [kKmerMaxCalls] reads of each call run here
+        std::vector<uint64_t> call_runs;           // [kKmerMaxCalls] times each call was run here
+        uint64_t calls_beyond = 0;                 // calls >= kKmerMaxCalls run here (the curve is complete by then)
+        uint64_t call_end = 0;                     // 1 + the highest call run here
+        uint64_t pass_reads = 0;
         unsigned long long cap = 0, occupied_bound = 0;
         DevBuf d_slots, d_call_total, d_call_distinct, d_small, d_big, d_scalars;
+        DevBuf d_send, d_recv;                     // end of a sharded pass: entries grouped by owner, one received group
         std::vector<uint64_t> flat;                // fq_kmer_view::frequency
     } kmer;
 
@@ -390,13 +393,18 @@ KmerTable kmer_table_of(fq_ctx::Kmer &K)
     return KmerTable{K.d_slots.as<KmerSlot>(), K.cap - 1};
 }
 
-// (Re)allocate the table for at least `slots` slots (a power of two), keeping its entries.
-fq_status kmer_resize(fq_ctx *ctx, unsigned long long slots)
+// (Re)allocate the table for at least `slots` slots (a power of two), keeping its entries (or, with keep == false, empty).
+fq_status kmer_resize(fq_ctx *ctx, unsigned long long slots, bool keep = true)
 {
     fq_ctx::Kmer &K = ctx->kmer;
     unsigned long long cap = 1ull << 20;
     while (cap < slots) cap <<= 1;
     if (cap <= K.cap) return FQ_OK;
+    if (!keep) {
+        CK(cudaStreamSynchronize(ctx->stream));
+        K.d_slots.release();
+        K.cap = 0;
+    }
     DevBuf ns;
     CK(ns.ensure(cap * sizeof(KmerSlot)));
     KmerTable to{ns.as<KmerSlot>(), cap - 1};
@@ -410,34 +418,70 @@ fq_status kmer_resize(fq_ctx *ctx, unsigned long long slots)
     return FQ_OK;
 }
 
-// One batch: which trim() calls of the reference it spans, which of them still feed the table, where curve points fall
-// (trim.cpp:157-185), then the counting kernel.
+// The reference's sequence of trim() calls in one pass (trim.cpp:157-185), from the state at the start of the pass:
+// reads(c) is the number of reads of call c.  A call feeds the table while the curve is collected (trim.cpp:260-262); at
+// its end a point is taken if the running read count crossed another multiple of split_size.  The call that follows the
+// last point still feeds the table: `collecting` is cleared only after the point is pushed.
+struct KmerWalk {
+    std::vector<std::pair<uint32_t, uint64_t>> points;     // (call, TOTAL_NUMBER)
+    uint32_t counted = 0;                                  // calls [0, counted) feed the table
+    bool collecting = false;                               // still collecting after the last call walked
+};
+
+template <class Reads>
+fq_status kmer_walk(fq_ctx *ctx, const fq_ctx::Kmer &K, uint64_t n_calls, Reads reads, KmerWalk *w)
+{
+    w->points.clear();
+    w->counted = 0;
+    w->collecting = K.collecting;
+    uint64_t total = K.total_reads;
+    for (uint64_t call = 0; call < n_calls && w->collecting; ++call) {
+        if (call >= kKmerMaxCalls) return fail(ctx, FQ_ERR_ARG, "k-mer rarefaction: more than 65536 trim() batches while the curve is collected");
+        w->counted = (uint32_t)call + 1;
+        total += reads((uint32_t)call);
+        const uint64_t index = total / K.split_size;
+        const uint64_t n_points = K.samples.size() + w->points.size();
+        if (index > n_points && n_points < K.num_subsample) w->points.push_back(std::make_pair((uint32_t)call, total));
+        if (n_points >= K.num_subsample) w->collecting = false;
+    }
+    return FQ_OK;
+}
+
+// One batch: which trim() calls of the reference it spans (from its position in the input, so batches may run in any order
+// and on any context of a sharded table), which of them still feed the table, then the counting kernel.
 fq_status kmer_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint32_t n, int n_mates, uint32_t max_len, uint64_t first_record_index, int is_final, bool trimmed)
 {
     fq_ctx::Kmer &K = ctx->kmer;
     if ((first_record_index % FQ_REF_BATCH) != 0 || (!is_final && (n % FQ_REF_BATCH) != 0))
         return fail(ctx, FQ_ERR_ARG, "k-mer rarefaction needs batches that start on a 32768-record boundary and hold a multiple of 32768 records");
-    const uint32_t first_call = K.pass_calls;
-    uint64_t counted_reads = 0;
-    for (uint32_t b0 = 0; b0 < n; b0 += FQ_REF_BATCH) {
-        const uint32_t reads = std::min<uint32_t>(FQ_REF_BATCH, n - b0);
-        for (int m = 0; m < n_mates; ++m) {
-            const uint32_t call = K.pass_calls++;
-            if (K.collecting) {                              // this call's reads go through update_kmer (trim.cpp:260-262)
-                if (call >= kKmerMaxCalls) return fail(ctx, FQ_ERR_ARG, "k-mer rarefaction: more than 65536 trim() batches while the curve is collected");
-                K.pass_counted = call + 1;
-                counted_reads += reads;
-            }
-            K.total_reads += reads;
-            if (K.collecting) {                              // end of trim(): trim.cpp:157-185
-                const uint64_t index = K.total_reads / K.split_size;
-                const uint64_t n_points = K.samples.size() + K.pass_points.size();
-                if (index > n_points && n_points < K.num_subsample) K.pass_points.push_back(std::make_pair(call, K.total_reads));
-                if (n_points >= K.num_subsample) K.collecting = false;
-            }
-        }
+    // call = (first_record_index / 32768 + chunk) * n_mates + mate; only the final batch may end in a partial chunk, so every
+    // call in front of this batch holds 32768 reads
+    const uint64_t first_call = first_record_index / FQ_REF_BATCH * (uint64_t)n_mates;
+    const uint64_t n_calls = (uint64_t)(n + FQ_REF_BATCH - 1) / FQ_REF_BATCH * (uint64_t)n_mates;
+    auto reads_of = [&](uint64_t call) -> uint32_t {
+        if (call < first_call) return FQ_REF_BATCH;
+        const uint64_t b0 = (call - first_call) / (uint64_t)n_mates * FQ_REF_BATCH;
+        return (uint32_t)std::min<uint64_t>(FQ_REF_BATCH, n - b0);
+    };
+    KmerWalk w;
+    fq_status st = kmer_walk(ctx, K, first_call + n_calls, reads_of, &w);
+    if (st != FQ_OK) return st;
+    if (K.call_reads.size() != kKmerMaxCalls) {
+        K.call_reads.assign(kKmerMaxCalls, 0);
+        K.call_runs.assign(kKmerMaxCalls, 0);
     }
-    if (K.pass_counted <= first_call || counted_reads == 0) return FQ_OK;
+    uint64_t counted_reads = 0;
+    for (uint64_t call = first_call; call < first_call + n_calls; ++call) {
+        const uint32_t reads = reads_of(call);
+        if (call < kKmerMaxCalls) {
+            K.call_reads[call] += reads;
+            K.call_runs[call] += 1;
+        } else K.calls_beyond += 1;
+        if (call < w.counted) counted_reads += reads;
+        K.pass_reads += reads;
+    }
+    K.call_end = std::max(K.call_end, first_call + n_calls);
+    if (w.counted <= first_call || counted_reads == 0) return FQ_OK;
     // room for every k-mer this batch can add (load factor <= 1/2); the bound on the occupied slots is made exact when it matters
     const unsigned long long per_read = max_len >= K.k ? (unsigned long long)(max_len - K.k + 1) : 0ull;
     unsigned long long need = K.occupied_bound + counted_reads * per_read;
@@ -463,7 +507,7 @@ fq_status kmer_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint
     ka.res[1] = trimmed ? ctx->d_res[1].as<uint2>() : nullptr;
     ka.n_rec = n; ka.n_mates = (uint32_t)n_mates; ka.k = K.k;
     ka.replace_q = ctx->dopt.replace_q; ka.in_off = ctx->dopt.in_off;
-    ka.first_call = first_call; ka.stop_call = K.pass_counted;
+    ka.first_call = (uint32_t)first_call; ka.stop_call = w.counted;
     ka.T = kmer_table_of(K);
     ka.call_total = K.d_call_total.as<unsigned long long>();
     k_kmer<<<(n * n_mates + 255) / 256, 256, 0, ctx->stream>>>(ka);
@@ -851,7 +895,7 @@ void fq_destroy(fq_ctx *ctx)
     ctx->d_tile.release(); ctx->d_info.release(); ctx->d_stats.release(); ctx->d_rows.release();
     ctx->d_adp_codes.release(); ctx->d_adp_off.release(); ctx->d_adp_or.release();
     for (DevBuf *b : {&ctx->kmer.d_slots, &ctx->kmer.d_call_total, &ctx->kmer.d_call_distinct, &ctx->kmer.d_small,
-                      &ctx->kmer.d_big, &ctx->kmer.d_scalars}) b->release();
+                      &ctx->kmer.d_big, &ctx->kmer.d_scalars, &ctx->kmer.d_send, &ctx->kmer.d_recv}) b->release();
     ctx->h_stats.release();
     if (ctx->h_info) cudaFreeHost(ctx->h_info);
     for (auto &e : ctx->ev) if (e) cudaEventDestroy(e);
@@ -1099,57 +1143,8 @@ fq_status fq_kmer_enable(fq_ctx *ctx, uint32_t k, uint64_t split_size, uint32_t 
 fq_status fq_kmer_end_pass(fq_ctx *ctx)
 {
     if (!ctx) return FQ_ERR_ARG;
-    fq_ctx::Kmer &K = ctx->kmer;
-    if (!K.enabled) return FQ_OK;
-    CK(cudaSetDevice(ctx->device));
-    // the pass's table -> distinct k-mers per first call, histogram of counts
-    const uint32_t big_cap = 1u << 20;
-    CK(cudaMemsetAsync(K.d_call_distinct.p, 0, (size_t)kKmerMaxCalls * 8, ctx->stream));
-    CK(cudaMemsetAsync(K.d_small.p, 0, (size_t)kKmerSmallCounts * 8, ctx->stream));
-    CK(cudaMemsetAsync(K.d_scalars.p, 0, 64, ctx->stream));
-    k_kmer_summarize<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), K.d_call_distinct.as<unsigned long long>(), K.d_small.as<unsigned long long>(),
-                                                              K.d_big.as<uint32_t>(), big_cap, reinterpret_cast<uint32_t *>(K.d_scalars.as<uint8_t>() + 16),
-                                                              K.d_scalars.as<unsigned long long>());
-    ctx->launches++;
-    const uint32_t nc = std::max(K.pass_calls, 1u);
-    std::vector<unsigned long long> call_total(nc), call_distinct(nc), small(kKmerSmallCounts);
-    unsigned long long n_distinct = 0;
-    uint32_t n_big = 0;
-    CK(cudaMemcpyAsync(call_total.data(), K.d_call_total.p, (size_t)std::min(nc, kKmerMaxCalls) * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(call_distinct.data(), K.d_call_distinct.p, (size_t)std::min(nc, kKmerMaxCalls) * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(small.data(), K.d_small.p, (size_t)kKmerSmallCounts * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(&n_distinct, K.d_scalars.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(&n_big, K.d_scalars.as<uint8_t>() + 16, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    if (n_big > big_cap) return fail(ctx, FQ_ERR_ARG, "k-mer rarefaction: more than 2^20 k-mers with counts above 65535");
-    std::vector<uint32_t> big(n_big);
-    if (n_big) CK(cudaMemcpy(big.data(), K.d_big.p, (size_t)n_big * 4, cudaMemcpyDeviceToHost));
-    // points of the curve taken in this pass (trim.cpp:165-178): table size and instances after their call
-    unsigned long long run_d = 0, run_t = 0, all_t = 0;
-    size_t next = 0;
-    for (uint32_t c = 0; c < std::min(nc, kKmerMaxCalls); ++c) {
-        run_d += call_distinct[c];
-        run_t += call_total[c];
-        while (next < K.pass_points.size() && K.pass_points[next].first == c) {
-            K.samples.push_back(fq_rarefaction{K.pass_points[next].second, run_d, run_t});
-            ++next;
-        }
-    }
-    all_t = run_t;
-    // FaQCs.cpp:518-537 / 737-756: frequency histogram of the table, and one point if the curve is still empty
-    for (uint32_t c = 1; c < kKmerSmallCounts; ++c)
-        if (small[c]) K.freq[c] += small[c];
-    for (uint32_t c : big) K.freq[c] += 1;
-    if (K.collecting && K.samples.empty()) K.samples.push_back(fq_rarefaction{K.total_reads, n_distinct, all_t});
-    // a new table for the next pass
-    K.pass_calls = K.pass_counted = 0;
-    K.pass_points.clear();
-    K.occupied_bound = 0;
-    k_kmer_clear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K));
-    ctx->launches++;
-    CK(cudaMemsetAsync(K.d_call_total.p, 0, (size_t)kKmerMaxCalls * 8, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    return FQ_OK;
+    fq_ctx *const ctxs[1] = {ctx};
+    return fq_kmer_end_pass_all(ctxs, 1, nullptr);
 }
 
 fq_status fq_kmer_results(fq_ctx *ctx, fq_kmer_view *view)
@@ -1253,6 +1248,9 @@ struct NcclApi {
     ncclResult_t (*AllReduce)(const void *, void *, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*GroupStart)() = nullptr;
     ncclResult_t (*GroupEnd)() = nullptr;
+    ncclResult_t (*Send)(const void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
+    ncclResult_t (*Recv)(void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
+    ncclResult_t (*AllGather)(const void *, void *, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
     const char *(*GetErrorString)(ncclResult_t) = nullptr;
     bool ok = false;
 };
@@ -1273,8 +1271,12 @@ NcclApi &nccl()
         a.AllReduce = reinterpret_cast<decltype(a.AllReduce)>(sym("ncclAllReduce"));
         a.GroupStart = reinterpret_cast<decltype(a.GroupStart)>(sym("ncclGroupStart"));
         a.GroupEnd = reinterpret_cast<decltype(a.GroupEnd)>(sym("ncclGroupEnd"));
+        a.Send = reinterpret_cast<decltype(a.Send)>(sym("ncclSend"));
+        a.Recv = reinterpret_cast<decltype(a.Recv)>(sym("ncclRecv"));
+        a.AllGather = reinterpret_cast<decltype(a.AllGather)>(sym("ncclAllGather"));
         a.GetErrorString = reinterpret_cast<decltype(a.GetErrorString)>(sym("ncclGetErrorString"));
-        a.ok = a.GetUniqueId && a.CommInitRank && a.CommInitAll && a.CommDestroy && a.AllReduce && a.GroupStart && a.GroupEnd && a.GetErrorString;
+        a.ok = a.GetUniqueId && a.CommInitRank && a.CommInitAll && a.CommDestroy && a.AllReduce && a.GroupStart && a.GroupEnd && a.GetErrorString &&
+               a.Send && a.Recv && a.AllGather;
         return a;
     }();
     return api;
@@ -1284,6 +1286,7 @@ NcclApi &nccl()
 struct fq_comm {
     ncclComm_t comm = nullptr;
     int device = 0;
+    int n_ranks = 1, rank = 0;
 };
 
 #define NK(ctx_, call)                                                                                          \
@@ -1312,6 +1315,8 @@ fq_status fq_comm_init_rank(fq_ctx *ctx, int n_ranks, int rank, const uint8_t id
     memcpy(&u, id, FQ_COMM_ID_BYTES);
     fq_comm *c = new fq_comm();
     c->device = ctx->device;
+    c->n_ranks = n_ranks;
+    c->rank = rank;
     ncclResult_t r = nccl().CommInitRank(&c->comm, n_ranks, u, rank);
     if (r != ncclSuccess) { delete c; return fail(ctx, FQ_ERR_CUDA, std::string("ncclCommInitRank: ") + nccl().GetErrorString(r)); }
     *out = c;
@@ -1331,6 +1336,8 @@ fq_status fq_comm_init_all(fq_ctx *const *ctxs, int n, fq_comm **out)
         out[i] = new fq_comm();
         out[i]->comm = comms[i];
         out[i]->device = devs[i];
+        out[i]->n_ranks = n;
+        out[i]->rank = i;
     }
     return FQ_OK;
 }
@@ -1422,5 +1429,358 @@ fq_status fq_merge_stats(fq_ctx *dst, fq_ctx *src)
 }
 
 float fq_last_allreduce_ms(const fq_ctx *ctx) { return ctx ? ctx->allreduce_ms : 0.0f; }
+
+// ---- k-mer rarefaction: end of a pass, over one context or a table sharded over several ------------------------------
+namespace {
+
+constexpr uint32_t kKmerBigCap = 1u << 20;         // counts >= kKmerSmallCounts listed per context
+
+// What one context contributes to the end of a pass, as one flat u64 block: summed over the contexts (on the host, or one
+// ncclAllReduce across ranks).  Per-context scalars have one entry per context, zero in the others' blocks.
+struct KmerSum {
+    size_t call_total, call_distinct, call_reads, call_runs, small, n_distinct, pass_reads, calls_beyond, n_big, call_end, total;
+    explicit KmerSum(size_t n_shards)
+    {
+        size_t o = 0;
+        call_total = o;    o += kKmerMaxCalls;      // k-mer instances per call
+        call_distinct = o; o += kKmerMaxCalls;      // k-mers first seen in each call (of the context's share of the keys)
+        call_reads = o;    o += kKmerMaxCalls;      // reads per call
+        call_runs = o;     o += kKmerMaxCalls;      // times each call was run
+        small = o;         o += kKmerSmallCounts;   // k-mers per count, counts below kKmerSmallCounts
+        n_distinct = o++;
+        pass_reads = o++;
+        calls_beyond = o++;                         // calls >= kKmerMaxCalls run
+        n_big = o;         o += n_shards;           // per context: k-mers with a larger count (listed separately)
+        call_end = o;      o += n_shards;           // per context: 1 + its highest call
+        total = o;
+    }
+};
+
+struct ScopedDevBuf : DevBuf {
+    ~ScopedDevBuf() { release(); }
+};
+
+// Occupied slots of the context's table per owner.
+fq_status kmer_owner_counts(fq_ctx *ctx, uint32_t n_shards, uint64_t *counts)
+{
+    fq_ctx::Kmer &K = ctx->kmer;
+    CK(cudaSetDevice(ctx->device));
+    CK(K.d_scalars.ensure(64 + (size_t)n_shards * 8));
+    CK(cudaMemsetAsync(K.d_scalars.p, 0, (size_t)n_shards * 8, ctx->stream));
+    k_kmer_partition_count<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), n_shards, K.d_scalars.as<unsigned long long>());
+    ctx->launches++;
+    CK(cudaMemcpyAsync(counts, K.d_scalars.p, (size_t)n_shards * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return FQ_OK;
+}
+
+// The table's entries into d_send grouped by owner (group j at offsets[j]); the table is then cleared -- first grown, empty,
+// if `incoming` entries need more than half of it -- and takes back the context's own group.
+fq_status kmer_scatter(fq_ctx *ctx, uint32_t n_shards, uint32_t me, const uint64_t *counts, uint64_t incoming, std::vector<uint64_t> *offsets)
+{
+    fq_ctx::Kmer &K = ctx->kmer;
+    CK(cudaSetDevice(ctx->device));
+    offsets->assign(n_shards + 1, 0);
+    for (uint32_t j = 0; j < n_shards; ++j) (*offsets)[j + 1] = (*offsets)[j] + counts[j];
+    CK(K.d_send.ensure(std::max<uint64_t>(offsets->back(), 1) * sizeof(KmerSlot)));
+    CK(cudaMemcpyAsync(K.d_scalars.p, offsets->data(), (size_t)n_shards * 8, cudaMemcpyHostToDevice, ctx->stream));
+    k_kmer_partition_scatter<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), n_shards, K.d_scalars.as<unsigned long long>(), K.d_send.as<KmerSlot>());
+    k_kmer_clear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K));
+    ctx->launches += 2;
+    fq_status st = kmer_resize(ctx, 2 * incoming, false);
+    if (st != FQ_OK) return st;
+    if (counts[me]) {
+        k_kmer_merge<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), K.d_send.as<KmerSlot>() + (*offsets)[me], counts[me]);
+        ctx->launches++;
+    }
+    CK(cudaGetLastError());
+    return FQ_OK;
+}
+
+fq_status kmer_merge_received(fq_ctx *ctx, uint64_t n)
+{
+    if (!n) return FQ_OK;
+    k_kmer_merge<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(ctx->kmer), ctx->kmer.d_recv.as<KmerSlot>(), n);
+    ctx->launches++;
+    CK(cudaGetLastError());
+    return FQ_OK;
+}
+
+// The context's share of the table -> its summary block; `big` gets its list of counts >= kKmerSmallCounts.
+fq_status kmer_summarize(fq_ctx *ctx, const KmerSum &S, uint32_t me, std::vector<uint64_t> *flat, std::vector<uint32_t> *big)
+{
+    fq_ctx::Kmer &K = ctx->kmer;
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaMemsetAsync(K.d_call_distinct.p, 0, (size_t)kKmerMaxCalls * 8, ctx->stream));
+    CK(cudaMemsetAsync(K.d_small.p, 0, (size_t)kKmerSmallCounts * 8, ctx->stream));
+    CK(cudaMemsetAsync(K.d_scalars.p, 0, 64, ctx->stream));
+    k_kmer_summarize<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), K.d_call_distinct.as<unsigned long long>(), K.d_small.as<unsigned long long>(),
+                                                              K.d_big.as<uint32_t>(), kKmerBigCap, reinterpret_cast<uint32_t *>(K.d_scalars.as<uint8_t>() + 16),
+                                                              K.d_scalars.as<unsigned long long>());
+    ctx->launches++;
+    flat->assign(S.total, 0);
+    uint64_t *F = flat->data();
+    uint32_t n_big = 0;
+    CK(cudaMemcpyAsync(F + S.call_total, K.d_call_total.p, (size_t)kKmerMaxCalls * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(F + S.call_distinct, K.d_call_distinct.p, (size_t)kKmerMaxCalls * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(F + S.small, K.d_small.p, (size_t)kKmerSmallCounts * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(F + S.n_distinct, K.d_scalars.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&n_big, K.d_scalars.as<uint8_t>() + 16, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (!K.call_reads.empty()) {
+        std::copy(K.call_reads.begin(), K.call_reads.end(), F + S.call_reads);
+        std::copy(K.call_runs.begin(), K.call_runs.end(), F + S.call_runs);
+    }
+    F[S.pass_reads] = K.pass_reads;
+    F[S.calls_beyond] = K.calls_beyond;
+    F[S.n_big + me] = n_big;
+    F[S.call_end + me] = K.call_end;
+    if (big) {
+        big->resize(std::min(n_big, kKmerBigCap));
+        if (!big->empty()) CK(cudaMemcpy(big->data(), K.d_big.p, big->size() * 4, cudaMemcpyDeviceToHost));
+    }
+    return FQ_OK;
+}
+
+// The whole pass's summary -> the pass's points, histogram and end state (FaQCs.cpp:518-537, 737-756); every context of
+// the run computes the same from the same summary.  Then a new table for the next pass.
+fq_status kmer_finish(fq_ctx *ctx, const KmerSum &S, uint32_t n_shards, const std::vector<uint64_t> &sum, const std::vector<uint32_t> &big)
+{
+    fq_ctx::Kmer &K = ctx->kmer;
+    const uint64_t *F = sum.data();
+    uint64_t call_end = 0;
+    for (uint32_t j = 0; j < n_shards; ++j) {
+        if (F[S.n_big + j] > kKmerBigCap) return fail(ctx, FQ_ERR_ARG, "k-mer rarefaction: more than 2^20 k-mers with counts above 65535");
+        call_end = std::max(call_end, F[S.call_end + j]);
+    }
+    // every call up to the highest one run must have been run exactly once, on one of the contexts
+    const uint32_t nc = (uint32_t)std::min<uint64_t>(call_end, kKmerMaxCalls);
+    for (uint32_t c = 0; c < nc; ++c) {
+        const uint64_t runs = F[S.call_runs + c];
+        if (runs != 1) {
+            char msg[200];
+            if (runs == 0) snprintf(msg, sizeof msg, "k-mer rarefaction: trim() call %u of the pass was never run: a batch in front of the last one is missing", c);
+            else snprintf(msg, sizeof msg, "k-mer rarefaction: trim() call %u of the pass was run %llu times: batches with the same first_record_index", c,
+                          (unsigned long long)runs);
+            return fail(ctx, FQ_ERR_ARG, msg);
+        }
+    }
+    if (F[S.calls_beyond] != (call_end > kKmerMaxCalls ? call_end - kKmerMaxCalls : 0))
+        return fail(ctx, FQ_ERR_ARG, "k-mer rarefaction: the trim() calls beyond the 65536th were not each run once");
+    KmerWalk w;
+    fq_status st = kmer_walk(ctx, K, call_end, [&](uint32_t c) { return F[S.call_reads + c]; }, &w);
+    if (st != FQ_OK) return st;
+    // points of the curve taken in this pass (trim.cpp:165-178): table size and instances after their call
+    unsigned long long run_d = 0, run_t = 0;
+    size_t next = 0;
+    for (uint32_t c = 0; c < nc; ++c) {
+        run_d += F[S.call_distinct + c];
+        run_t += F[S.call_total + c];
+        while (next < w.points.size() && w.points[next].first == c) {
+            K.samples.push_back(fq_rarefaction{w.points[next].second, run_d, run_t});
+            ++next;
+        }
+    }
+    // FaQCs.cpp:518-537 / 737-756: frequency histogram of the table, and one point if the curve is still empty
+    for (uint32_t c = 1; c < kKmerSmallCounts; ++c)
+        if (F[S.small + c]) K.freq[c] += F[S.small + c];
+    for (uint32_t c : big) K.freq[c] += 1;
+    K.total_reads += F[S.pass_reads];
+    K.collecting = w.collecting;
+    if (K.collecting && K.samples.empty()) K.samples.push_back(fq_rarefaction{K.total_reads, F[S.n_distinct], run_t});
+    // a new table for the next pass
+    if (!K.call_reads.empty()) {
+        std::fill(K.call_reads.begin(), K.call_reads.end(), 0);
+        std::fill(K.call_runs.begin(), K.call_runs.end(), 0);
+    }
+    K.calls_beyond = K.call_end = K.pass_reads = 0;
+    K.occupied_bound = 0;
+    CK(cudaSetDevice(ctx->device));
+    k_kmer_clear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K));
+    ctx->launches++;
+    CK(cudaMemsetAsync(K.d_call_total.p, 0, (size_t)kKmerMaxCalls * 8, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    K.d_send.release();
+    K.d_recv.release();
+    return FQ_OK;
+}
+
+fq_status nccl_allgather_u64(fq_ctx *ctx, const fq_comm *c, const std::vector<uint64_t> &mine, std::vector<uint64_t> *all)
+{
+    const size_t m = mine.size();
+    ScopedDevBuf d;
+    CK(d.ensure((size_t)(c->n_ranks + 1) * m * 8));
+    uint64_t *send = d.as<uint64_t>() + (size_t)c->n_ranks * m;
+    all->assign((size_t)c->n_ranks * m, 0);
+    CK(cudaMemcpyAsync(send, mine.data(), m * 8, cudaMemcpyHostToDevice, ctx->stream));
+    NK(ctx, nccl().AllGather(send, d.p, m, ncclUint64, c->comm, ctx->stream));
+    CK(cudaMemcpyAsync(all->data(), d.p, all->size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return FQ_OK;
+}
+
+fq_status nccl_sum_u64(fq_ctx *ctx, const fq_comm *c, std::vector<uint64_t> *v)
+{
+    ScopedDevBuf d;
+    CK(d.ensure(v->size() * 8));
+    CK(cudaMemcpyAsync(d.p, v->data(), v->size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    NK(ctx, nccl().AllReduce(d.p, d.p, v->size(), ncclUint64, ncclSum, c->comm, ctx->stream));
+    CK(cudaMemcpyAsync(v->data(), d.p, v->size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return FQ_OK;
+}
+
+// Every rank's list of large counts (n_big[j] of rank j) on every rank.
+fq_status nccl_gather_big(fq_ctx *ctx, const fq_comm *c, const uint64_t *n_big, std::vector<uint32_t> *big)
+{
+    uint64_t most = 1;
+    for (int j = 0; j < c->n_ranks; ++j) most = std::max(most, n_big[j]);
+    ScopedDevBuf d;
+    CK(d.ensure((size_t)c->n_ranks * most * 4));
+    NK(ctx, nccl().AllGather(ctx->kmer.d_big.p, d.p, most, ncclUint32, c->comm, ctx->stream));
+    std::vector<uint32_t> all((size_t)c->n_ranks * most);
+    CK(cudaMemcpyAsync(all.data(), d.p, all.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    big->clear();
+    for (int j = 0; j < c->n_ranks; ++j) big->insert(big->end(), all.begin() + (size_t)j * most, all.begin() + (size_t)j * most + n_big[j]);
+    return FQ_OK;
+}
+
+fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
+{
+    fq_ctx *ctx = ctxs[0];
+    const fq_comm *cm = comm ? comm[0] : nullptr;
+    if (cm && (n != 1 || cm->device != ctx->device)) return fail(ctx, FQ_ERR_ARG, "fq_kmer_end_pass_all: with a communicator, pass this process's one context on its device");
+    if (cm && !nccl().ok) return fail(ctx, FQ_ERR_STATE, "NCCL (libnccl.so.2) could not be loaded");
+    const uint32_t n_shards = cm ? (uint32_t)cm->n_ranks : (uint32_t)n;
+    const uint32_t rank0 = cm ? (uint32_t)cm->rank : 0;         // shard index of ctxs[0]
+    if (n_shards > kKmerMaxOwners) return fail(ctx, FQ_ERR_ARG, "fq_kmer_end_pass_all: more than 1024 contexts");
+    for (int i = 0; i < n; ++i) {
+        fq_ctx *const c = ctxs[i];
+        c->error.clear();
+        CK(cudaSetDevice(c->device));
+        CK(cudaStreamSynchronize(c->stream));
+    }
+    // 1. agree on the parameters; 2. occupied slots per owner: header {enabled, k, split_size, num_subsample, counts[n_shards]}
+    const size_t H = 4 + n_shards;
+    std::vector<uint64_t> head((size_t)n_shards * H, 0);
+    for (int i = 0; i < n; ++i) {
+        const fq_ctx::Kmer &K = ctxs[i]->kmer;
+        uint64_t *h = head.data() + (size_t)(rank0 + i) * H;
+        h[0] = K.enabled; h[1] = K.k; h[2] = K.split_size; h[3] = K.num_subsample;
+        if (K.enabled && n_shards > 1) {
+            fq_status st = kmer_owner_counts(ctxs[i], n_shards, h + 4);
+            if (st != FQ_OK) return st;
+        }
+    }
+    if (cm) {
+        const std::vector<uint64_t> mine(head.begin() + (size_t)rank0 * H, head.begin() + (size_t)(rank0 + 1) * H);
+        fq_status st = nccl_allgather_u64(ctx, cm, mine, &head);
+        if (st != FQ_OK) return st;
+    }
+    for (uint32_t j = 1; j < n_shards; ++j)
+        if (head[(size_t)j * H] != head[0]) return fail(ctx, FQ_ERR_ARG, "fq_kmer_end_pass_all: k-mer rarefaction is enabled on some contexts only");
+    if (!head[0]) return FQ_OK;
+    for (uint32_t j = 1; j < n_shards; ++j) {
+        const uint64_t *a = head.data(), *b = head.data() + (size_t)j * H;
+        if (a[1] != b[1] || a[2] != b[2] || a[3] != b[3]) {
+            char msg[240];
+            snprintf(msg, sizeof msg, "fq_kmer_end_pass_all: context %u counts k = %llu, split_size = %llu, num_subsample = %llu; context 0 k = %llu, "
+                     "split_size = %llu, num_subsample = %llu", j, (unsigned long long)b[1], (unsigned long long)b[2], (unsigned long long)b[3],
+                     (unsigned long long)a[1], (unsigned long long)a[2], (unsigned long long)a[3]);
+            return fail(ctx, FQ_ERR_ARG, msg);
+        }
+    }
+    auto counts = [&](uint32_t from, uint32_t to) { return head[(size_t)from * H + 4 + to]; };
+    // 3, 4. exchange the groups in n_shards - 1 rounds (round r: shard s sends to s + r, receives from s - r) and merge
+    if (n_shards > 1) {
+        std::vector<std::vector<uint64_t>> offsets(n);
+        for (int i = 0; i < n; ++i) {
+            const uint32_t me = rank0 + i;
+            uint64_t incoming = 0, largest = 1;
+            for (uint32_t j = 0; j < n_shards; ++j) {
+                incoming += counts(j, me);
+                if (j != me) largest = std::max(largest, counts(j, me));
+            }
+            fq_status st = kmer_scatter(ctxs[i], n_shards, me, head.data() + (size_t)me * H + 4, incoming, &offsets[i]);
+            if (st != FQ_OK) return st;
+            fq_ctx *const c = ctxs[i];
+            fq_ctx *ctx = c;
+            CK(c->kmer.d_recv.ensure(largest * sizeof(KmerSlot)));
+        }
+        for (int i = 0; i < n; ++i) {           // every send buffer is complete before another context reads it
+            fq_ctx *ctx = ctxs[i];
+            CK(cudaSetDevice(ctx->device));
+            CK(cudaStreamSynchronize(ctx->stream));
+        }
+        for (uint32_t r = 1; r < n_shards; ++r) {
+            for (int i = 0; i < n; ++i) {
+                fq_ctx *ctx = ctxs[i];
+                const uint32_t me = rank0 + i, dst = (me + r) % n_shards, src = (me + n_shards - r) % n_shards;
+                const uint64_t n_out = counts(me, dst), n_in = counts(src, me);
+                CK(cudaSetDevice(ctx->device));
+                if (cm) {
+                    if (!n_out && !n_in) continue;      // both ends know the counts: neither posts a transfer
+                    NK(ctx, nccl().GroupStart());
+                    if (n_out) NK(ctx, nccl().Send(ctx->kmer.d_send.as<KmerSlot>() + offsets[i][dst], 2 * n_out, ncclUint64, (int)dst, cm->comm, ctx->stream));
+                    if (n_in) NK(ctx, nccl().Recv(ctx->kmer.d_recv.p, 2 * n_in, ncclUint64, (int)src, cm->comm, ctx->stream));
+                    NK(ctx, nccl().GroupEnd());
+                } else if (n_in) {
+                    const fq_ctx *from = ctxs[src];
+                    CK(cudaMemcpyPeerAsync(ctx->kmer.d_recv.p, ctx->device, from->kmer.d_send.as<KmerSlot>() + offsets[src][me], from->device,
+                                           n_in * sizeof(KmerSlot), ctx->stream));
+                }
+                fq_status st = kmer_merge_received(ctx, n_in);
+                if (st != FQ_OK) return st;
+            }
+        }
+    }
+    // 5. summarise each shard; 6. combine
+    const KmerSum S(n_shards);
+    std::vector<uint64_t> sum, flat;
+    std::vector<uint32_t> big, part;
+    for (int i = 0; i < n; ++i) {
+        fq_status st = kmer_summarize(ctxs[i], S, rank0 + i, &flat, cm ? nullptr : &part);
+        if (st != FQ_OK) return st;
+        if (sum.empty()) sum.assign(S.total, 0);
+        for (size_t k = 0; k < S.total; ++k) sum[k] += flat[k];
+        big.insert(big.end(), part.begin(), part.end());
+    }
+    if (cm) {
+        fq_status st = nccl_sum_u64(ctx, cm, &sum);
+        if (st == FQ_OK) {
+            for (uint32_t j = 0; j < n_shards; ++j)
+                if (sum[S.n_big + j] > kKmerBigCap) return fail(ctx, FQ_ERR_ARG, "k-mer rarefaction: more than 2^20 k-mers with counts above 65535");
+            st = nccl_gather_big(ctx, cm, sum.data() + S.n_big, &big);
+        }
+        if (st != FQ_OK) return st;
+    }
+    // 7. the pass's points and histogram, identically on every context
+    for (int i = 0; i < n; ++i) {
+        fq_status st = kmer_finish(ctxs[i], S, n_shards, sum, big);
+        if (st != FQ_OK) return st;
+    }
+    return FQ_OK;
+}
+
+}  // namespace
+
+fq_status fq_kmer_end_pass_all(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
+{
+    if (!ctxs || n < 1) return FQ_ERR_ARG;
+    for (int i = 0; i < n; ++i) {
+        if (!ctxs[i]) return FQ_ERR_ARG;
+        for (int j = 0; j < i; ++j)
+            if (ctxs[j] == ctxs[i]) return fail(ctxs[0], FQ_ERR_ARG, "fq_kmer_end_pass_all: a context is listed twice");
+    }
+    if (comm && !comm[0]) return fail(ctxs[0], FQ_ERR_ARG, "fq_kmer_end_pass_all: null communicator");
+    const fq_status st = kmer_end_pass_impl(ctxs, n, comm);
+    if (st != FQ_OK) {          // the verdict is the run's: every context reports it
+        std::string msg;
+        for (int i = 0; i < n && msg.empty(); ++i) msg = ctxs[i]->error;
+        for (int i = 0; i < n; ++i) ctxs[i]->error = msg;
+    }
+    return st;
+}
 
 }  // extern "C"

@@ -175,4 +175,72 @@ __global__ void __launch_bounds__(256) k_kmer_count(KmerTable T, unsigned long l
     if ((threadIdx.x & 31) == 0 && mine) atomicAdd(n_distinct, mine);
 }
 
+// ---- a table sharded over n contexts: end of pass ---------------------------------------------------------------------
+// Every context counted its own batches into its own table.  At the end of the pass each k-mer gets one owner context;
+// every context sends its entries to their owners, and each owner merges what it receives into a cleared table (counts add,
+// first calls take the minimum), so the owners' tables together hold the table one context would have built.
+constexpr uint32_t kKmerMaxOwners = 1024;
+
+// The slot index uses the low bits of the hash, the owner the high half: a shard's keys still spread over its whole table.
+__device__ __forceinline__ uint32_t kmer_owner(unsigned long long key, uint32_t n)
+{
+    return (uint32_t)(((kmer_hash(key) >> 32) * n) >> 32);
+}
+
+// Occupied slots per owner (count[n], zeroed by the caller).
+__global__ void __launch_bounds__(256) k_kmer_partition_count(KmerTable T, uint32_t n, unsigned long long *count)
+{
+    __shared__ uint32_t h[kKmerMaxOwners];
+    for (uint32_t j = threadIdx.x; j < n; j += blockDim.x) h[j] = 0;
+    __syncthreads();
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i <= T.cap_mask; i += (unsigned long long)gridDim.x * blockDim.x) {
+        const unsigned long long key = T.slots[i].key;
+        if (key != kKmerEmpty) atomicAdd(&h[kmer_owner(key, n)], 1u);
+    }
+    __syncthreads();
+    for (uint32_t j = threadIdx.x; j < n; j += blockDim.x)
+        if (h[j]) atomicAdd(&count[j], (unsigned long long)h[j]);
+}
+
+// The occupied slots into `out`, grouped by owner: cursor[j] starts at group j's offset.  The lanes of a warp that share an
+// owner take their places with one atomic.  (The grid stride is a multiple of 32 and the capacity a power of two >= 32, so
+// every lane of a warp makes the same number of trips.)
+__global__ void __launch_bounds__(256) k_kmer_partition_scatter(KmerTable T, uint32_t n, unsigned long long *cursor, KmerSlot *out)
+{
+    const uint32_t lane = threadIdx.x & 31;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i <= T.cap_mask; i += (unsigned long long)gridDim.x * blockDim.x) {
+        const KmerSlot e = T.slots[i];
+        const bool used = e.key != kKmerEmpty;
+        const uint32_t active = __ballot_sync(0xffffffffu, used);
+        if (!used) continue;
+        const uint32_t owner = kmer_owner(e.key, n);
+        const uint32_t peers = __match_any_sync(active, owner);
+        const uint32_t leader = __ffs(peers) - 1;
+        unsigned long long base = 0;
+        if (lane == leader) base = atomicAdd(&cursor[owner], (unsigned long long)__popc(peers));
+        base = __shfl_sync(peers, base, leader);
+        out[base + __popc(peers & ((1u << lane) - 1u))] = e;
+    }
+}
+
+// Entries of other tables into T: counts add, the first call is the smallest.
+__global__ void __launch_bounds__(256) k_kmer_merge(KmerTable T, const KmerSlot *in, unsigned long long n)
+{
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
+        const KmerSlot e = in[i];
+        unsigned long long slot = kmer_hash(e.key) & T.cap_mask;
+        for (;;) {
+            KmerSlot *const p = &T.slots[slot];
+            unsigned long long prev = *reinterpret_cast<volatile unsigned long long *>(&p->key);
+            if (prev == kKmerEmpty) prev = atomicCAS(&p->key, kKmerEmpty, e.key);
+            if (prev == kKmerEmpty || prev == e.key) {
+                atomicAdd(&p->count, e.count);
+                if (e.first_call < *reinterpret_cast<volatile uint32_t *>(&p->first_call)) atomicMin(&p->first_call, e.first_call);
+                break;
+            }
+            slot = (slot + 1) & T.cap_mask;
+        }
+    }
+}
+
 }  // namespace fq

@@ -1,10 +1,12 @@
 """Multi-GPU merge of the statistics through the library's own collective (fq_allreduce_stats: one
-ncclAllReduce(u64, sum) over NVLink + a max of the row counters; include/faqcs_b200.h).
+ncclAllReduce(u64, sum) over NVLink + a max of the row counters; include/faqcs_b200.h), and the end of a k-mer
+rarefaction pass over a table sharded across contexts (fq_kmer_end_pass_all).
 
 Two launch shapes, both ending in the same C call:
   * one process per GPU (torchrun): rank 0 draws the NCCL id (fq_comm_unique_id), the launcher's process group
-    broadcasts those 128 bytes, every rank joins (fq_comm_init_rank) and calls fq_allreduce_stats on its one context;
-  * one process, several GPUs: fq_comm_init_all over the contexts, one fq_allreduce_stats call for all of them.
+    broadcasts those 128 bytes, every rank joins (fq_comm_init_rank) and calls the library on its one context;
+  * one process, several GPUs: fq_comm_init_all over the contexts (statistics) or no communicator at all (k-mer pass), one
+    call for all of them.
 The reference's counterpart is the `omp critical` merge at the end of trim() (trim.cpp:120-154).
 """
 from __future__ import annotations
@@ -24,8 +26,8 @@ def _check(eng: Engine, st: int):
         raise FaqcsError(st, eng.lib.fq_last_error(eng.ctx).decode(errors="replace"))
 
 
-def allreduce_engine_stats(eng: Engine, dist, dev) -> float:
-    """One context per process: merge over the ranks of `dist` (torch.distributed).  Returns the device ms of the collective."""
+def _rank_comm(eng: Engine, dist, dev) -> C.c_void_p:
+    """This rank's communicator: rank 0 draws the NCCL id, the launcher's group broadcasts it, every rank joins."""
     import torch
     ident = torch.zeros(COMM_ID_BYTES, dtype=torch.uint8, device=dev)
     if dist.get_rank() == 0:
@@ -36,6 +38,12 @@ def allreduce_engine_stats(eng: Engine, dist, dev) -> float:
     raw = (C.c_uint8 * COMM_ID_BYTES)(*ident.cpu().tolist())
     comm = C.c_void_p()
     _check(eng, eng.lib.fq_comm_init_rank(eng.ctx, dist.get_world_size(), dist.get_rank(), raw, C.byref(comm)))
+    return comm
+
+
+def allreduce_engine_stats(eng: Engine, dist, dev) -> float:
+    """One context per process: merge over the ranks of `dist` (torch.distributed).  Returns the device ms of the collective."""
+    comm = _rank_comm(eng, dist, dev)
     try:
         ctxs = (C.c_void_p * 1)(eng.ctx)
         comms = (C.c_void_p * 1)(comm)
@@ -58,3 +66,23 @@ def allreduce_local_engines(engines: Sequence[Engine]) -> float:
     finally:
         for c in comms:
             e0.lib.fq_comm_destroy(c)
+
+
+def kmer_end_pass_local(engines: Sequence[Engine]):
+    """End of a k-mer rarefaction pass whose batches ran on these contexts (one process, any devices, a device may repeat):
+    the per-context tables are merged, and every engine's kmer_results() returns the whole run's curve and histogram."""
+    n = len(engines)
+    e0 = engines[0]
+    ctxs = (C.c_void_p * n)(*[e.ctx for e in engines])
+    _check(e0, e0.lib.fq_kmer_end_pass_all(ctxs, n, None))
+
+
+def kmer_end_pass_ranks(eng: Engine, dist, dev):
+    """The same with one context per process: the tables are merged over the ranks of `dist` (torch.distributed)."""
+    comm = _rank_comm(eng, dist, dev)
+    try:
+        ctxs = (C.c_void_p * 1)(eng.ctx)
+        comms = (C.c_void_p * 1)(comm)
+        _check(eng, eng.lib.fq_kmer_end_pass_all(ctxs, 1, comms))
+    finally:
+        eng.lib.fq_comm_destroy(comm)

@@ -781,8 +781,11 @@ struct Run {
             if (fq_create(&f, o.devices[ctxs.size()], &c) != FQ_OK) throw string(fq_last_error(nullptr));
             ctxs.push_back(c);
             if (pieces_mode) check(fq_set_output_pieces(c, 1), c);
+            if (o.kmer_rarefaction) check(fq_kmer_enable(c, o.kmer, o.split_size, o.num_subsample), c);   // one shard of the pass's table
         }
     }
+    // end of an input's pass: the contexts' k-mer tables merge into the run's curve and histogram (FaQCs.cpp:518-537, 737-756)
+    void kmer_end_pass() { check(fq_kmer_end_pass_all(ctxs.data(), (int)ctxs.size(), nullptr)); }
     void set_quality_everywhere(int q) { for (fq_ctx *c : ctxs) check(fq_set_quality(c, q), c); }
 };
 
@@ -1354,10 +1357,6 @@ int main(int argc, char *argv[])
         const bool timing = getenv("FAQCS_B200_TIMING") != nullptr;
         const double t_start = now_s();
         if (o.devices.empty()) o.devices.push_back(o.device);
-        if (o.kmer_rarefaction && o.devices.size() > 1) {
-            cerr << "**Warning** --kmer_rarefaction keeps one k-mer table: running on device " << o.devices[0] << " only" << endl;
-            o.devices.resize(1);
-        }
         if (fq_create(&f, o.devices[0], &ctx) != FQ_OK) throw string(fq_last_error(nullptr));
         if (o.kmer_rarefaction && fq_kmer_enable(ctx, o.kmer, o.split_size, o.num_subsample) != FQ_OK) throw string(fq_last_error(ctx));
         const double t_created = now_s();
@@ -1370,12 +1369,12 @@ int main(int argc, char *argv[])
         if (R.pieces_mode) R.check(fq_set_output_pieces(ctx, 1));
         if (o.has_paired()) {
             process(R, true);
-            R.check(fq_kmer_end_pass(ctx));        // FaQCs.cpp:518-537
+            R.kmer_end_pass();                     // FaQCs.cpp:518-537
         }
         if (o.has_unpaired()) {
             R.first_batch = true;      // offset detection only if still unknown; the NextSeq check runs per input (FaQCs.cpp:586,673-683)
             process(R, false);
-            R.check(fq_kmer_end_pass(ctx));        // FaQCs.cpp:737-756
+            R.kmer_end_pass();                     // FaQCs.cpp:737-756
         }
         const double t_processed = now_s();
         if (R.ctxs.size() > 1) {

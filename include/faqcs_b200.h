@@ -245,7 +245,8 @@ fq_status fq_autodetect(fq_ctx *ctx, const uint8_t *r1, size_t n1,
  * Replaces: trim() x2 + the routing/emit loop for one batch
  * (FaQCs.cpp:279-361 / 416-496 / 621-659 / 685-720).
  * first_record_index: global index of the batch's first record in its file
- * (used only for thread-count emulation); is_final: last batch of the file. */
+ * (used for thread-count emulation and for the k-mer rarefaction's trim() call
+ * numbers); is_final: last batch of the file. */
 fq_status fq_process_host(fq_ctx *ctx, const uint8_t *r1, size_t n1,
                           const uint8_t *r2, size_t n2,
                           uint64_t first_record_index, int is_final,
@@ -336,12 +337,22 @@ float     fq_last_allreduce_ms(const fq_ctx *ctx);
  * in device memory while the curve is being collected (one table per pass over an input, as in the reference); the points
  * of the curve are taken where the reference takes them -- at the end of the trim() call (32768 reads of one mate) whose
  * running read count crossed another multiple of split_size -- so batches must start on 32768-record boundaries and, unless
- * final, hold a multiple of 32768 records.  Single context only (the table does not shard, SURVEY 8(e)).
- *   fq_kmer_enable    once, before the first batch: k (Options::kmer, 2..31), Options::split_size, Options::num_subsample
- *                     (already doubled where the reference doubles it, options.cpp:506-523)
- *   fq_kmer_end_pass  after the last batch of an input (paired files, then the unpaired file)
- *   fq_kmer_results   PlotInfo::kmer_rarefaction and PlotInfo::kmer_frequency_histogram (what plot.cpp:683-733 prints);
- *                     the view's pointers belong to the context and stay valid until its next fq_kmer_* call
+ * final, hold a multiple of 32768 records.  A batch's calls follow from its first_record_index (the global index of its
+ * first record in the input): call = (first_record_index / 32768 + chunk) * n_mates + mate, so the batches of a pass may run
+ * in any order and on several contexts, each batch exactly once.
+ *   fq_kmer_enable        once, before the first batch: k (Options::kmer, 2..31), Options::split_size, Options::num_subsample
+ *                         (already doubled where the reference doubles it, options.cpp:506-523); the same on every context
+ *   fq_kmer_end_pass      after the last batch of an input (paired files, then the unpaired file), one context
+ *   fq_kmer_end_pass_all  the same for a table sharded over several contexts (below)
+ *   fq_kmer_results       PlotInfo::kmer_rarefaction and PlotInfo::kmer_frequency_histogram (what plot.cpp:683-733 prints);
+ *                         the view's pointers belong to the context and stay valid until its next fq_kmer_* call
+ *
+ * Sharded table: every context counts its own batches into its own table.  At the end of the pass every k-mer has one owner
+ * context (from the high half of its hash); the contexts send their entries to the owners in n - 1 rounds (in round r,
+ * context i sends its group for i + r and receives the group of i - r: memory = the context's entries + one received group),
+ * and each owner merges them into its cleared table (counts add, first calls take the minimum).  The owners' summaries are
+ * then summed, so every context ends the pass with the same curve, histogram and state.  FQ_ERR_ARG if the contexts differ in
+ * k, split_size or num_subsample, or if a trim() call below the highest one was run other than exactly once.
  */
 typedef struct fq_rarefaction {
     uint64_t num_seq;          /* TOTAL_NUMBER when the point was taken */
@@ -356,6 +367,11 @@ typedef struct fq_kmer_view {
 } fq_kmer_view;
 fq_status fq_kmer_enable(fq_ctx *ctx, uint32_t k, uint64_t split_size, uint32_t num_subsample);
 fq_status fq_kmer_end_pass(fq_ctx *ctx);
+/* End of one input's pass (FaQCs.cpp:518-537, 737-756) for a k-mer table sharded over n contexts.
+ * comm == NULL: all n contexts of the run live in this process (same or different devices).
+ * comm != NULL: n == 1, this process's context of an n-rank job (fq_comm_init_rank).
+ * Afterwards fq_kmer_results returns the merged curve and histogram on every context. */
+fq_status fq_kmer_end_pass_all(fq_ctx *const *ctx, int n, fq_comm *const *comm);
 fq_status fq_kmer_results(fq_ctx *ctx, fq_kmer_view *view);
 
 /* Zero the accumulators (new run on the same context). */
