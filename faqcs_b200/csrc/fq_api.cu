@@ -16,6 +16,7 @@
 #include <map>
 #include <mutex>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "fq_adapter.cuh"
@@ -34,40 +35,48 @@ namespace {
 
 std::string g_create_error;
 
-struct DevBuf {
+// Device (cudaMalloc) or pinned host (cudaMallocHost) memory with one owner: move-only, freed by its destructor.
+// ensure() grows it with 1/8 headroom and does not keep the contents.
+template <bool Pinned>
+struct Buf {
     void *p = nullptr;
     size_t cap = 0;
+    Buf() = default;
+    Buf(const Buf &) = delete;
+    Buf &operator=(const Buf &) = delete;
+    Buf(Buf &&o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    Buf &operator=(Buf &&o) noexcept
+    {
+        if (this != &o) {
+            release();
+            p = std::exchange(o.p, nullptr);
+            cap = std::exchange(o.cap, 0);
+        }
+        return *this;
+    }
+    ~Buf() { release(); }
     cudaError_t ensure(size_t bytes)
     {
         if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
+        release();
         const size_t want = bytes + bytes / 8 + 256;
-        cudaError_t e = cudaMalloc(&p, want);
+        cudaError_t e = Pinned ? cudaMallocHost(&p, want) : cudaMalloc(&p, want);
         if (e == cudaSuccess) cap = want;
         return e;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+    void release()
+    {
+        if (p) {
+            if (Pinned) cudaFreeHost(p);
+            else cudaFree(p);
+        }
+        p = nullptr;
+        cap = 0;
+    }
     template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
-
-struct PinnedBuf {
-    void *p = nullptr;
-    size_t cap = 0;
-    cudaError_t ensure(size_t bytes)
-    {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-        const size_t want = bytes + bytes / 8 + 256;
-        cudaError_t e = cudaMallocHost(&p, want);
-        if (e == cudaSuccess) cap = want;
-        return e;
-    }
-    void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
-};
+using DevBuf = Buf<false>;
+using HostBuf = Buf<true>;
 
 const char *kPhiX = "__PhiX174_NC_001422__";                       // FaQCs.h:29-30
 const char *kPhiXComplement = "__PhiX174_NC_001422_complement__";
@@ -97,13 +106,11 @@ struct fq_ctx {
     DevBuf d_raw[2], d_chunk[2], d_nl[2], d_rec[2], d_canon[2], d_adp[2], d_adp_best[2], d_res[2], d_dbg[2], d_tile, d_out[2][4];
     DevBuf d_raw_slot[2][2];           // pipelined submit: raw input slots
     DevBuf d_info, d_stats, d_rows;
-    BatchInfo *h_info = nullptr;       // pinned
+    HostBuf h_info;                    // one BatchInfo
     StatsLayout L{};
-    PinnedBuf h_out[2][4], h_dbg[2], h_stats, h_pieces[2][4];
+    HostBuf h_out[2][4], h_dbg[2], h_stats, h_pieces[2][4];
     DevBuf d_pieces[2][4];
     bool pieces = false;               // fq_set_output_pieces
-    int out_slot = 0;                   // which d_out / h_out set process_common fills
-    bool async_out = false;            // D2H on s_out, caller waits on ev_out
     cudaStream_t s_in = nullptr, s_out = nullptr;
     cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_comp[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
     // pipelined path: an input slot is busy from submit until run returns, an output slot from run until wait
@@ -146,6 +153,15 @@ struct fq_ctx {
     size_t smem_optin = 0;
     float allreduce_ms = 0.0f;
     const void *last_dev_out[4] = {nullptr, nullptr, nullptr, nullptr};
+
+    // The buffers free themselves after this; fq_destroy makes the device current first.
+    ~fq_ctx()
+    {
+        for (cudaEvent_t e : {ev_in[0], ev_in[1], ev_comp[0], ev_comp[1], ev_out[0], ev_out[1], ev[0], ev[1], ev[2], ev[3], ev[4]})
+            if (e) cudaEventDestroy(e);
+        for (cudaStream_t s : {s_in, s_out, stream})
+            if (s) cudaStreamDestroy(s);
+    }
 };
 
 namespace {
@@ -228,8 +244,7 @@ fq_status ensure_stats_rows(fq_ctx *ctx, uint32_t rows)
     DevBuf nb;
     CK(nb.ensure(newL.total * 8));
     CK(cudaMemcpy(nb.p, newv.data(), newL.total * 8, cudaMemcpyHostToDevice));
-    ctx->d_stats.release();
-    ctx->d_stats = nb;
+    ctx->d_stats = std::move(nb);
     ctx->L = newL;
     return FQ_OK;
 }
@@ -288,6 +303,37 @@ void refresh_dev_opts(fq_ctx *ctx)
     d.n_adapters = o.n_adapters;
 }
 
+// A fresh BatchInfo on the device, through the pinned mirror, ahead of the batch's kernels.
+cudaError_t reset_info(fq_ctx *ctx)
+{
+    BatchInfo init{};
+    init.err_record = 0xffffffffu;
+    init.detect_key = ~0ull;
+    *ctx->h_info.as<BatchInfo>() = init;
+    return cudaMemcpyAsync(ctx->d_info.p, ctx->h_info.p, sizeof(BatchInfo), cudaMemcpyHostToDevice, ctx->stream);
+}
+
+// The device's BatchInfo once the stream has caught up with it.
+cudaError_t read_info(fq_ctx *ctx, BatchInfo *hi)
+{
+    cudaError_t e = cudaMemcpyAsync(ctx->h_info.p, ctx->d_info.p, sizeof(BatchInfo), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e == cudaSuccess) *hi = *ctx->h_info.as<BatchInfo>();
+    return e;
+}
+
+// Every context's stream drained, each with its device current.  Like the rest of an entry point over several contexts,
+// a failure is reported on ctxs[0].
+fq_status sync_all(fq_ctx *const *ctxs, int n)
+{
+    fq_ctx *const ctx = ctxs[0];
+    for (int i = 0; i < n; ++i) {
+        CK(cudaSetDevice(ctxs[i]->device));
+        CK(cudaStreamSynchronize(ctxs[i]->stream));
+    }
+    return FQ_OK;
+}
+
 // Framing of one mate: count -> scan -> (sync) -> scatter -> records.
 fq_status frame_mate(fq_ctx *ctx, int m, const uint8_t *d_raw, size_t n, uint32_t *n_rec_out)
 {
@@ -296,6 +342,7 @@ fq_status frame_mate(fq_ctx *ctx, int m, const uint8_t *d_raw, size_t n, uint32_
     if (n >= (1ull << 30)) return fail(ctx, FQ_ERR_ARG, "batch larger than 1 GiB per mate: split it");
     if ((reinterpret_cast<uintptr_t>(d_raw) & 15) != 0) return fail(ctx, FQ_ERR_ARG, "device input must be 16-byte aligned");
     BatchInfo *info = ctx->d_info.as<BatchInfo>();
+    BatchInfo hi{};
     // single-pass segmented line index: one contiguous segment per resident warp, no cross-warp dependency
     int frame_ctas = 4;                                     // resident CTAs per SM -> exactly one wave of segments
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&frame_ctas, k_frame_lines<false>, kFrameThreads, 0));
@@ -324,16 +371,15 @@ fq_status frame_mate(fq_ctx *ctx, int m, const uint8_t *d_raw, size_t n, uint32_
             else k_frame_lines<true><<<grid, kFrameThreads, 0, ctx->stream>>>(d_raw, n, seg_bytes, n_seg, ctx->d_nl[m].as<uint32_t>(), seg_cap, seg_count, info, m, 0);
             k_scan_segments<<<1, 1024, 0, ctx->stream>>>(seg_count, n_seg, seg_base, info, m);
             ctx->launches += 2;
-            CK(cudaMemcpyAsync(ctx->h_info, info, sizeof(BatchInfo), cudaMemcpyDeviceToHost, ctx->stream));
-            CK(cudaStreamSynchronize(ctx->stream));
-            if (exact || !ctx->h_info->frame_exact[m]) break;
+            CK(read_info(ctx, &hi));
+            if (exact || !hi.frame_exact[m]) break;
             ctx->frame_exact[m] = true;                   // the fast instance gave up: run the exact one
         }
-        n_lines = ctx->h_info->n_lines[m];
-        if (ctx->h_info->seg_overflow == 0) break;
-        seg_cap = ctx->h_info->seg_overflow + 64;           // very short lines: repeat once with the exact need
+        n_lines = hi.n_lines[m];
+        if (hi.seg_overflow == 0) break;
+        seg_cap = hi.seg_overflow + 64;           // very short lines: repeat once with the exact need
     }
-    const bool had_cr = ctx->h_info->n_cr[m] != 0;
+    const bool had_cr = hi.n_cr[m] != 0;
     if (had_cr) {
         // CRLF input (or stray CRs): exact CR count, to be compared with the CRs that sit right before a '\n'
         CK(cudaMemsetAsync(&info->n_cr[m], 0, 4, ctx->stream));
@@ -354,11 +400,10 @@ fq_status frame_mate(fq_ctx *ctx, int m, const uint8_t *d_raw, size_t n, uint32_
     ctx->launches++;
     if (had_cr) {
         // exact CR count against the CRs that close a line: any other one cuts its line short (strpbrk, fastq.cpp:44)
-        CK(cudaMemcpyAsync(ctx->h_info, info, sizeof(BatchInfo), cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        if (ctx->h_info->n_cr[m] != ctx->h_info->n_cr_eol[m]) {
+        CK(read_info(ctx, &hi));
+        if (hi.n_cr[m] != hi.n_cr_eol[m]) {
             // the lengths (and a possible |seq| != |qual| verdict) of k_build_records are void for such lines: redo them
-            if ((ctx->h_info->err & ~kErrLenMismatch) == 0) {
+            if ((hi.err & ~kErrLenMismatch) == 0) {
                 const uint32_t zero = 0, none = 0xffffffffu;
                 CK(cudaMemcpyAsync(&info->err, &zero, 4, cudaMemcpyHostToDevice, ctx->stream));
                 CK(cudaMemcpyAsync(&info->err_record, &none, 4, cudaMemcpyHostToDevice, ctx->stream));
@@ -412,8 +457,7 @@ fq_status kmer_resize(fq_ctx *ctx, unsigned long long slots, bool keep = true)
     if (K.cap) k_kmer_rehash<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), to);
     ctx->launches += K.cap ? 2 : 1;
     CK(cudaStreamSynchronize(ctx->stream));
-    K.d_slots.release();
-    K.d_slots = ns;
+    K.d_slots = std::move(ns);
     K.cap = cap;
     return FQ_OK;
 }
@@ -515,8 +559,9 @@ fq_status kmer_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint
     return FQ_OK;
 }
 
+// Outputs go to the d_out / h_out set `slot`.  With async_copy the D2H runs on s_out and the caller waits on ev_out.
 fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint8_t *d_r2, size_t n2, bool paired,
-                         uint64_t first_record_index, int is_final, int copy_out, fq_batch_out *out)
+                         uint64_t first_record_index, int is_final, int copy_out, int slot, bool async_copy, fq_batch_out *out)
 {
     memset(out, 0, sizeof(*out));
     for (auto &p : ctx->last_dev_out) p = nullptr;
@@ -528,11 +573,7 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
     if (o.filter_adapter && o.num_thread && (first_record_index % FQ_REF_BATCH) != 0)
         return fail(ctx, FQ_ERR_ARG, "thread-count emulation needs batches that start on a 32768-record boundary");
     BatchInfo *info = ctx->d_info.as<BatchInfo>();
-    BatchInfo init{};
-    init.err_record = 0xffffffffu;
-    init.detect_key = ~0ull;
-    *ctx->h_info = init;
-    CK(cudaMemcpyAsync(info, ctx->h_info, sizeof(BatchInfo), cudaMemcpyHostToDevice, ctx->stream));
+    CK(reset_info(ctx));
     CK(cudaEventRecord(ctx->ev[0], ctx->stream));
 
     uint32_t n_rec[2] = {0, 0};
@@ -553,15 +594,12 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
         return FQ_OK;
     }
     // second look at the framing scalars: max length, CR accounting, |seq| != |qual|
-    CK(cudaMemcpyAsync(ctx->h_info, info, sizeof(BatchInfo), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    {
-        BatchInfo hi = *ctx->h_info;
-        st = map_device_error(ctx, hi);
-        if (st != FQ_OK) return st;
-    }
+    BatchInfo hi;
+    CK(read_info(ctx, &hi));
+    st = map_device_error(ctx, hi);
+    if (st != FQ_OK) return st;
     CK(cudaEventRecord(ctx->ev[4], ctx->stream));
-    const uint32_t max_len = std::max(ctx->h_info->max_len[0], ctx->h_info->max_len[1]);
+    const uint32_t max_len = std::max(hi.max_len[0], hi.max_len[1]);
     if (max_len > kResLenMask) return fail(ctx, FQ_ERR_ARG, "read longer than 16 Mi bases");
     st = ensure_stats_rows(ctx, max_len);
     if (st != FQ_OK) return st;
@@ -727,11 +765,11 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
         // paired run takes mate 1 OR mate 2 of each pair, i.e. up to sum_i max(rec1_i, rec2_i) <= n1 + n2 bytes
         const size_t cap[4] = {paired ? n1 : 0, paired ? n2 : 0, paired ? n1 + n2 : n1, o.discard ? n1 + n2 : 0};
         for (int s = 0; s < 4; ++s) {
-            if (cap[s]) CK(ctx->d_out[ctx->out_slot][s].ensure(cap[s] + 16));
-            ea.out[s] = ctx->d_out[ctx->out_slot][s].as<uint8_t>();
+            if (cap[s]) CK(ctx->d_out[slot][s].ensure(cap[s] + 16));
+            ea.out[s] = ctx->d_out[slot][s].as<uint8_t>();
             if (pieces && cap[s]) {       // at most one piece per record and mate
-                CK(ctx->d_pieces[ctx->out_slot][s].ensure(((size_t)n * (s == 3 && paired ? 2 : 1) + 1) * sizeof(fq_out_piece)));
-                ea.pieces[s] = ctx->d_pieces[ctx->out_slot][s].as<fq_out_piece>();
+                CK(ctx->d_pieces[slot][s].ensure(((size_t)n * (s == 3 && paired ? 2 : 1) + 1) * sizeof(fq_out_piece)));
+                ea.pieces[s] = ctx->d_pieces[slot][s].as<fq_out_piece>();
             }
         }
     }
@@ -755,15 +793,13 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
         ctx->launches++;
     }
     CK(cudaEventRecord(ctx->ev[3], ctx->stream));
-    CK(cudaMemcpyAsync(ctx->h_info, info, sizeof(BatchInfo), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
+    CK(read_info(ctx, &hi));
     CK(cudaGetLastError());
     cudaEventElapsedTime(&ctx->t_seg[0], ctx->ev[0], ctx->ev[3]);
     cudaEventElapsedTime(&ctx->t_seg[1], ctx->ev[0], ctx->ev[4]);
     cudaEventElapsedTime(&ctx->t_seg[2], ctx->ev[4], ctx->ev[1]);
     cudaEventElapsedTime(&ctx->t_seg[3], ctx->ev[1], ctx->ev[2]);
     cudaEventElapsedTime(&ctx->t_seg[4], ctx->ev[2], ctx->ev[3]);
-    const BatchInfo hi = *ctx->h_info;
     st = map_device_error(ctx, hi);
     if (st != FQ_OK) return st;
     out->n_valid[0] = hi.n_valid[0];
@@ -772,7 +808,7 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
     out->paired_base_length = hi.paired_bases;
     for (int s = 0; s < 4; ++s) {
         out->bytes[s] = o.qc_only ? 0 : hi.out_bytes[s];
-        ctx->last_dev_out[s] = out->bytes[s] ? ctx->d_out[ctx->out_slot][s].p : nullptr;
+        ctx->last_dev_out[s] = out->bytes[s] ? ctx->d_out[slot][s].p : nullptr;
         out->n_pieces[s] = pieces ? hi.out_pieces[s] : 0;
         out->literal_bytes[s] = pieces ? hi.out_literal[s] : 0;
     }
@@ -780,9 +816,9 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
         // D2H of the four streams: on the compute stream (synchronous API) or, pipelined, on the copy-out
         // stream behind an event so that it overlaps the next batch's kernels
         cudaStream_t cs = ctx->stream;
-        if (ctx->async_out) {
-            CK(cudaEventRecord(ctx->ev_comp[ctx->out_slot], ctx->stream));
-            CK(cudaStreamWaitEvent(ctx->s_out, ctx->ev_comp[ctx->out_slot], 0));
+        if (async_copy) {
+            CK(cudaEventRecord(ctx->ev_comp[slot], ctx->stream));
+            CK(cudaStreamWaitEvent(ctx->s_out, ctx->ev_comp[slot], 0));
             cs = ctx->s_out;
         }
         for (int s = 0; s < 4; ++s) {
@@ -790,18 +826,18 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
             // pieces mode: only the literal bytes and the piece list travel
             const size_t nb = pieces ? out->literal_bytes[s] : out->bytes[s];
             if (nb) {
-                CK(ctx->h_out[ctx->out_slot][s].ensure(nb));
-                CK(cudaMemcpyAsync(ctx->h_out[ctx->out_slot][s].p, ctx->d_out[ctx->out_slot][s].p, nb, cudaMemcpyDeviceToHost, cs));
-                out->data[s] = static_cast<const uint8_t *>(ctx->h_out[ctx->out_slot][s].p);
+                CK(ctx->h_out[slot][s].ensure(nb));
+                CK(cudaMemcpyAsync(ctx->h_out[slot][s].p, ctx->d_out[slot][s].p, nb, cudaMemcpyDeviceToHost, cs));
+                out->data[s] = static_cast<const uint8_t *>(ctx->h_out[slot][s].p);
             }
             if (pieces && out->n_pieces[s]) {
                 const size_t pb = out->n_pieces[s] * sizeof(fq_out_piece);
-                CK(ctx->h_pieces[ctx->out_slot][s].ensure(pb));
-                CK(cudaMemcpyAsync(ctx->h_pieces[ctx->out_slot][s].p, ctx->d_pieces[ctx->out_slot][s].p, pb, cudaMemcpyDeviceToHost, cs));
-                out->pieces[s] = static_cast<const fq_out_piece *>(ctx->h_pieces[ctx->out_slot][s].p);
+                CK(ctx->h_pieces[slot][s].ensure(pb));
+                CK(cudaMemcpyAsync(ctx->h_pieces[slot][s].p, ctx->d_pieces[slot][s].p, pb, cudaMemcpyDeviceToHost, cs));
+                out->pieces[s] = static_cast<const fq_out_piece *>(ctx->h_pieces[slot][s].p);
             }
         }
-        if (ctx->async_out) CK(cudaEventRecord(ctx->ev_out[ctx->out_slot], ctx->s_out));
+        if (async_copy) CK(cudaEventRecord(ctx->ev_out[slot], ctx->s_out));
     }
     if (ctx->debug_results) {
         for (int m = 0; m < n_mates; ++m) {
@@ -854,7 +890,7 @@ fq_status fq_create(const fq_options *opt, int device, fq_ctx **out)
             CK(cudaEventCreateWithFlags(&ctx->ev_out[k], cudaEventDisableTiming));
         }
         for (auto &e : ctx->ev) CK(cudaEventCreate(&e));
-        CK(cudaMallocHost(reinterpret_cast<void **>(&ctx->h_info), sizeof(BatchInfo)));
+        CK(ctx->h_info.ensure(sizeof(BatchInfo)));
         CK(ctx->d_info.ensure(sizeof(BatchInfo)));
         CK(ctx->d_rows.ensure(sizeof(StatsRows)));
         CK(cudaMemset(ctx->d_rows.p, 0, sizeof(StatsRows)));
@@ -877,29 +913,9 @@ void fq_destroy(fq_ctx *ctx)
 {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    for (int m = 0; m < 2; ++m) {
-        ctx->d_raw[m].release(); ctx->d_chunk[m].release(); ctx->d_nl[m].release(); ctx->d_rec[m].release(); ctx->d_canon[m].release();
-        ctx->d_adp[m].release(); ctx->d_adp_best[m].release(); ctx->d_res[m].release(); ctx->d_dbg[m].release();
-        ctx->h_dbg[m].release();
-    }
-    for (int k = 0; k < 2; ++k) {
-        for (int s = 0; s < 4; ++s) { ctx->d_out[k][s].release(); ctx->h_out[k][s].release(); ctx->d_pieces[k][s].release(); ctx->h_pieces[k][s].release(); }
-        for (int m = 0; m < 2; ++m) ctx->d_raw_slot[k][m].release();
-        if (ctx->ev_in[k]) cudaEventDestroy(ctx->ev_in[k]);
-        if (ctx->ev_comp[k]) cudaEventDestroy(ctx->ev_comp[k]);
-        if (ctx->ev_out[k]) cudaEventDestroy(ctx->ev_out[k]);
-    }
-    if (ctx->s_in) cudaStreamDestroy(ctx->s_in);
-    if (ctx->s_out) cudaStreamDestroy(ctx->s_out);
-    ctx->d_tile.release(); ctx->d_info.release(); ctx->d_stats.release(); ctx->d_rows.release();
-    ctx->d_adp_codes.release(); ctx->d_adp_off.release(); ctx->d_adp_or.release();
-    for (DevBuf *b : {&ctx->kmer.d_slots, &ctx->kmer.d_call_total, &ctx->kmer.d_call_distinct, &ctx->kmer.d_small,
-                      &ctx->kmer.d_big, &ctx->kmer.d_scalars, &ctx->kmer.d_send, &ctx->kmer.d_recv}) b->release();
-    ctx->h_stats.release();
-    if (ctx->h_info) cudaFreeHost(ctx->h_info);
-    for (auto &e : ctx->ev) if (e) cudaEventDestroy(e);
-    if (ctx->stream) cudaStreamDestroy(ctx->stream);
+    // copies queued by fq_submit_host / fq_run may still target buffers the destructor frees
+    for (cudaStream_t s : {ctx->stream, ctx->s_in, ctx->s_out})
+        if (s) cudaStreamSynchronize(s);
     delete ctx;
 }
 
@@ -954,11 +970,7 @@ fq_status fq_autodetect(fq_ctx *ctx, const uint8_t *r1, size_t n1, const uint8_t
         for (int m = 0; m < (paired ? 2 : 1); ++m) {
             const uint8_t *h = m ? r2 : r1;
             const size_t n = m ? n2 : n1;
-            BatchInfo init{};
-            init.err_record = 0xffffffffu;
-            init.detect_key = ~0ull;
-            *ctx->h_info = init;
-            CK(cudaMemcpyAsync(ctx->d_info.p, ctx->h_info, sizeof(BatchInfo), cudaMemcpyHostToDevice, ctx->stream));
+            CK(reset_info(ctx));
             uint32_t n_rec = 0;
             if (n) {
                 CK(ctx->d_raw[m].ensure(n + 16));
@@ -972,13 +984,13 @@ fq_status fq_autodetect(fq_ctx *ctx, const uint8_t *r1, size_t n1, const uint8_t
                                                                                  ctx->d_info.as<BatchInfo>());
                 ctx->launches++;
             }
-            CK(cudaMemcpyAsync(ctx->h_info, ctx->d_info.p, sizeof(BatchInfo), cudaMemcpyDeviceToHost, ctx->stream));
-            CK(cudaStreamSynchronize(ctx->stream));
-            fq_status st = map_device_error(ctx, *ctx->h_info);
+            BatchInfo hi;
+            CK(read_info(ctx, &hi));
+            fq_status st = map_device_error(ctx, hi);
             if (st != FQ_OK) return st;
-            if (ctx->h_info->detect_key == ~0ull)
+            if (hi.detect_key == ~0ull)
                 return fail(ctx, FQ_ERR_OFFSET, "trim.cpp:auto_detect_quality_offset: Unknown quality format!");
-            detected[m] = (int)(ctx->h_info->detect_key & 0xff);
+            detected[m] = (int)(hi.detect_key & 0xff);
         }
         if (paired && detected[0] != detected[1])
             return fail(ctx, FQ_ERR_OFFSET, "FaQCs.cpp:process_paired: I/O Error (inconsistent quality offset detection between reads one and two)");
@@ -1008,10 +1020,8 @@ fq_status fq_process_host(fq_ctx *ctx, const uint8_t *r1, size_t n1, const uint8
         CK(ctx->d_raw[1].ensure(n2 + 16));
         if (n2) CK(cudaMemcpyAsync(ctx->d_raw[1].p, r2, n2, cudaMemcpyHostToDevice, ctx->stream));
     }
-    ctx->out_slot = 0;
-    ctx->async_out = false;
     return process_common(ctx, ctx->d_raw[0].as<uint8_t>(), n1, paired ? ctx->d_raw[1].as<uint8_t>() : nullptr, n2, paired,
-                          first_record_index, is_final, 1, out);
+                          first_record_index, is_final, 1, 0, false, out);
 }
 
 // ---- pipelined host path: submit (H2D on its own stream) / run (kernels) / wait (D2H on its own stream) ----
@@ -1050,12 +1060,9 @@ fq_status fq_run(fq_ctx *ctx, uint64_t ticket)
     if (ctx->debug_results) return fail(ctx, FQ_ERR_STATE, "fq_run: per-read debug results are only available through the synchronous entry points");
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[slot], 0));
-    ctx->out_slot = slot;
-    ctx->async_out = true;
     fq_ctx::Finished &f = ctx->fin[slot];
     fq_status st = process_common(ctx, ctx->d_raw_slot[slot][0].as<uint8_t>(), p.n1, p.paired ? ctx->d_raw_slot[slot][1].as<uint8_t>() : nullptr,
-                                  p.n2, p.paired, p.first, p.is_final, 1, &f.out);
-    ctx->async_out = false;
+                                  p.n2, p.paired, p.first, p.is_final, 1, slot, true, &f.out);
     p.busy = false;                       // the kernels are done with the raw input slot
     if (st != FQ_OK) return st;
     f.busy = true;
@@ -1083,10 +1090,8 @@ fq_status fq_process_device(fq_ctx *ctx, const void *d_r1, size_t n1, const void
 {
     if (!ctx || !out || (!d_r1 && n1) || (!d_r2 && n2)) return FQ_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
-    ctx->out_slot = 0;
-    ctx->async_out = false;
     return process_common(ctx, static_cast<const uint8_t *>(d_r1), n1, static_cast<const uint8_t *>(d_r2), n2, d_r2 != nullptr,
-                          first_record_index, is_final, copy_out, out);
+                          first_record_index, is_final, copy_out, 0, false, out);
 }
 
 fq_status fq_device_outputs(fq_ctx *ctx, const void *d_out[FQ_NUM_STREAM])
@@ -1357,11 +1362,10 @@ fq_status fq_allreduce_stats(fq_ctx *const *ctxs, int n, fq_comm *const *comms)
     if (!ctxs || !comms || n < 1) return FQ_ERR_ARG;
     fq_ctx *ctx = ctxs[0];
     if (!nccl().ok) return fail(ctx, FQ_ERR_STATE, "NCCL (libnccl.so.2) could not be loaded");
-    for (int i = 0; i < n; ++i) {
+    for (int i = 0; i < n; ++i)
         if (!ctxs[i] || !comms[i] || comms[i]->device != ctxs[i]->device) return fail(ctx, FQ_ERR_ARG, "fq_allreduce_stats: communicator and context are on different devices");
-        CK(cudaSetDevice(ctxs[i]->device));
-        CK(cudaStreamSynchronize(ctxs[i]->stream));
-    }
+    fq_status st = sync_all(ctxs, n);
+    if (st != FQ_OK) return st;
     // 1. every rank must use the same layout: agree on the row capacity (MAX), grow where needed
     std::vector<DevBuf> d_cap(n);
     std::vector<uint32_t> cap(n);
@@ -1378,7 +1382,7 @@ fq_status fq_allreduce_stats(fq_ctx *const *ctxs, int n, fq_comm *const *comms)
         CK(cudaSetDevice(ctxs[i]->device));
         CK(cudaMemcpyAsync(&cap[i], d_cap[i].p, 4, cudaMemcpyDeviceToHost, ctxs[i]->stream));
         CK(cudaStreamSynchronize(ctxs[i]->stream));
-        fq_status st = ensure_stats_rows(ctxs[i], cap[i]);
+        st = ensure_stats_rows(ctxs[i], cap[i]);
         if (st != FQ_OK) return st;
         if (ctxs[i]->L.rows != cap[i] && ctxs[i]->L.rows != std::max(64u, round_up(cap[i], 64)))
             return fail(ctx, FQ_ERR_STATE, "fq_allreduce_stats: row capacities disagree");
@@ -1454,10 +1458,6 @@ struct KmerSum {
         call_end = o;      o += n_shards;           // per context: 1 + its highest call
         total = o;
     }
-};
-
-struct ScopedDevBuf : DevBuf {
-    ~ScopedDevBuf() { release(); }
 };
 
 // Occupied slots of the context's table per owner.
@@ -1608,7 +1608,7 @@ fq_status kmer_finish(fq_ctx *ctx, const KmerSum &S, uint32_t n_shards, const st
 fq_status nccl_allgather_u64(fq_ctx *ctx, const fq_comm *c, const std::vector<uint64_t> &mine, std::vector<uint64_t> *all)
 {
     const size_t m = mine.size();
-    ScopedDevBuf d;
+    DevBuf d;
     CK(d.ensure((size_t)(c->n_ranks + 1) * m * 8));
     uint64_t *send = d.as<uint64_t>() + (size_t)c->n_ranks * m;
     all->assign((size_t)c->n_ranks * m, 0);
@@ -1621,7 +1621,7 @@ fq_status nccl_allgather_u64(fq_ctx *ctx, const fq_comm *c, const std::vector<ui
 
 fq_status nccl_sum_u64(fq_ctx *ctx, const fq_comm *c, std::vector<uint64_t> *v)
 {
-    ScopedDevBuf d;
+    DevBuf d;
     CK(d.ensure(v->size() * 8));
     CK(cudaMemcpyAsync(d.p, v->data(), v->size() * 8, cudaMemcpyHostToDevice, ctx->stream));
     NK(ctx, nccl().AllReduce(d.p, d.p, v->size(), ncclUint64, ncclSum, c->comm, ctx->stream));
@@ -1635,7 +1635,7 @@ fq_status nccl_gather_big(fq_ctx *ctx, const fq_comm *c, const uint64_t *n_big, 
 {
     uint64_t most = 1;
     for (int j = 0; j < c->n_ranks; ++j) most = std::max(most, n_big[j]);
-    ScopedDevBuf d;
+    DevBuf d;
     CK(d.ensure((size_t)c->n_ranks * most * 4));
     NK(ctx, nccl().AllGather(ctx->kmer.d_big.p, d.p, most, ncclUint32, c->comm, ctx->stream));
     std::vector<uint32_t> all((size_t)c->n_ranks * most);
@@ -1648,19 +1648,16 @@ fq_status nccl_gather_big(fq_ctx *ctx, const fq_comm *c, const uint64_t *n_big, 
 
 fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
 {
-    fq_ctx *ctx = ctxs[0];
+    fq_ctx *const ctx0 = ctxs[0];
     const fq_comm *cm = comm ? comm[0] : nullptr;
-    if (cm && (n != 1 || cm->device != ctx->device)) return fail(ctx, FQ_ERR_ARG, "fq_kmer_end_pass_all: with a communicator, pass this process's one context on its device");
-    if (cm && !nccl().ok) return fail(ctx, FQ_ERR_STATE, "NCCL (libnccl.so.2) could not be loaded");
+    if (cm && (n != 1 || cm->device != ctx0->device)) return fail(ctx0, FQ_ERR_ARG, "fq_kmer_end_pass_all: with a communicator, pass this process's one context on its device");
+    if (cm && !nccl().ok) return fail(ctx0, FQ_ERR_STATE, "NCCL (libnccl.so.2) could not be loaded");
     const uint32_t n_shards = cm ? (uint32_t)cm->n_ranks : (uint32_t)n;
     const uint32_t rank0 = cm ? (uint32_t)cm->rank : 0;         // shard index of ctxs[0]
-    if (n_shards > kKmerMaxOwners) return fail(ctx, FQ_ERR_ARG, "fq_kmer_end_pass_all: more than 1024 contexts");
-    for (int i = 0; i < n; ++i) {
-        fq_ctx *const c = ctxs[i];
-        c->error.clear();
-        CK(cudaSetDevice(c->device));
-        CK(cudaStreamSynchronize(c->stream));
-    }
+    if (n_shards > kKmerMaxOwners) return fail(ctx0, FQ_ERR_ARG, "fq_kmer_end_pass_all: more than 1024 contexts");
+    for (int i = 0; i < n; ++i) ctxs[i]->error.clear();
+    fq_status st = sync_all(ctxs, n);
+    if (st != FQ_OK) return st;
     // 1. agree on the parameters; 2. occupied slots per owner: header {enabled, k, split_size, num_subsample, counts[n_shards]}
     const size_t H = 4 + n_shards;
     std::vector<uint64_t> head((size_t)n_shards * H, 0);
@@ -1669,17 +1666,17 @@ fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
         uint64_t *h = head.data() + (size_t)(rank0 + i) * H;
         h[0] = K.enabled; h[1] = K.k; h[2] = K.split_size; h[3] = K.num_subsample;
         if (K.enabled && n_shards > 1) {
-            fq_status st = kmer_owner_counts(ctxs[i], n_shards, h + 4);
+            st = kmer_owner_counts(ctxs[i], n_shards, h + 4);
             if (st != FQ_OK) return st;
         }
     }
     if (cm) {
         const std::vector<uint64_t> mine(head.begin() + (size_t)rank0 * H, head.begin() + (size_t)(rank0 + 1) * H);
-        fq_status st = nccl_allgather_u64(ctx, cm, mine, &head);
+        st = nccl_allgather_u64(ctx0, cm, mine, &head);
         if (st != FQ_OK) return st;
     }
     for (uint32_t j = 1; j < n_shards; ++j)
-        if (head[(size_t)j * H] != head[0]) return fail(ctx, FQ_ERR_ARG, "fq_kmer_end_pass_all: k-mer rarefaction is enabled on some contexts only");
+        if (head[(size_t)j * H] != head[0]) return fail(ctx0, FQ_ERR_ARG, "fq_kmer_end_pass_all: k-mer rarefaction is enabled on some contexts only");
     if (!head[0]) return FQ_OK;
     for (uint32_t j = 1; j < n_shards; ++j) {
         const uint64_t *a = head.data(), *b = head.data() + (size_t)j * H;
@@ -1688,7 +1685,7 @@ fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
             snprintf(msg, sizeof msg, "fq_kmer_end_pass_all: context %u counts k = %llu, split_size = %llu, num_subsample = %llu; context 0 k = %llu, "
                      "split_size = %llu, num_subsample = %llu", j, (unsigned long long)b[1], (unsigned long long)b[2], (unsigned long long)b[3],
                      (unsigned long long)a[1], (unsigned long long)a[2], (unsigned long long)a[3]);
-            return fail(ctx, FQ_ERR_ARG, msg);
+            return fail(ctx0, FQ_ERR_ARG, msg);
         }
     }
     auto counts = [&](uint32_t from, uint32_t to) { return head[(size_t)from * H + 4 + to]; };
@@ -1696,26 +1693,22 @@ fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
     if (n_shards > 1) {
         std::vector<std::vector<uint64_t>> offsets(n);
         for (int i = 0; i < n; ++i) {
+            fq_ctx *const ctx = ctxs[i];
             const uint32_t me = rank0 + i;
             uint64_t incoming = 0, largest = 1;
             for (uint32_t j = 0; j < n_shards; ++j) {
                 incoming += counts(j, me);
                 if (j != me) largest = std::max(largest, counts(j, me));
             }
-            fq_status st = kmer_scatter(ctxs[i], n_shards, me, head.data() + (size_t)me * H + 4, incoming, &offsets[i]);
+            st = kmer_scatter(ctx, n_shards, me, head.data() + (size_t)me * H + 4, incoming, &offsets[i]);
             if (st != FQ_OK) return st;
-            fq_ctx *const c = ctxs[i];
-            fq_ctx *ctx = c;
-            CK(c->kmer.d_recv.ensure(largest * sizeof(KmerSlot)));
+            CK(ctx->kmer.d_recv.ensure(largest * sizeof(KmerSlot)));
         }
-        for (int i = 0; i < n; ++i) {           // every send buffer is complete before another context reads it
-            fq_ctx *ctx = ctxs[i];
-            CK(cudaSetDevice(ctx->device));
-            CK(cudaStreamSynchronize(ctx->stream));
-        }
+        st = sync_all(ctxs, n);                 // every send buffer is complete before another context reads it
+        if (st != FQ_OK) return st;
         for (uint32_t r = 1; r < n_shards; ++r) {
             for (int i = 0; i < n; ++i) {
-                fq_ctx *ctx = ctxs[i];
+                fq_ctx *const ctx = ctxs[i];
                 const uint32_t me = rank0 + i, dst = (me + r) % n_shards, src = (me + n_shards - r) % n_shards;
                 const uint64_t n_out = counts(me, dst), n_in = counts(src, me);
                 CK(cudaSetDevice(ctx->device));
@@ -1730,7 +1723,7 @@ fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
                     CK(cudaMemcpyPeerAsync(ctx->kmer.d_recv.p, ctx->device, from->kmer.d_send.as<KmerSlot>() + offsets[src][me], from->device,
                                            n_in * sizeof(KmerSlot), ctx->stream));
                 }
-                fq_status st = kmer_merge_received(ctx, n_in);
+                st = kmer_merge_received(ctx, n_in);
                 if (st != FQ_OK) return st;
             }
         }
@@ -1740,24 +1733,24 @@ fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
     std::vector<uint64_t> sum, flat;
     std::vector<uint32_t> big, part;
     for (int i = 0; i < n; ++i) {
-        fq_status st = kmer_summarize(ctxs[i], S, rank0 + i, &flat, cm ? nullptr : &part);
+        st = kmer_summarize(ctxs[i], S, rank0 + i, &flat, cm ? nullptr : &part);
         if (st != FQ_OK) return st;
         if (sum.empty()) sum.assign(S.total, 0);
         for (size_t k = 0; k < S.total; ++k) sum[k] += flat[k];
         big.insert(big.end(), part.begin(), part.end());
     }
     if (cm) {
-        fq_status st = nccl_sum_u64(ctx, cm, &sum);
+        st = nccl_sum_u64(ctx0, cm, &sum);
         if (st == FQ_OK) {
             for (uint32_t j = 0; j < n_shards; ++j)
-                if (sum[S.n_big + j] > kKmerBigCap) return fail(ctx, FQ_ERR_ARG, "k-mer rarefaction: more than 2^20 k-mers with counts above 65535");
-            st = nccl_gather_big(ctx, cm, sum.data() + S.n_big, &big);
+                if (sum[S.n_big + j] > kKmerBigCap) return fail(ctx0, FQ_ERR_ARG, "k-mer rarefaction: more than 2^20 k-mers with counts above 65535");
+            st = nccl_gather_big(ctx0, cm, sum.data() + S.n_big, &big);
         }
         if (st != FQ_OK) return st;
     }
     // 7. the pass's points and histogram, identically on every context
     for (int i = 0; i < n; ++i) {
-        fq_status st = kmer_finish(ctxs[i], S, n_shards, sum, big);
+        st = kmer_finish(ctxs[i], S, n_shards, sum, big);
         if (st != FQ_OK) return st;
     }
     return FQ_OK;
