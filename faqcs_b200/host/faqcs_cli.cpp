@@ -14,6 +14,7 @@
 #include <unistd.h>
 #include <zlib.h>
 
+#include "fork_join.hpp"
 #include "pgzip.hpp"
 
 #include <algorithm>
@@ -399,9 +400,9 @@ static size_t count_newlines(const uint8_t *buf, size_t n)
 }
 
 // ---- input: gz or plain, whole records per batch -------------------------------------------------
-// Plain files are read with read(2) straight into the pinned batch buffer; gzip input (magic 1f 8b) goes
-// through zlib like the reference's reader (fastq.cpp:8-30) -- except blocked gzip (BGZF: bgzip, bcl-convert, samtools),
-// whose members carry their compressed size in the header and are inflated by several threads at once.
+// Plain files are read with pread straight into the pinned batch buffer.  Gzip input (magic 1f 8b) is inflated by several
+// threads: blocked gzip (BGZF: bgzip, bcl-convert, samtools) member by member, as its members carry their compressed size in
+// the header, and ordinary gzip by entering the deflate stream at block boundaries (pgzip.hpp).
 static int g_input_files = 2;      // files read at the same time (two mates, or one file of unpaired reads)
 static int inflate_threads()      // per input file: the cores divided among the files, 2 .. 32
 {
@@ -423,72 +424,189 @@ static size_t bgzf_member_size(const uint8_t *p, size_t avail)
     return 0;
 }
 
+// pread until all n bytes are in; an I/O error or the end of the file before that is the reader's error
+static void pread_full(int fd, uint8_t *dst, size_t n, off_t at)
+{
+    for (size_t done = 0; done < n;) {
+        const ssize_t got = pread(fd, dst + done, n - done, at + (off_t)done);
+        if (got < 0 && errno == EINTR) continue;
+        if (got <= 0) throw "fastq.cpp:next_read: Unable to read header";
+        done += (size_t)got;
+    }
+}
+
 struct Source {
+    // Sliced: a regular plain file, read by kIoThreads threads into disjoint slices of the buffer (a single read(2) stream is
+    //   a single-core page-cache copy).
+    // Zlib: one zlib stream, as the reference reads every input (fastq.cpp:8-30): small or FAQCS_B200_PGZIP=0 gzip, and any
+    //   input that is not a regular file (pipes, process substitution, /dev/stdin), whose bytes cannot be read twice to sniff
+    //   the format; zlib passes plain text through.
+    // Bgzf, Pgzip: blocked and ordinary gzip, inflated by several threads.
+    enum class Mode { Sliced, Zlib, Bgzf, Pgzip };
+    Mode mode = Mode::Sliced;
+    bool bgzf = false, pgzip = false;     // open()'s choice, as reported by tests/host_io_harness.cpp (a Bgzf file may go on to Zlib)
     int fd = -1;
-    gzFile gz = nullptr;
     bool eof = false;
-    bool bgzf = false;
-    off_t cpos = 0, csize = 0;            // BGZF: next member, file size
-    vector<uint8_t> cbuf;                 // BGZF: compressed members of one fill
+    off_t pos = 0, size = 0;              // Sliced, Bgzf, Pgzip: the next byte of the file to read, the file size
+    vector<uint8_t> cbuf;                 // Bgzf, Pgzip: compressed bytes of one fill / round
+    gzFile gz = nullptr;                  // Zlib
+    struct {                              // Pgzip
+        bool in_member = false;
+        size_t bit = 0;                   // first undecoded bit of the member's deflate stream, relative to byte pos
+        size_t window_len = 0;            // valid bytes at the end of window (output of this member so far, at most 32 KiB)
+        vector<uint8_t> window;           // the last 32 KiB of output
+        deque<pgz::Bytes> pend;           // decoded pieces not yet handed out (the front one from pend_off on)
+        size_t pend_off = 0;
+        size_t span = 0;                  // compressed bytes looked at per round
+        size_t min_piece = 256u << 10;    // a thread gets at least this much compressed data
+        int solo_rounds = 0;              // rounds left in which no entry points are looked for
+        uint32_t crc = 0;
+        uint64_t isize = 0;
+    } pz;
     bool open(const string &fn)
     {
         fd = ::open(fn.c_str(), O_RDONLY);
         if (fd < 0) return false;
-        unsigned char head[64];
-        const ssize_t got = ::read(fd, head, sizeof(head));
-        lseek(fd, 0, SEEK_SET);
         struct stat st;
-        if (got >= 18 && bgzf_member_size(head, (size_t)got) && fstat(fd, &st) == 0 && S_ISREG(st.st_mode) && !getenv("FAQCS_B200_NO_BGZF")) {
-            bgzf = true;
-            csize = st.st_size;
-            return true;
-        }
-        if (got >= 2 && head[0] == 0x1f && head[1] == 0x8b) {
-            // ordinary gzip: several threads enter the deflate stream at block boundaries (pgzip.hpp); FAQCS_B200_PGZIP=0: one zlib stream
+        if (fstat(fd, &st) != 0 || !S_ISREG(st.st_mode)) return open_zlib();      // no sniffing: bytes read from a pipe are gone
+        size = st.st_size;
+        unsigned char head[64];
+        const ssize_t got = pread(fd, head, sizeof(head), 0);
+        if (got >= 18 && bgzf_member_size(head, (size_t)got) && !getenv("FAQCS_B200_NO_BGZF")) mode = Mode::Bgzf;
+        else if (got >= 2 && head[0] == 0x1f && head[1] == 0x8b) {
+            // FAQCS_B200_PGZIP=0: one zlib stream.  FAQCS_B200_PGZIP_MIN / _PIECE / _SPAN: smallest file, smallest piece,
+            // bytes per round (the tests shrink them)
             const char *e = getenv("FAQCS_B200_PGZIP");
-            // (FAQCS_B200_PGZIP_MIN / _PIECE / _SPAN: smallest file, smallest piece, bytes per round -- the tests shrink them)
             const char *m = getenv("FAQCS_B200_PGZIP_MIN"), *pc = getenv("FAQCS_B200_PGZIP_PIECE"), *sp = getenv("FAQCS_B200_PGZIP_SPAN");
-            if (pc) pz_min_piece = (size_t)strtoull(pc, nullptr, 10);
-            if (sp) pz_span = (size_t)strtoull(sp, nullptr, 10);
-            if (fstat(fd, &st) == 0 && S_ISREG(st.st_mode) && st.st_size >= (off_t)(m ? strtoull(m, nullptr, 10) : (4u << 20)) && !(e && e[0] == '0')) {
-                pgzip = true;
-                csize = st.st_size;
-                pz_window.assign(pgz::kWin, 0);
-                return true;
-            }
-            return open_zlib();
+            if (size < (off_t)(m ? strtoull(m, nullptr, 10) : (4u << 20)) || (e && e[0] == '0')) return open_zlib();
+            if (pc) pz.min_piece = (size_t)strtoull(pc, nullptr, 10);
+            if (sp) pz.span = (size_t)strtoull(sp, nullptr, 10);
+            pz.window.assign(pgz::kWin, 0);
+            mode = Mode::Pgzip;
         }
-        detect_sliced();
+        bgzf = mode == Mode::Bgzf;
+        pgzip = mode == Mode::Pgzip;
         return true;
     }
-    // ---- ordinary gzip, inflated by several threads (pgzip.hpp) ----
-    bool pgzip = false, pz_in_member = false;
-    size_t pz_bit = 0;                    // first undecoded bit of the member's deflate stream, relative to byte cpos
-    size_t pz_window_len = 0;             // valid bytes at the end of pz_window (output of this member so far, at most 32 KiB)
-    vector<uint8_t> pz_window;            // the last 32 KiB of output
-    deque<pgz::Bytes> pz_pend;            // decoded pieces not yet handed out (the front one from pz_pend_off on)
-    size_t pz_pend_off = 0;
-    size_t pz_span = 0;                   // compressed bytes looked at per round
-    size_t pz_min_piece = 256u << 10;     // a thread gets at least this much compressed data
-    int pz_solo_rounds = 0;               // rounds left in which no entry points are looked for
-    uint32_t pz_crc = 0;
-    uint64_t pz_isize = 0;
-    void pz_read(size_t want)
+    bool open_zlib()
+    {
+        mode = Mode::Zlib;
+        gz = gzdopen(fd, "r");
+        if (!gz) return false;
+        gzbuffer(gz, 1 << 20);
+        return true;
+    }
+    void close()
+    {
+        if (gz) gzclose(gz);
+        else if (fd >= 0) ::close(fd);
+        gz = nullptr;
+        fd = -1;
+    }
+    // append to buf[have..cap); returns the bytes now in buf and the newlines in the appended part
+    size_t fill(uint8_t *buf, size_t have, size_t cap, size_t *new_lines)
+    {
+        switch (mode) {
+            case Mode::Sliced: return fill_sliced(buf, have, cap, new_lines);
+            case Mode::Zlib: return fill_zlib(buf, have, cap, new_lines);
+            case Mode::Bgzf: return fill_bgzf(buf, have, cap, new_lines);
+            case Mode::Pgzip: return fill_pgzip(buf, have, cap, new_lines);
+        }
+        return have;
+    }
+    size_t fill_sliced(uint8_t *buf, size_t have, size_t cap, size_t *new_lines)
+    {
+        const size_t want = (size_t)min<off_t>((off_t)(cap - have), size - pos);
+        const int nt = want >= io_slice_min() && want >= (size_t)kIoThreads ? kIoThreads : 1;
+        const size_t per = (want + nt - 1) / nt;
+        vector<size_t> lines(nt, 0);
+        fork_join(nt, [&](int t) {
+            const size_t lo = min(want, per * t), hi = min(want, per * (t + 1));
+            pread_full(fd, buf + have + lo, hi - lo, pos + (off_t)lo);       // the file shrank, or an I/O error: throws
+            lines[t] = count_newlines(buf + have + lo, hi - lo);
+        });
+        for (size_t l : lines) *new_lines += l;
+        pos += (off_t)want;
+        if (pos >= size) eof = true;
+        return have + want;
+    }
+    size_t fill_zlib(uint8_t *buf, size_t have, size_t cap, size_t *new_lines)
+    {
+        size_t n = have;
+        while (!eof && n < cap) {
+            const int got = gzread(gz, buf + n, (unsigned)min<size_t>(cap - n, 1u << 30));
+            if (got < 0) throw "fastq.cpp:next_read: Unable to read header";
+            if (got == 0) eof = true;
+            n += (size_t)got;
+        }
+        *new_lines += count_newlines(buf + have, n - have);
+        return n;
+    }
+    void read_cbuf(size_t want)
     {
         cbuf.resize(want);
-        for (size_t done = 0; done < want;) {
-            const ssize_t got = pread(fd, cbuf.data() + done, want - done, cpos + (off_t)done);
-            if (got < 0 && errno == EINTR) continue;
-            if (got <= 0) throw "fastq.cpp:next_read: Unable to read header";
-            done += (size_t)got;
-        }
+        pread_full(fd, cbuf.data(), want, pos);
     }
-    // the header of the member at cpos (RFC 1952); false: no further member (end of file, or bytes that are not gzip: ignored as gzread does)
+    // BGZF: members up to the buffer's capacity, inflated by inflate_threads() threads into their places.  Anything that is
+    // not a BGZF member (plain gzip members appended to the file) hands the rest of the file to zlib.
+    size_t fill_bgzf(uint8_t *buf, size_t have, size_t cap, size_t *new_lines)
+    {
+        struct Member { size_t in, in_len, out, out_len; uint32_t crc; };
+        vector<Member> members;
+        size_t n = have;
+        const size_t want = (size_t)min<off_t>(size - pos, (off_t)(cap - have) + (1 << 16));
+        read_cbuf(want);
+        size_t p = 0;
+        bool to_zlib = false;
+        while (p < want) {
+            const size_t msize = bgzf_member_size(cbuf.data() + p, want - p);
+            if (msize == 0) { to_zlib = want - p >= 18 || pos + (off_t)want >= size; break; }   // not BGZF (or a cut header: next fill)
+            if (p + msize > want) break;                                                        // cut member: next fill
+            const uint8_t *m = cbuf.data() + p;
+            const size_t hdr = 12 + (m[10] | (size_t)m[11] << 8);
+            if (msize < hdr + 8) throw "corrupt BGZF member";
+            const uint32_t crc = m[msize - 8] | (uint32_t)m[msize - 7] << 8 | (uint32_t)m[msize - 6] << 16 | (uint32_t)m[msize - 5] << 24;
+            const size_t isize = m[msize - 4] | (size_t)m[msize - 3] << 8 | (size_t)m[msize - 2] << 16 | (size_t)m[msize - 1] << 24;
+            if (n + isize > cap) break;
+            members.push_back(Member{p + hdr, msize - hdr - 8, n, isize, crc});
+            n += isize;
+            p += msize;
+        }
+        const int nt = (int)max<size_t>(1, min<size_t>((size_t)inflate_threads(), members.size() / 4));
+        vector<size_t> lines(nt, 0);
+        fork_join(nt, [&](int t) {
+            z_stream zs{};
+            if (inflateInit2(&zs, -15) != Z_OK) throw "fastq.cpp:next_read: Unable to read header";
+            const size_t lo = members.size() * t / nt, hi = members.size() * (t + 1) / nt;
+            bool ok = true;
+            for (size_t k = lo; ok && k < hi; ++k) {
+                const Member &mb = members[k];
+                zs.next_in = cbuf.data() + mb.in; zs.avail_in = (uInt)mb.in_len;
+                zs.next_out = buf + mb.out; zs.avail_out = (uInt)mb.out_len;
+                const int rc = mb.out_len || mb.in_len ? inflate(&zs, Z_FINISH) : Z_STREAM_END;
+                ok = rc == Z_STREAM_END && zs.avail_out == 0 && (uint32_t)crc32(crc32(0L, Z_NULL, 0), buf + mb.out, (uInt)mb.out_len) == mb.crc;
+                inflateReset(&zs);
+            }
+            inflateEnd(&zs);
+            if (!ok) throw "fastq.cpp:next_read: Unable to read header";       // what a failed gzgets turns into
+            if (hi > lo) lines[t] = count_newlines(buf + members[lo].out, members[hi - 1].out + members[hi - 1].out_len - members[lo].out);
+        });
+        for (size_t l : lines) *new_lines += l;
+        pos += (off_t)p;
+        if (pos >= size) eof = true;
+        if (to_zlib) {                       // the rest of the file through zlib, from this member on
+            if (lseek(fd, pos, SEEK_SET) < 0 || !open_zlib()) throw "fastq.cpp:next_read: Unable to read header";
+            if (n < cap) return fill_zlib(buf, n, cap, new_lines);
+        }
+        return n;
+    }
+    // ---- ordinary gzip, inflated by several threads (pgzip.hpp) ----
+    // the header of the member at pos (RFC 1952); false: no further member (end of file, or bytes that are not gzip: ignored as gzread does)
     bool pz_member_header()
     {
-        const size_t want = (size_t)min<off_t>(csize - cpos, 1 << 16);
+        const size_t want = (size_t)min<off_t>(size - pos, 1 << 16);
         if (want < 18) return false;
-        pz_read(want);
+        read_cbuf(want);
         const uint8_t *h = cbuf.data();
         if (h[0] != 0x1f || h[1] != 0x8b) return false;
         if (h[2] != 8 || (h[3] & 0xe0)) throw "fastq.cpp:next_read: Unable to read header";
@@ -498,77 +616,72 @@ struct Source {
         if (h[3] & 16) { while (p < want && h[p]) ++p; ++p; }
         if (h[3] & 2) p += 2;
         if (p >= want) throw "fastq.cpp:next_read: Unable to read header";
-        cpos += (off_t)p;
-        pz_bit = 0;
-        pz_window_len = 0;
-        pz_crc = (uint32_t)crc32(0L, Z_NULL, 0);
-        pz_isize = 0;
-        pz_in_member = true;
+        pos += (off_t)p;
+        pz.bit = 0;
+        pz.window_len = 0;
+        pz.crc = (uint32_t)crc32(0L, Z_NULL, 0);
+        pz.isize = 0;
+        pz.in_member = true;
         return true;
     }
-    // one round: more decoded bytes into pz_pend (or eof)
+    // one round: more decoded bytes into pz.pend (or eof)
     void pz_produce()
     {
-        if (!pz_in_member && (cpos >= csize || !pz_member_header())) { eof = true; return; }
+        if (!pz.in_member && (pos >= size || !pz_member_header())) { eof = true; return; }
         const int threads = inflate_threads();
-        if (!pz_span) pz_span = max<size_t>((size_t)threads * (2u << 20), 8u << 20);
+        if (!pz.span) pz.span = max<size_t>((size_t)threads * (2u << 20), 8u << 20);
         for (;;) {
-            const size_t want = (size_t)min<off_t>(csize - cpos, (off_t)pz_span);
-            pz_read(want);
+            const size_t want = (size_t)min<off_t>(size - pos, (off_t)pz.span);
+            read_cbuf(want);
             // a stream without entry points (stored or fixed blocks, blocks larger than a piece) is left to one thread for a few
             // rounds instead of being searched again and again
-            const int use = pz_solo_rounds > 0 ? 1 : threads;
-            if (pz_solo_rounds > 0) --pz_solo_rounds;
-            pgz::Result R = pgz::inflate_parallel(cbuf.data(), want, pz_bit, pz_window, pz_window_len, use, pz_min_piece);
-            if (use > 1 && R.pieces.size() == 1 && !R.error) pz_solo_rounds = 8;
+            const int use = pz.solo_rounds > 0 ? 1 : threads;
+            if (pz.solo_rounds > 0) --pz.solo_rounds;
+            pgz::Result R = pgz::inflate_parallel(cbuf.data(), want, pz.bit, pz.window, pz.window_len, use, pz.min_piece);
+            if (use > 1 && R.pieces.size() == 1 && !R.error) pz.solo_rounds = 8;
             if (R.error) throw "fastq.cpp:next_read: Unable to read header";
             size_t total = 0;
             for (const pgz::Piece &pc : R.pieces) total += pc.out.size();
             if (total == 0 && !R.stream_end) {
                 // not one whole block in this span: look at more of the file -- or the file is cut short: what one zlib stream
                 // still gets out of it is handed out and the input ends there, as it does for gzread / gzgets (fastq.cpp:8-30)
-                if ((off_t)want >= csize - cpos) {
+                if ((off_t)want >= size - pos) {
                     pgz::Bytes tail;
-                    if (!pgz::inflate_truncated_tail(cbuf.data(), want, pz_bit, pz_window.data() + (pgz::kWin - pz_window_len), pz_window_len, tail))
+                    if (!pgz::inflate_truncated_tail(cbuf.data(), want, pz.bit, pz.window.data() + (pgz::kWin - pz.window_len), pz.window_len, tail))
                         throw "fastq.cpp:next_read: Unable to read header";
-                    if (tail.size()) pz_pend.push_back(std::move(tail));
-                    cpos = csize;
-                    pz_in_member = false;
+                    if (tail.size()) pz.pend.push_back(std::move(tail));
+                    pos = size;
+                    pz.in_member = false;
                     return;
                 }
-                pz_span *= 2;
+                pz.span *= 2;
                 continue;
             }
             // CRC-32 of the pieces in parallel, combined in order (RFC 1952 trailer)
             vector<uint32_t> crcs(R.pieces.size());
-            {
-                vector<thread> th;
-                for (size_t q = 0; q < R.pieces.size(); ++q)
-                    th.emplace_back([&, q] {
-                        uLong c = crc32(0L, Z_NULL, 0);
-                        const pgz::Bytes &o = R.pieces[q].out;
-                        for (size_t at = 0; at < o.size(); at += 1u << 30) c = crc32(c, o.data() + at, (uInt)min<size_t>(o.size() - at, 1u << 30));
-                        crcs[q] = (uint32_t)c;
-                    });
-                for (thread &x : th) x.join();
-            }
+            fork_join((int)R.pieces.size(), [&](int q) {
+                uLong c = crc32(0L, Z_NULL, 0);
+                const pgz::Bytes &o = R.pieces[q].out;
+                for (size_t at = 0; at < o.size(); at += 1u << 30) c = crc32(c, o.data() + at, (uInt)min<size_t>(o.size() - at, 1u << 30));
+                crcs[q] = (uint32_t)c;
+            });
             for (size_t q = 0; q < R.pieces.size(); ++q) {
-                pz_crc = (uint32_t)crc32_combine(pz_crc, crcs[q], (z_off_t)R.pieces[q].out.size());
-                if (R.pieces[q].out.size()) pz_pend.push_back(std::move(R.pieces[q].out));
+                pz.crc = (uint32_t)crc32_combine(pz.crc, crcs[q], (z_off_t)R.pieces[q].out.size());
+                if (R.pieces[q].out.size()) pz.pend.push_back(std::move(R.pieces[q].out));
             }
-            pz_isize += total;
-            pz_window_len = min(pgz::kWin, pz_window_len + total);
-            cpos += (off_t)(R.end_bit >> 3);
-            pz_bit = R.end_bit & 7;
+            pz.isize += total;
+            pz.window_len = min(pgz::kWin, pz.window_len + total);
+            pos += (off_t)(R.end_bit >> 3);
+            pz.bit = R.end_bit & 7;
             if (R.stream_end) {
-                if (csize - cpos < 8) { cpos = csize; pz_in_member = false; return; }      // the file ends inside the trailer: cut short, as above
+                if (size - pos < 8) { pos = size; pz.in_member = false; return; }      // the file ends inside the trailer: cut short, as above
                 uint8_t t[8];
-                if (pread(fd, t, 8, cpos) != 8) throw "fastq.cpp:next_read: Unable to read header";
+                pread_full(fd, t, 8, pos);
                 const uint32_t crc = t[0] | (uint32_t)t[1] << 8 | (uint32_t)t[2] << 16 | (uint32_t)t[3] << 24;
                 const uint32_t isz = t[4] | (uint32_t)t[5] << 8 | (uint32_t)t[6] << 16 | (uint32_t)t[7] << 24;
-                if (crc != pz_crc || isz != (uint32_t)pz_isize) throw "fastq.cpp:next_read: Unable to read header";
-                cpos += 8;
-                pz_in_member = false;
+                if (crc != pz.crc || isz != (uint32_t)pz.isize) throw "fastq.cpp:next_read: Unable to read header";
+                pos += 8;
+                pz.in_member = false;
             }
             return;
         }
@@ -577,158 +690,17 @@ struct Source {
     {
         size_t n = have;
         while (n < cap) {
-            if (pz_pend.empty()) {
+            if (pz.pend.empty()) {
                 if (eof) break;
                 pz_produce();           // sets eof when the file holds no further member
                 continue;
             }
-            const pgz::Bytes &front = pz_pend.front();
-            const size_t take = min(cap - n, front.size() - pz_pend_off);
-            memcpy(buf + n, front.data() + pz_pend_off, take);
-            pz_pend_off += take;
+            const pgz::Bytes &front = pz.pend.front();
+            const size_t take = min(cap - n, front.size() - pz.pend_off);
+            memcpy(buf + n, front.data() + pz.pend_off, take);
+            pz.pend_off += take;
             n += take;
-            if (pz_pend_off == front.size()) { pz_pend.pop_front(); pz_pend_off = 0; }
-        }
-        *new_lines += count_newlines(buf + have, n - have);
-        return n;
-    }
-    bool open_zlib()
-    {
-        gz = gzdopen(fd, "r");
-        if (!gz) return false;
-        gzbuffer(gz, 1 << 20);
-        return true;
-    }
-    // BGZF: members up to the buffer's capacity, inflated by inflate_threads() threads into their places.  Anything that is
-    // not a BGZF member (plain gzip members appended to the file) hands the rest of the file to zlib.
-    size_t fill_bgzf(uint8_t *buf, size_t have, size_t cap, size_t *new_lines)
-    {
-        struct Member { size_t in, in_len, out, out_len; uint32_t crc; };
-        vector<Member> members;
-        size_t n = have;
-        const size_t want = (size_t)min<off_t>(csize - cpos, (off_t)(cap - have) + (1 << 16));
-        cbuf.resize(want);
-        for (size_t done = 0; done < want;) {
-            const ssize_t got = pread(fd, cbuf.data() + done, want - done, cpos + (off_t)done);
-            if (got < 0 && errno == EINTR) continue;
-            if (got <= 0) throw "fastq.cpp:next_read: Unable to read header";
-            done += (size_t)got;
-        }
-        size_t p = 0;
-        bool to_zlib = false;
-        while (p < want) {
-            const size_t size = bgzf_member_size(cbuf.data() + p, want - p);
-            if (size == 0) { to_zlib = want - p >= 18 || cpos + (off_t)want >= csize; break; }   // not BGZF (or a cut header: next fill)
-            if (p + size > want) break;                                                          // cut member: next fill
-            const uint8_t *m = cbuf.data() + p;
-            const size_t hdr = 12 + (m[10] | (size_t)m[11] << 8);
-            if (size < hdr + 8) throw "corrupt BGZF member";
-            const uint32_t crc = m[size - 8] | (uint32_t)m[size - 7] << 8 | (uint32_t)m[size - 6] << 16 | (uint32_t)m[size - 5] << 24;
-            const size_t isize = m[size - 4] | (size_t)m[size - 3] << 8 | (size_t)m[size - 2] << 16 | (size_t)m[size - 1] << 24;
-            if (n + isize > cap) break;
-            members.push_back(Member{p + hdr, size - hdr - 8, n, isize, crc});
-            n += isize;
-            p += size;
-        }
-        const int nt = (int)max<size_t>(1, min<size_t>((size_t)inflate_threads(), members.size() / 4));
-        vector<size_t> lines(nt, 0);
-        vector<int> bad(nt, 0);
-        vector<thread> th;
-        for (int t = 0; t < nt; ++t) {
-            auto job = [&, t] {
-                z_stream zs{};
-                if (inflateInit2(&zs, -15) != Z_OK) { bad[t] = 1; return; }
-                const size_t lo = members.size() * t / nt, hi = members.size() * (t + 1) / nt;
-                for (size_t k = lo; k < hi; ++k) {
-                    const Member &mb = members[k];
-                    zs.next_in = cbuf.data() + mb.in; zs.avail_in = (uInt)mb.in_len;
-                    zs.next_out = buf + mb.out; zs.avail_out = (uInt)mb.out_len;
-                    const int rc = mb.out_len || mb.in_len ? inflate(&zs, Z_FINISH) : Z_STREAM_END;
-                    if (rc != Z_STREAM_END || zs.avail_out != 0 || (uint32_t)crc32(crc32(0L, Z_NULL, 0), buf + mb.out, (uInt)mb.out_len) != mb.crc) { bad[t] = 1; break; }
-                    inflateReset(&zs);
-                }
-                inflateEnd(&zs);
-                if (hi > lo) lines[t] = count_newlines(buf + members[lo].out, members[hi - 1].out + members[hi - 1].out_len - members[lo].out);
-            };
-            if (t + 1 < nt) th.emplace_back(job); else job();
-        }
-        for (thread &x : th) x.join();
-        for (int t = 0; t < nt; ++t) {
-            if (bad[t]) throw "fastq.cpp:next_read: Unable to read header";       // what a failed gzgets turns into
-            *new_lines += lines[t];
-        }
-        cpos += (off_t)p;
-        if (cpos >= csize) eof = true;
-        if (to_zlib) {                       // the rest of the file through zlib, from this member on
-            bgzf = false;
-            lseek(fd, cpos, SEEK_SET);
-            if (!open_zlib()) throw "fastq.cpp:next_read: Unable to read header";
-            if (n < cap) return fill(buf, n, cap, new_lines);
-        }
-        return n;
-    }
-    void close()
-    {
-        if (gz) gzclose(gz);
-        else if (fd >= 0) ::close(fd);
-        gz = nullptr;
-        fd = -1;
-    }
-    // Regular plain file: the byte range of a batch is known up front, so it is read by kIoThreads threads with
-    // pread into disjoint slices of the buffer (a single read(2) stream is a single-core page-cache copy).
-    bool sliced = false;
-    off_t pos = 0, size = 0;
-    void detect_sliced()
-    {
-        struct stat st;
-        if (!gz && fstat(fd, &st) == 0 && S_ISREG(st.st_mode)) { sliced = true; size = st.st_size; pos = 0; }
-    }
-    // append to buf[have..cap); returns the bytes now in buf and the newlines in the appended part
-    size_t fill(uint8_t *buf, size_t have, size_t cap, size_t *new_lines)
-    {
-        size_t n = have;
-        if (bgzf) return fill_bgzf(buf, have, cap, new_lines);
-        if (pgzip) return fill_pgzip(buf, have, cap, new_lines);
-        if (sliced) {
-            const size_t want = (size_t)min<off_t>((off_t)(cap - have), size - pos);
-            const int nt = want >= io_slice_min() && want >= (size_t)kIoThreads ? kIoThreads : 1;
-            const size_t per = (want + nt - 1) / nt;
-            vector<thread> th;
-            vector<size_t> lines(nt, 0);
-            vector<int> bad(nt, 0);
-            for (int t = 0; t < nt; ++t) {
-                const size_t lo = min(want, per * t), hi = min(want, per * (t + 1));
-                auto job = [this, buf, have, lo, hi, t, &lines, &bad] {
-                    size_t done = lo;
-                    while (done < hi) {
-                        const ssize_t got = pread(fd, buf + have + done, hi - done, pos + (off_t)done);
-                        if (got < 0 && errno == EINTR) continue;
-                        if (got <= 0) { bad[t] = 1; return; }       // the file shrank or an I/O error
-                        done += (size_t)got;
-                    }
-                    lines[t] = count_newlines(buf + have + lo, hi - lo);
-                };
-                if (t + 1 < nt) th.emplace_back(job); else job();
-            }
-            for (thread &x : th) x.join();
-            for (int t = 0; t < nt; ++t) {
-                if (bad[t]) throw "fastq.cpp:next_read: Unable to read header";
-                *new_lines += lines[t];
-            }
-            pos += (off_t)want;
-            n += want;
-            if (pos >= size) eof = true;
-            return n;
-        }
-        while (!eof && n < cap) {
-            const size_t want = min<size_t>(cap - n, 1u << 30);
-            const ssize_t got = gz ? (ssize_t)gzread(gz, buf + n, (unsigned)want) : ::read(fd, buf + n, want);
-            if (got < 0) {
-                if (!gz && errno == EINTR) continue;
-                throw "fastq.cpp:next_read: Unable to read header";
-            }
-            if (got == 0) { eof = true; break; }
-            n += (size_t)got;
+            if (pz.pend_off == front.size()) { pz.pend.pop_front(); pz.pend_off = 0; }
         }
         *new_lines += count_newlines(buf + have, n - have);
         return n;
@@ -792,8 +764,7 @@ struct Run {
 static int open_out(const string &fn, const char *what, bool append = false)
 {
     const int fd = ::open(fn.c_str(), O_RDWR | O_CREAT | (append ? 0 : O_TRUNC), 0666);      // O_RDWR: shared mappings need read access
-    if (fd >= 0 && append) lseek(fd, 0, SEEK_END);
-    if (fd < 0) { cerr << "Unable to open " << fn << " for writing " << what << endl; throw "I/O error"; }
+    if (fd < 0 || (append && lseek(fd, 0, SEEK_END) < 0 && errno != ESPIPE)) { cerr << "Unable to open " << fn << " for writing " << what << endl; throw "I/O error"; }
     return fd;
 }
 static void write_all(int fd, const uint8_t *p, size_t n)
@@ -836,24 +807,13 @@ static void write_bgzf(int fd, const uint8_t *p, size_t n)
     const size_t blocks = (n + kBlock - 1) / kBlock;
     const int nt = (int)max<size_t>(1, min<size_t>((size_t)inflate_threads(), blocks / 8));      // deflate is the slow side: as many threads as the readers get
     vector<vector<uint8_t>> part(nt);
-    vector<int> bad(nt, 0);
-    vector<thread> th;
-    for (int t = 0; t < nt; ++t) {
-        auto job = [&, t] {
-            z_stream zs{};
-            if (deflateInit2(&zs, 4, Z_DEFLATED, -15, 8, Z_DEFAULT_STRATEGY) != Z_OK) { bad[t] = 1; return; }
-            try {
-                for (size_t b = blocks * t / nt; b < blocks * (t + 1) / nt; ++b) bgzf_member(part[t], zs, p + b * kBlock, min(kBlock, n - b * kBlock));
-            } catch (...) { bad[t] = 1; }
-            deflateEnd(&zs);
-        };
-        if (t + 1 < nt) th.emplace_back(job); else job();
-    }
-    for (thread &x : th) x.join();
-    for (int t = 0; t < nt; ++t) {
-        if (bad[t]) throw "I/O error while compressing the trimmed reads";
-        write_all(fd, part[t].data(), part[t].size());
-    }
+    fork_join(nt, [&](int t) {
+        z_stream zs{};
+        if (deflateInit2(&zs, 4, Z_DEFLATED, -15, 8, Z_DEFAULT_STRATEGY) != Z_OK) throw "I/O error while compressing the trimmed reads";
+        const unique_ptr<z_stream, int (*)(z_streamp)> end(&zs, deflateEnd);
+        for (size_t b = blocks * t / nt; b < blocks * (t + 1) / nt; ++b) bgzf_member(part[t], zs, p + b * kBlock, min(kBlock, n - b * kBlock));
+    });
+    for (const vector<uint8_t> &b : part) write_all(fd, b.data(), b.size());
 }
 static void close_bgzf(int fd)
 {
@@ -863,33 +823,48 @@ static void close_bgzf(int fd)
 
 // Large appends to a regular file: reserve the range (posix_fallocate reports a full disk as an error instead of a
 // SIGBUS later), map it and let kIoThreads threads copy disjoint slices -- write(2) calls on one file serialise on its
-// inode lock, page faults into a shared mapping do not.  Anything unusual falls back to write(2).
+// inode lock, page faults into a shared mapping do not.  dst stays null when the file cannot be mapped (not a regular file,
+// the position not at its end, no room, mmap refused); the caller then writes with write(2).
+struct AppendMap {
+    uint8_t *dst = nullptr;
+    void *m = MAP_FAILED;
+    size_t len = 0;
+    off_t end = 0;
+    AppendMap(int fd, size_t n)
+    {
+        struct stat st;
+        const off_t base = lseek(fd, 0, SEEK_CUR);
+        if (base < 0 || fstat(fd, &st) != 0 || !S_ISREG(st.st_mode) || st.st_size != base || posix_fallocate(fd, base, (off_t)n) != 0) return;
+        const long page = sysconf(_SC_PAGESIZE);
+        const off_t map_off = base / page * page;
+        len = (size_t)(base - map_off) + n;
+        end = base + (off_t)n;
+        m = mmap(nullptr, len, PROT_READ | PROT_WRITE, MAP_SHARED, fd, map_off);
+        if (m != MAP_FAILED) dst = (uint8_t *)m + (base - map_off);
+        else if (ftruncate(fd, base) != 0) throw "I/O error while writing the trimmed reads";
+    }
+    AppendMap(const AppendMap &) = delete;
+    AppendMap &operator=(const AppendMap &) = delete;
+    ~AppendMap() { if (m != MAP_FAILED) munmap(m, len); }
+    // all n bytes are in place: the next write goes after them
+    void finish(int fd) const { if (lseek(fd, end, SEEK_SET) < 0) throw "I/O error while writing the trimmed reads"; }
+};
+
 static void write_mapped(int fd, const uint8_t *p, size_t n)
 {
-    struct stat st;
-    const off_t base = lseek(fd, 0, SEEK_CUR);
-    if (n < io_slice_min() || n < (size_t)kIoThreads || base < 0 || fstat(fd, &st) != 0 || !S_ISREG(st.st_mode) || st.st_size != base) { write_all(fd, p, n); return; }
-    if (posix_fallocate(fd, base, (off_t)n) != 0) { write_all(fd, p, n); return; }
-    const long page = sysconf(_SC_PAGESIZE);
-    const off_t map_off = base / page * page;
-    const size_t lead = (size_t)(base - map_off), map_len = lead + n;
-    void *m = mmap(nullptr, map_len, PROT_READ | PROT_WRITE, MAP_SHARED, fd, map_off);
-    if (m == MAP_FAILED) {
-        if (ftruncate(fd, base) != 0) throw "I/O error while writing the trimmed reads";
-        write_all(fd, p, n);
-        return;
+    if (n >= io_slice_min() && n >= (size_t)kIoThreads) {
+        AppendMap a(fd, n);
+        if (a.dst) {
+            const size_t per = (n + kIoThreads - 1) / kIoThreads;
+            fork_join(kIoThreads, [&](int t) {
+                const size_t lo = min(n, per * t), hi = min(n, per * (t + 1));
+                memcpy(a.dst + lo, p + lo, hi - lo);
+            });
+            a.finish(fd);
+            return;
+        }
     }
-    uint8_t *dst = (uint8_t *)m + lead;
-    const size_t per = (n + kIoThreads - 1) / kIoThreads;
-    vector<thread> th;
-    for (int t = 0; t < kIoThreads; ++t) {
-        const size_t lo = min(n, per * t), hi = min(n, per * (t + 1));
-        auto job = [dst, p, lo, hi] { memcpy(dst + lo, p + lo, hi - lo); };
-        if (t + 1 < kIoThreads) th.emplace_back(job); else job();
-    }
-    for (thread &x : th) x.join();
-    munmap(m, map_len);
-    lseek(fd, base + (off_t)n, SEEK_SET);
+    write_all(fd, p, n);
 }
 
 // Pieces mode (fq_set_output_pieces): a stream of one batch is a list of pieces of the batch's own input buffers plus the
@@ -898,75 +873,46 @@ static void write_mapped(int fd, const uint8_t *p, size_t n)
 static void write_pieces(int fd, const fq_out_piece *pc, size_t n_pc, const uint8_t *const src[3], size_t total)
 {
     if (total == 0) return;
-    struct stat st;
-    const off_t base = lseek(fd, 0, SEEK_CUR);
-    const bool mappable = base >= 0 && fstat(fd, &st) == 0 && S_ISREG(st.st_mode) && st.st_size == base && total >= (size_t)kIoThreads &&
-                          posix_fallocate(fd, base, (off_t)total) == 0;
-    uint8_t *dst = nullptr;
-    void *m = MAP_FAILED;
-    size_t map_len = 0;
-    if (mappable) {
-        const long page = sysconf(_SC_PAGESIZE);
-        const off_t map_off = base / page * page;
-        map_len = (size_t)(base - map_off) + total;
-        m = mmap(nullptr, map_len, PROT_READ | PROT_WRITE, MAP_SHARED, fd, map_off);
-        if (m == MAP_FAILED) { if (ftruncate(fd, base) != 0) throw "I/O error while writing the trimmed reads"; }
-        else dst = (uint8_t *)m + (base - map_off);
-    }
-    if (!dst) {                                   // pipes, odd files: gather the pieces with writev
-        vector<iovec> iov;
-        iov.reserve(1024);
-        auto flush = [&] {
-            size_t done = 0;
-            while (done < iov.size()) {
-                ssize_t w = writev(fd, iov.data() + done, (int)min<size_t>(iov.size() - done, 1024));
-                if (w < 0) { if (errno == EINTR) continue; throw "I/O error while writing the trimmed reads"; }
-                while (w > 0 && done < iov.size()) {
-                    if ((size_t)w >= iov[done].iov_len) { w -= (ssize_t)iov[done].iov_len; ++done; }
-                    else { iov[done].iov_base = (uint8_t *)iov[done].iov_base + w; iov[done].iov_len -= (size_t)w; w = 0; }
-                }
-            }
-            iov.clear();
-        };
-        for (size_t k = 0; k < n_pc; ++k) {
-            if (pc[k].source > 2) throw "pieces of a stream do not add up to its size";
-            iov.push_back(iovec{(void *)(src[pc[k].source] + pc[k].offset), pc[k].length});
-            if (iov.size() == 1024) flush();
-        }
-        flush();
-        return;
-    }
-    const int nt = kIoThreads;
-    size_t part_bytes[kIoThreads] = {0};
-    {
-        vector<thread> th;
-        for (int t = 0; t < nt; ++t) {
-            auto job = [&, t] {
+    if (total >= (size_t)kIoThreads) {
+        AppendMap a(fd, total);
+        if (a.dst) {
+            const int nt = kIoThreads;
+            size_t start[kIoThreads + 1] = {0};
+            fork_join(nt, [&](int t) {
                 size_t b = 0;
                 for (size_t k = n_pc * t / nt; k < n_pc * (t + 1) / nt; ++k) b += pc[k].source < 3 ? pc[k].length : total + 1;     // unknown source: fail below
-                part_bytes[t] = b;
-            };
-            if (t + 1 < nt) th.emplace_back(job); else job();
-        }
-        for (thread &x : th) x.join();
-    }
-    size_t start[kIoThreads + 1] = {0};
-    for (int t = 0; t < nt; ++t) start[t + 1] = start[t] + part_bytes[t];
-    const bool consistent = start[nt] == total;
-    if (consistent) {
-        vector<thread> th;
-        for (int t = 0; t < nt; ++t) {
-            auto job = [&, t] {
-                uint8_t *d = dst + start[t];
+                start[t + 1] = b;
+            });
+            for (int t = 0; t < nt; ++t) start[t + 1] += start[t];
+            if (start[nt] != total) throw "pieces of a stream do not add up to its size";
+            fork_join(nt, [&](int t) {
+                uint8_t *d = a.dst + start[t];
                 for (size_t k = n_pc * t / nt; k < n_pc * (t + 1) / nt; ++k) { memcpy(d, src[pc[k].source] + pc[k].offset, pc[k].length); d += pc[k].length; }
-            };
-            if (t + 1 < nt) th.emplace_back(job); else job();
+            });
+            a.finish(fd);
+            return;
         }
-        for (thread &x : th) x.join();
     }
-    munmap(m, map_len);
-    if (!consistent) throw "pieces of a stream do not add up to its size";
-    lseek(fd, base + (off_t)total, SEEK_SET);
+    vector<iovec> iov;                                // pipes, odd files: gather the pieces with writev
+    iov.reserve(1024);
+    auto flush = [&] {
+        size_t done = 0;
+        while (done < iov.size()) {
+            ssize_t w = writev(fd, iov.data() + done, (int)min<size_t>(iov.size() - done, 1024));
+            if (w < 0) { if (errno == EINTR) continue; throw "I/O error while writing the trimmed reads"; }
+            while (w > 0 && done < iov.size()) {
+                if ((size_t)w >= iov[done].iov_len) { w -= (ssize_t)iov[done].iov_len; ++done; }
+                else { iov[done].iov_base = (uint8_t *)iov[done].iov_base + w; iov[done].iov_len -= (size_t)w; w = 0; }
+            }
+        }
+        iov.clear();
+    };
+    for (size_t k = 0; k < n_pc; ++k) {
+        if (pc[k].source > 2) throw "pieces of a stream do not add up to its size";
+        iov.push_back(iovec{(void *)(src[pc[k].source] + pc[k].offset), pc[k].length});
+        if (iov.size() == 1024) flush();
+    }
+    flush();
 }
 
 static double now_s() { return chrono::duration<double>(chrono::steady_clock::now().time_since_epoch()).count(); }

@@ -20,8 +20,9 @@
 #include <cstdint>
 #include <cstring>
 #include <memory>
-#include <thread>
 #include <vector>
+
+#include "fork_join.hpp"
 
 namespace pgz {
 
@@ -231,36 +232,30 @@ inline Result inflate_parallel(const uint8_t *comp, size_t n, size_t start_bit, 
     start[0] = start_bit;
     // the first piece knows its window and is inflated once, the others twice: it gets two shares of the span
     const size_t span = (total_bits - start_bit) / (T + 1);
-    {   // 1. entry points of the pieces
-        std::vector<std::thread> th;
-        for (int i = 1; i < T; ++i)
-            // (blocks of a FASTQ file are tens of KiB of compressed data: a piece whose first quarter holds no entry point is left
-            // to the piece in front of it)
-            th.emplace_back([&, i] { start[i] = find_block_start(comp, n, (start_bit + span * (i + 1) + 7) & ~(size_t)7, start_bit + span * (i + 1) + span / 4, D.A); });
-        for (auto &t : th) t.join();
-    }
+    // 1. entry points of the pieces (blocks of a FASTQ file are tens of KiB of compressed data: a piece whose first quarter holds
+    // no entry point is left to the piece in front of it)
+    fork_join(T - 1, [&](int j) {
+        const int i = j + 1;
+        start[i] = find_block_start(comp, n, (start_bit + span * (i + 1) + 7) & ~(size_t)7, start_bit + span * (i + 1) + span / 4, D.A);
+    });
     std::vector<int> idx;           // pieces with an entry point, in order
     for (int i = 0; i < T; ++i)
         if (start[i] != ~(size_t)0 && (idx.empty() || start[i] > start[idx.back()])) idx.push_back(i);
     std::vector<Piece> P(idx.size());
-    {   // 2. every piece up to the entry point of the next one; the first with the true window, the others with both marker sets
-        std::vector<std::thread> th;
-        for (size_t q = 0; q < idx.size(); ++q)
-            th.emplace_back([&, q] {
-                Piece &pc = P[q];
-                pc.start_bit = start[idx[q]];
-                const size_t stop = q + 1 < idx.size() ? start[idx[q + 1]] : ~(size_t)0;
-                const size_t guess = ((std::min(stop, total_bits) - pc.start_bit) >> 3) * 5 + (1u << 16);      // FASTQ deflates 2-4.5 x
-                if (q == 0) pc.end = inflate_from(comp, n, pc.start_bit, stop, window.data() + (kWin - window_len), window_len, 0, pc.out, pc.end_bit, guess);
-                else {
-                    pc.end = inflate_from(comp, n, pc.start_bit, stop, D.A, kWin, 0, pc.out, pc.end_bit, guess);
-                    size_t end_b = 0;
-                    const End eb = inflate_from(comp, n, pc.start_bit, stop, D.B, kWin, 0, pc.out_b, end_b, pc.out.size() + 64);
-                    if (eb != pc.end || end_b != pc.end_bit || pc.out_b.size() != pc.out.size()) pc.end = End::Error;
-                }
-            });
-        for (auto &t : th) t.join();
-    }
+    // 2. every piece up to the entry point of the next one; the first with the true window, the others with both marker sets
+    fork_join((int)idx.size(), [&](int q) {
+        Piece &pc = P[q];
+        pc.start_bit = start[idx[q]];
+        const size_t stop = q + 1 < (int)idx.size() ? start[idx[q + 1]] : ~(size_t)0;
+        const size_t guess = ((std::min(stop, total_bits) - pc.start_bit) >> 3) * 5 + (1u << 16);      // FASTQ deflates 2-4.5 x
+        if (q == 0) pc.end = inflate_from(comp, n, pc.start_bit, stop, window.data() + (kWin - window_len), window_len, 0, pc.out, pc.end_bit, guess);
+        else {
+            pc.end = inflate_from(comp, n, pc.start_bit, stop, D.A, kWin, 0, pc.out, pc.end_bit, guess);
+            size_t end_b = 0;
+            const End eb = inflate_from(comp, n, pc.start_bit, stop, D.B, kWin, 0, pc.out_b, end_b, pc.out.size() + 64);
+            if (eb != pc.end || end_b != pc.end_bit || pc.out_b.size() != pc.out.size()) pc.end = End::Error;
+        }
+    });
     // 3. stitch: a piece counts only if the accepted output ends exactly on its first bit
     if (P[0].end == End::Error) { R.error = true; return R; }
     size_t accepted = 1;
@@ -277,17 +272,12 @@ inline Result inflate_parallel(const uint8_t *comp, size_t n, size_t start_bit, 
         // a marker in the tail may point at a byte of this piece's own window only: positions are relative to win[q]
         slide_window(w, pc.out.data(), nq);
     }
-    {
-        std::vector<std::thread> th;
-        for (size_t q = 1; q < accepted; ++q)
-            th.emplace_back([&, q] {
-                Piece &pc = P[q];
-                const size_t nq = pc.out.size(), tail = std::min(nq, kWin);
-                resolve(pc.out.data(), pc.out_b.data(), nq - tail, win[q].data());
-                pc.out_b.release();
-            });
-        for (auto &t : th) t.join();
-    }
+    fork_join((int)accepted - 1, [&](int j) {
+        Piece &pc = P[j + 1];
+        const size_t nq = pc.out.size(), tail = std::min(nq, kWin);
+        resolve(pc.out.data(), pc.out_b.data(), nq - tail, win[j + 1].data());
+        pc.out_b.release();
+    });
     window = w;
     R.end_bit = P.back().end_bit;
     R.stream_end = P.back().end == End::StreamEnd;
