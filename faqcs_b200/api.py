@@ -104,6 +104,10 @@ class CKmerView(C.Structure):
                 ("n_frequency", C.c_uint64), ("frequency", C.POINTER(C.c_uint64))]
 
 
+class CDupView(C.Structure):
+    _fields_ = [("units", C.c_uint64), ("distinct", C.c_uint64), ("n_levels", C.c_uint64), ("levels", C.POINTER(C.c_uint64))]
+
+
 class CStatsView(C.Structure):
     _fields_ = [
         ("filter_stats", C.c_uint64 * NUM_STAT), ("n_adapters", C.c_uint32),
@@ -319,6 +323,9 @@ class Engine:
             L.fq_allreduce_stats.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
             L.fq_merge_stats.argtypes = [C.c_void_p, C.c_void_p]
             L.fq_kmer_end_pass_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
+            L.fq_dup_enable.argtypes = [C.c_void_p]
+            L.fq_dup_end_pass_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
+            L.fq_dup_results.argtypes = [C.c_void_p, C.POINTER(CDupView)]
             L.fq_last_allreduce_ms.argtypes = [C.c_void_p]
             L.fq_last_allreduce_ms.restype = C.c_float
             L.fq_device_outputs.argtypes = [C.c_void_p, C.POINTER(C.c_void_p * NUM_STREAM)]
@@ -378,6 +385,25 @@ class Engine:
         if v.n_frequency:
             freq[:] = np.ctypeslib.as_array(v.frequency, (v.n_frequency, 2))
         return rare, freq
+
+    def dup_enable(self):
+        """Sequence duplication statistics (fq_dup_enable): every read (single-end) or pair of the following batches is counted
+        by the bytes of its sequence line(s) as framed.  Call before the first batch of a pass."""
+        self._check(self.lib.fq_dup_enable(self.ctx))
+
+    def dup_end_pass(self):
+        """End of one input's pass on this context alone (fq_dup_end_pass_all with n = 1); dist_stats has the sharded forms."""
+        ctxs = (C.c_void_p * 1)(self.ctx)
+        self._check(self.lib.fq_dup_end_pass_all(ctxs, 1, None))
+
+    def dup_results(self) -> dict:
+        """The last finished pass: {"units", "distinct", "levels": [m, 2] uint64 = (multiplicity, distinct keys), ascending}."""
+        v = CDupView()
+        self._check(self.lib.fq_dup_results(self.ctx, C.byref(v)))
+        levels = np.zeros((v.n_levels, 2), np.uint64)
+        if v.n_levels:
+            levels[:] = np.ctypeslib.as_array(v.levels, (v.n_levels, 2))
+        return {"units": int(v.units), "distinct": int(v.distinct), "levels": levels}
 
     def set_quality(self, quality: int):
         """Options::quality for the following batches (the reference's NextSeq adjustment, FaQCs.cpp:272-277)."""

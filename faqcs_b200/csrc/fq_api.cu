@@ -21,6 +21,7 @@
 
 #include "fq_adapter.cuh"
 #include "fq_common.cuh"
+#include "fq_dup.cuh"
 #include "fq_emit.cuh"
 #include "fq_frame.cuh"
 #include "fq_kmer.cuh"
@@ -77,6 +78,15 @@ struct Buf {
 };
 using DevBuf = Buf<false>;
 using HostBuf = Buf<true>;
+
+// An open-addressing table of KmerSlot in device memory (fq_kmer.cuh) with the buffers of its end-of-pass exchange: the k-mer
+// table and the duplication table of a context.
+struct HashTable {
+    unsigned long long min_cap = 1ull << 20;       // slots of a new table (a power of two)
+    unsigned long long cap = 0, occupied_bound = 0;
+    DevBuf d_slots, d_scalars;
+    DevBuf d_send, d_recv;                         // end of a sharded pass: entries grouped by owner, one received group
+};
 
 const char *kPhiX = "__PhiX174_NC_001422__";                       // FaQCs.h:29-30
 const char *kPhiXComplement = "__PhiX174_NC_001422_complement__";
@@ -135,11 +145,21 @@ struct fq_ctx {
         uint64_t calls_beyond = 0;                 // calls >= kKmerMaxCalls run here (the curve is complete by then)
         uint64_t call_end = 0;                     // 1 + the highest call run here
         uint64_t pass_reads = 0;
-        unsigned long long cap = 0, occupied_bound = 0;
-        DevBuf d_slots, d_call_total, d_call_distinct, d_small, d_big, d_scalars;
-        DevBuf d_send, d_recv;                     // end of a sharded pass: entries grouped by owner, one received group
+        HashTable T;
+        DevBuf d_call_total, d_call_distinct, d_small, d_big;
         std::vector<uint64_t> flat;                // fq_kmer_view::frequency
     } kmer;
+
+    // duplication statistics (fq_dup_*, fq_dup.cuh): one key per read or pair
+    struct Dup {
+        bool enabled = false;
+        uint32_t n_mates = 0;                      // mates per unit in the current pass (0: no batch yet)
+        uint64_t units = 0;                        // units of the current pass counted here
+        HashTable T{1ull << 16};                   // small, so that modest inputs already exercise the growth
+        DevBuf d_small, d_big;                     // end of a pass: the histogram of counts
+        uint64_t res_units = 0, res_distinct = 0;  // the last finished pass (fq_dup_view)
+        std::vector<uint64_t> levels;
+    } dup;
 
     // host-side stats views handed out by fq_stats
     std::vector<uint64_t> v_adapter_reads, v_adapter_bases, v_pre_q, v_post_q, v_pre_b, v_post_b, v_hist[4], v_pre_comp,
@@ -432,33 +452,55 @@ fq_status map_device_error(fq_ctx *ctx, const BatchInfo &hi)
     return fail(ctx, FQ_ERR_STATE, "unknown device error");
 }
 
-// ---- k-mer rarefaction: host side of fq_kmer.cuh ---------------------------------------------------------
-KmerTable kmer_table_of(fq_ctx::Kmer &K)
+// ---- the hash tables (k-mer rarefaction, duplication statistics): host side of fq_kmer.cuh -------------------------
+KmerTable table_of(const HashTable &T)
 {
-    return KmerTable{K.d_slots.as<KmerSlot>(), K.cap - 1};
+    return KmerTable{T.d_slots.as<KmerSlot>(), T.cap - 1};
 }
 
 // (Re)allocate the table for at least `slots` slots (a power of two), keeping its entries (or, with keep == false, empty).
-fq_status kmer_resize(fq_ctx *ctx, unsigned long long slots, bool keep = true)
+fq_status table_resize(fq_ctx *ctx, HashTable &T, unsigned long long slots, bool keep = true)
 {
-    fq_ctx::Kmer &K = ctx->kmer;
-    unsigned long long cap = 1ull << 20;
+    unsigned long long cap = T.min_cap;
     while (cap < slots) cap <<= 1;
-    if (cap <= K.cap) return FQ_OK;
+    if (cap <= T.cap) return FQ_OK;
     if (!keep) {
         CK(cudaStreamSynchronize(ctx->stream));
-        K.d_slots.release();
-        K.cap = 0;
+        T.d_slots.release();
+        T.cap = 0;
     }
     DevBuf ns;
     CK(ns.ensure(cap * sizeof(KmerSlot)));
     KmerTable to{ns.as<KmerSlot>(), cap - 1};
     k_kmer_clear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(to);
-    if (K.cap) k_kmer_rehash<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), to);
-    ctx->launches += K.cap ? 2 : 1;
+    if (T.cap) k_kmer_rehash<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(T), to);
+    ctx->launches += T.cap ? 2 : 1;
     CK(cudaStreamSynchronize(ctx->stream));
-    K.d_slots = std::move(ns);
-    K.cap = cap;
+    T.d_slots = std::move(ns);
+    T.cap = cap;
+    return FQ_OK;
+}
+
+// Room for `adding` more keys at a load factor <= 1/2, before a batch; the bound on the occupied slots is made exact when it
+// matters.
+fq_status table_reserve(fq_ctx *ctx, HashTable &T, unsigned long long adding)
+{
+    unsigned long long need = T.occupied_bound + adding;
+    if (2 * need > T.cap && T.cap) {
+        CK(cudaMemsetAsync(T.d_scalars.p, 0, 16, ctx->stream));
+        k_kmer_count<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(T), T.d_scalars.as<unsigned long long>());
+        ctx->launches++;
+        unsigned long long occ = 0;
+        CK(cudaMemcpyAsync(&occ, T.d_scalars.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        T.occupied_bound = occ;
+        need = occ + adding;
+    }
+    if (2 * need > T.cap) {
+        fq_status st = table_resize(ctx, T, 2 * need);
+        if (st != FQ_OK) return st;
+    }
+    T.occupied_bound = need;
     return FQ_OK;
 }
 
@@ -526,24 +568,10 @@ fq_status kmer_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint
     }
     K.call_end = std::max(K.call_end, first_call + n_calls);
     if (w.counted <= first_call || counted_reads == 0) return FQ_OK;
-    // room for every k-mer this batch can add (load factor <= 1/2); the bound on the occupied slots is made exact when it matters
+    // room for every k-mer this batch can add
     const unsigned long long per_read = max_len >= K.k ? (unsigned long long)(max_len - K.k + 1) : 0ull;
-    unsigned long long need = K.occupied_bound + counted_reads * per_read;
-    if (2 * need > K.cap && K.cap) {
-        CK(cudaMemsetAsync(K.d_scalars.p, 0, 16, ctx->stream));
-        k_kmer_count<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), K.d_scalars.as<unsigned long long>());
-        ctx->launches++;
-        unsigned long long occ = 0;
-        CK(cudaMemcpyAsync(&occ, K.d_scalars.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        K.occupied_bound = occ;
-        need = occ + counted_reads * per_read;
-    }
-    if (2 * need > K.cap) {
-        fq_status st = kmer_resize(ctx, 2 * need);
-        if (st != FQ_OK) return st;
-    }
-    K.occupied_bound = need;
+    st = table_reserve(ctx, K.T, counted_reads * per_read);
+    if (st != FQ_OK) return st;
     KmerArgs ka{};
     ka.raw[0] = d_r1; ka.raw[1] = d_r2;
     ka.rec[0] = ctx->d_rec[0].as<Rec>(); ka.rec[1] = ctx->d_rec[1].as<Rec>();
@@ -552,10 +580,28 @@ fq_status kmer_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint
     ka.n_rec = n; ka.n_mates = (uint32_t)n_mates; ka.k = K.k;
     ka.replace_q = ctx->dopt.replace_q; ka.in_off = ctx->dopt.in_off;
     ka.first_call = (uint32_t)first_call; ka.stop_call = w.counted;
-    ka.T = kmer_table_of(K);
+    ka.T = table_of(K.T);
     ka.call_total = K.d_call_total.as<unsigned long long>();
     k_kmer<<<(n * n_mates + 255) / 256, 256, 0, ctx->stream>>>(ka);
     ctx->launches++;
+    return FQ_OK;
+}
+
+// One batch of duplication statistics: room for one key per unit, then one insert per unit.
+fq_status dup_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint32_t n, int n_mates)
+{
+    fq_ctx::Dup &D = ctx->dup;
+    fq_status st = table_reserve(ctx, D.T, n);
+    if (st != FQ_OK) return st;
+    DupArgs da{};
+    da.raw[0] = d_r1; da.raw[1] = d_r2;
+    da.rec[0] = ctx->d_rec[0].as<Rec>(); da.rec[1] = ctx->d_rec[1].as<Rec>();
+    da.n_rec = n; da.n_mates = (uint32_t)n_mates;
+    da.T = table_of(D.T);
+    k_dup<<<(n + 7) / 8, 256, 0, ctx->stream>>>(da);
+    ctx->launches++;
+    D.n_mates = (uint32_t)n_mates;
+    D.units += n;
     return FQ_OK;
 }
 
@@ -572,6 +618,8 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
     const DevOpts o = ctx->dopt;
     if (o.filter_adapter && o.num_thread && (first_record_index % FQ_REF_BATCH) != 0)
         return fail(ctx, FQ_ERR_ARG, "thread-count emulation needs batches that start on a 32768-record boundary");
+    if (ctx->dup.enabled && ctx->dup.n_mates && ctx->dup.n_mates != (paired ? 2u : 1u))
+        return fail(ctx, FQ_ERR_ARG, "duplication statistics: paired and single-end batches in one pass");
     BatchInfo *info = ctx->d_info.as<BatchInfo>();
     CK(reset_info(ctx));
     CK(cudaEventRecord(ctx->ev[0], ctx->stream));
@@ -732,6 +780,11 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
     // ---- k-mer rarefaction: raw reads under --qc_only (trim.cpp:260-262), trimmed survivors otherwise (trim.cpp:545-547)
     if (ctx->kmer.enabled) {
         st = kmer_batch(ctx, d_r1, d_r2, n, n_mates, max_len, first_record_index, is_final, !o.qc_only);
+        if (st != FQ_OK) return st;
+    }
+    // ---- duplication statistics: the sequence lines as framed
+    if (ctx->dup.enabled) {
+        st = dup_batch(ctx, d_r1, d_r2, n, n_mates);
         if (st != FQ_OK) return st;
     }
 
@@ -1140,9 +1193,9 @@ fq_status fq_kmer_enable(fq_ctx *ctx, uint32_t k, uint64_t split_size, uint32_t 
     CK(K.d_call_distinct.ensure((size_t)kKmerMaxCalls * 8));
     CK(K.d_small.ensure((size_t)kKmerSmallCounts * 8));
     CK(K.d_big.ensure((size_t)(1u << 20) * 4));
-    CK(K.d_scalars.ensure(64));
+    CK(K.T.d_scalars.ensure(64));
     CK(cudaMemset(K.d_call_total.p, 0, (size_t)kKmerMaxCalls * 8));
-    return kmer_resize(ctx, 1ull << 24);
+    return table_resize(ctx, K.T, 1ull << 24);
 }
 
 fq_status fq_kmer_end_pass(fq_ctx *ctx)
@@ -1461,46 +1514,44 @@ struct KmerSum {
 };
 
 // Occupied slots of the context's table per owner.
-fq_status kmer_owner_counts(fq_ctx *ctx, uint32_t n_shards, uint64_t *counts)
+fq_status table_owner_counts(fq_ctx *ctx, HashTable &T, uint32_t n_shards, uint64_t *counts)
 {
-    fq_ctx::Kmer &K = ctx->kmer;
     CK(cudaSetDevice(ctx->device));
-    CK(K.d_scalars.ensure(64 + (size_t)n_shards * 8));
-    CK(cudaMemsetAsync(K.d_scalars.p, 0, (size_t)n_shards * 8, ctx->stream));
-    k_kmer_partition_count<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), n_shards, K.d_scalars.as<unsigned long long>());
+    CK(T.d_scalars.ensure(64 + (size_t)n_shards * 8));
+    CK(cudaMemsetAsync(T.d_scalars.p, 0, (size_t)n_shards * 8, ctx->stream));
+    k_kmer_partition_count<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(T), n_shards, T.d_scalars.as<unsigned long long>());
     ctx->launches++;
-    CK(cudaMemcpyAsync(counts, K.d_scalars.p, (size_t)n_shards * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(counts, T.d_scalars.p, (size_t)n_shards * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return FQ_OK;
 }
 
 // The table's entries into d_send grouped by owner (group j at offsets[j]); the table is then cleared -- first grown, empty,
 // if `incoming` entries need more than half of it -- and takes back the context's own group.
-fq_status kmer_scatter(fq_ctx *ctx, uint32_t n_shards, uint32_t me, const uint64_t *counts, uint64_t incoming, std::vector<uint64_t> *offsets)
+fq_status table_scatter(fq_ctx *ctx, HashTable &T, uint32_t n_shards, uint32_t me, const uint64_t *counts, uint64_t incoming, std::vector<uint64_t> *offsets)
 {
-    fq_ctx::Kmer &K = ctx->kmer;
     CK(cudaSetDevice(ctx->device));
     offsets->assign(n_shards + 1, 0);
     for (uint32_t j = 0; j < n_shards; ++j) (*offsets)[j + 1] = (*offsets)[j] + counts[j];
-    CK(K.d_send.ensure(std::max<uint64_t>(offsets->back(), 1) * sizeof(KmerSlot)));
-    CK(cudaMemcpyAsync(K.d_scalars.p, offsets->data(), (size_t)n_shards * 8, cudaMemcpyHostToDevice, ctx->stream));
-    k_kmer_partition_scatter<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), n_shards, K.d_scalars.as<unsigned long long>(), K.d_send.as<KmerSlot>());
-    k_kmer_clear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K));
+    CK(T.d_send.ensure(std::max<uint64_t>(offsets->back(), 1) * sizeof(KmerSlot)));
+    CK(cudaMemcpyAsync(T.d_scalars.p, offsets->data(), (size_t)n_shards * 8, cudaMemcpyHostToDevice, ctx->stream));
+    k_kmer_partition_scatter<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(T), n_shards, T.d_scalars.as<unsigned long long>(), T.d_send.as<KmerSlot>());
+    k_kmer_clear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(T));
     ctx->launches += 2;
-    fq_status st = kmer_resize(ctx, 2 * incoming, false);
+    fq_status st = table_resize(ctx, T, 2 * incoming, false);
     if (st != FQ_OK) return st;
     if (counts[me]) {
-        k_kmer_merge<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), K.d_send.as<KmerSlot>() + (*offsets)[me], counts[me]);
+        k_kmer_merge<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(T), T.d_send.as<KmerSlot>() + (*offsets)[me], counts[me]);
         ctx->launches++;
     }
     CK(cudaGetLastError());
     return FQ_OK;
 }
 
-fq_status kmer_merge_received(fq_ctx *ctx, uint64_t n)
+fq_status table_merge_received(fq_ctx *ctx, HashTable &T, uint64_t n)
 {
     if (!n) return FQ_OK;
-    k_kmer_merge<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(ctx->kmer), ctx->kmer.d_recv.as<KmerSlot>(), n);
+    k_kmer_merge<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(T), T.d_recv.as<KmerSlot>(), n);
     ctx->launches++;
     CK(cudaGetLastError());
     return FQ_OK;
@@ -1513,10 +1564,10 @@ fq_status kmer_summarize(fq_ctx *ctx, const KmerSum &S, uint32_t me, std::vector
     CK(cudaSetDevice(ctx->device));
     CK(cudaMemsetAsync(K.d_call_distinct.p, 0, (size_t)kKmerMaxCalls * 8, ctx->stream));
     CK(cudaMemsetAsync(K.d_small.p, 0, (size_t)kKmerSmallCounts * 8, ctx->stream));
-    CK(cudaMemsetAsync(K.d_scalars.p, 0, 64, ctx->stream));
-    k_kmer_summarize<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K), K.d_call_distinct.as<unsigned long long>(), K.d_small.as<unsigned long long>(),
-                                                              K.d_big.as<uint32_t>(), kKmerBigCap, reinterpret_cast<uint32_t *>(K.d_scalars.as<uint8_t>() + 16),
-                                                              K.d_scalars.as<unsigned long long>());
+    CK(cudaMemsetAsync(K.T.d_scalars.p, 0, 64, ctx->stream));
+    k_kmer_summarize<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(K.T), K.d_call_distinct.as<unsigned long long>(), K.d_small.as<unsigned long long>(),
+                                                              K.d_big.as<uint32_t>(), kKmerBigCap, reinterpret_cast<uint32_t *>(K.T.d_scalars.as<uint8_t>() + 16),
+                                                              K.T.d_scalars.as<unsigned long long>());
     ctx->launches++;
     flat->assign(S.total, 0);
     uint64_t *F = flat->data();
@@ -1524,8 +1575,8 @@ fq_status kmer_summarize(fq_ctx *ctx, const KmerSum &S, uint32_t me, std::vector
     CK(cudaMemcpyAsync(F + S.call_total, K.d_call_total.p, (size_t)kKmerMaxCalls * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(F + S.call_distinct, K.d_call_distinct.p, (size_t)kKmerMaxCalls * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(F + S.small, K.d_small.p, (size_t)kKmerSmallCounts * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(F + S.n_distinct, K.d_scalars.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync(&n_big, K.d_scalars.as<uint8_t>() + 16, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(F + S.n_distinct, K.T.d_scalars.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&n_big, K.T.d_scalars.as<uint8_t>() + 16, 4, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     if (!K.call_reads.empty()) {
         std::copy(K.call_reads.begin(), K.call_reads.end(), F + S.call_reads);
@@ -1594,14 +1645,14 @@ fq_status kmer_finish(fq_ctx *ctx, const KmerSum &S, uint32_t n_shards, const st
         std::fill(K.call_runs.begin(), K.call_runs.end(), 0);
     }
     K.calls_beyond = K.call_end = K.pass_reads = 0;
-    K.occupied_bound = 0;
+    K.T.occupied_bound = 0;
     CK(cudaSetDevice(ctx->device));
-    k_kmer_clear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(kmer_table_of(K));
+    k_kmer_clear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(K.T));
     ctx->launches++;
     CK(cudaMemsetAsync(K.d_call_total.p, 0, (size_t)kKmerMaxCalls * 8, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    K.d_send.release();
-    K.d_recv.release();
+    K.T.d_send.release();
+    K.T.d_recv.release();
     return FQ_OK;
 }
 
@@ -1630,14 +1681,14 @@ fq_status nccl_sum_u64(fq_ctx *ctx, const fq_comm *c, std::vector<uint64_t> *v)
     return FQ_OK;
 }
 
-// Every rank's list of large counts (n_big[j] of rank j) on every rank.
-fq_status nccl_gather_big(fq_ctx *ctx, const fq_comm *c, const uint64_t *n_big, std::vector<uint32_t> *big)
+// Every rank's list of large counts (n_big[j] of rank j, at d_big on each) on every rank.
+fq_status nccl_gather_big(fq_ctx *ctx, const fq_comm *c, const void *d_big, const uint64_t *n_big, std::vector<uint32_t> *big)
 {
     uint64_t most = 1;
     for (int j = 0; j < c->n_ranks; ++j) most = std::max(most, n_big[j]);
     DevBuf d;
     CK(d.ensure((size_t)c->n_ranks * most * 4));
-    NK(ctx, nccl().AllGather(ctx->kmer.d_big.p, d.p, most, ncclUint32, c->comm, ctx->stream));
+    NK(ctx, nccl().AllGather(d_big, d.p, most, ncclUint32, c->comm, ctx->stream));
     std::vector<uint32_t> all((size_t)c->n_ranks * most);
     CK(cudaMemcpyAsync(all.data(), d.p, all.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
@@ -1646,16 +1697,91 @@ fq_status nccl_gather_big(fq_ctx *ctx, const fq_comm *c, const uint64_t *n_big, 
     return FQ_OK;
 }
 
-fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
+// Steps 3 and 4 of the end of a sharded pass, for either table (tab(ctx) is the context's table): the contexts' groups go to
+// their owners in n_shards - 1 rounds (round r: shard s sends to s + r, receives from s - r), and each owner merges them into
+// its cleared table.  head[s * H + kHeadCounts + j] = entries of shard s owned by shard j.
+constexpr size_t kHeadCounts = 4;
+
+using TableOf = HashTable &(*)(fq_ctx *);
+
+fq_status table_exchange(fq_ctx *const *ctxs, int n, const fq_comm *cm, uint32_t rank0, uint32_t n_shards, TableOf tab, const std::vector<uint64_t> &head, size_t H)
 {
+    auto counts = [&](uint32_t from, uint32_t to) { return head[(size_t)from * H + kHeadCounts + to]; };
+    std::vector<std::vector<uint64_t>> offsets(n);
+    for (int i = 0; i < n; ++i) {
+        fq_ctx *const ctx = ctxs[i];
+        const uint32_t me = rank0 + i;
+        uint64_t incoming = 0, largest = 1;
+        for (uint32_t j = 0; j < n_shards; ++j) {
+            incoming += counts(j, me);
+            if (j != me) largest = std::max(largest, counts(j, me));
+        }
+        fq_status st = table_scatter(ctx, tab(ctx), n_shards, me, head.data() + (size_t)me * H + kHeadCounts, incoming, &offsets[i]);
+        if (st != FQ_OK) return st;
+        CK(tab(ctx).d_recv.ensure(largest * sizeof(KmerSlot)));
+    }
+    fq_status st = sync_all(ctxs, n);       // every send buffer is complete before another context reads it
+    if (st != FQ_OK) return st;
+    for (uint32_t r = 1; r < n_shards; ++r) {
+        for (int i = 0; i < n; ++i) {
+            fq_ctx *const ctx = ctxs[i];
+            HashTable &T = tab(ctx);
+            const uint32_t me = rank0 + i, dst = (me + r) % n_shards, src = (me + n_shards - r) % n_shards;
+            const uint64_t n_out = counts(me, dst), n_in = counts(src, me);
+            CK(cudaSetDevice(ctx->device));
+            if (cm) {
+                if (!n_out && !n_in) continue;      // both ends know the counts: neither posts a transfer
+                NK(ctx, nccl().GroupStart());
+                if (n_out) NK(ctx, nccl().Send(T.d_send.as<KmerSlot>() + offsets[i][dst], 2 * n_out, ncclUint64, (int)dst, cm->comm, ctx->stream));
+                if (n_in) NK(ctx, nccl().Recv(T.d_recv.p, 2 * n_in, ncclUint64, (int)src, cm->comm, ctx->stream));
+                NK(ctx, nccl().GroupEnd());
+            } else if (n_in) {
+                fq_ctx *const from = ctxs[src];
+                CK(cudaMemcpyPeerAsync(T.d_recv.p, ctx->device, tab(from).d_send.as<KmerSlot>() + offsets[src][me], from->device,
+                                       n_in * sizeof(KmerSlot), ctx->stream));
+            }
+            st = table_merge_received(ctx, T, n_in);
+            if (st != FQ_OK) return st;
+        }
+    }
+    return FQ_OK;
+}
+
+// The arguments and the error reporting of an end of pass over n contexts, shared by both tables: impl runs the pass, with
+// ctxs[0] as shard rank0 of n_shards.
+using EndPassImpl = fq_status (*)(fq_ctx *const *ctxs, int n, const fq_comm *cm, uint32_t n_shards, uint32_t rank0);
+
+fq_status end_pass_entry(fq_ctx *const *ctxs, int n, fq_comm *const *comm, const char *name, EndPassImpl impl)
+{
+    if (!ctxs || n < 1) return FQ_ERR_ARG;
+    for (int i = 0; i < n; ++i) {
+        if (!ctxs[i]) return FQ_ERR_ARG;
+        for (int j = 0; j < i; ++j)
+            if (ctxs[j] == ctxs[i]) return fail(ctxs[0], FQ_ERR_ARG, std::string(name) + ": a context is listed twice");
+    }
+    if (comm && !comm[0]) return fail(ctxs[0], FQ_ERR_ARG, std::string(name) + ": null communicator");
+    fq_status st = FQ_OK;
     fq_ctx *const ctx0 = ctxs[0];
     const fq_comm *cm = comm ? comm[0] : nullptr;
-    if (cm && (n != 1 || cm->device != ctx0->device)) return fail(ctx0, FQ_ERR_ARG, "fq_kmer_end_pass_all: with a communicator, pass this process's one context on its device");
-    if (cm && !nccl().ok) return fail(ctx0, FQ_ERR_STATE, "NCCL (libnccl.so.2) could not be loaded");
     const uint32_t n_shards = cm ? (uint32_t)cm->n_ranks : (uint32_t)n;
-    const uint32_t rank0 = cm ? (uint32_t)cm->rank : 0;         // shard index of ctxs[0]
-    if (n_shards > kKmerMaxOwners) return fail(ctx0, FQ_ERR_ARG, "fq_kmer_end_pass_all: more than 1024 contexts");
-    for (int i = 0; i < n; ++i) ctxs[i]->error.clear();
+    if (cm && (n != 1 || cm->device != ctx0->device)) st = fail(ctx0, FQ_ERR_ARG, std::string(name) + ": with a communicator, pass this process's one context on its device");
+    else if (cm && !nccl().ok) st = fail(ctx0, FQ_ERR_STATE, "NCCL (libnccl.so.2) could not be loaded");
+    else if (n_shards > kKmerMaxOwners) st = fail(ctx0, FQ_ERR_ARG, std::string(name) + ": more than 1024 contexts");
+    else {
+        for (int i = 0; i < n; ++i) ctxs[i]->error.clear();
+        st = impl(ctxs, n, cm, n_shards, cm ? (uint32_t)cm->rank : 0u);
+    }
+    if (st != FQ_OK) {          // the verdict is the run's: every context reports it
+        std::string msg;
+        for (int i = 0; i < n && msg.empty(); ++i) msg = ctxs[i]->error;
+        for (int i = 0; i < n; ++i) ctxs[i]->error = msg;
+    }
+    return st;
+}
+
+fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, const fq_comm *cm, uint32_t n_shards, uint32_t rank0)
+{
+    fq_ctx *const ctx0 = ctxs[0];
     fq_status st = sync_all(ctxs, n);
     if (st != FQ_OK) return st;
     // 1. agree on the parameters; 2. occupied slots per owner: header {enabled, k, split_size, num_subsample, counts[n_shards]}
@@ -1666,7 +1792,7 @@ fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
         uint64_t *h = head.data() + (size_t)(rank0 + i) * H;
         h[0] = K.enabled; h[1] = K.k; h[2] = K.split_size; h[3] = K.num_subsample;
         if (K.enabled && n_shards > 1) {
-            st = kmer_owner_counts(ctxs[i], n_shards, h + 4);
+            st = table_owner_counts(ctxs[i], ctxs[i]->kmer.T, n_shards, h + kHeadCounts);
             if (st != FQ_OK) return st;
         }
     }
@@ -1688,45 +1814,10 @@ fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
             return fail(ctx0, FQ_ERR_ARG, msg);
         }
     }
-    auto counts = [&](uint32_t from, uint32_t to) { return head[(size_t)from * H + 4 + to]; };
-    // 3, 4. exchange the groups in n_shards - 1 rounds (round r: shard s sends to s + r, receives from s - r) and merge
+    // 3, 4. exchange the groups and merge
     if (n_shards > 1) {
-        std::vector<std::vector<uint64_t>> offsets(n);
-        for (int i = 0; i < n; ++i) {
-            fq_ctx *const ctx = ctxs[i];
-            const uint32_t me = rank0 + i;
-            uint64_t incoming = 0, largest = 1;
-            for (uint32_t j = 0; j < n_shards; ++j) {
-                incoming += counts(j, me);
-                if (j != me) largest = std::max(largest, counts(j, me));
-            }
-            st = kmer_scatter(ctx, n_shards, me, head.data() + (size_t)me * H + 4, incoming, &offsets[i]);
-            if (st != FQ_OK) return st;
-            CK(ctx->kmer.d_recv.ensure(largest * sizeof(KmerSlot)));
-        }
-        st = sync_all(ctxs, n);                 // every send buffer is complete before another context reads it
+        st = table_exchange(ctxs, n, cm, rank0, n_shards, [](fq_ctx *c) -> HashTable & { return c->kmer.T; }, head, H);
         if (st != FQ_OK) return st;
-        for (uint32_t r = 1; r < n_shards; ++r) {
-            for (int i = 0; i < n; ++i) {
-                fq_ctx *const ctx = ctxs[i];
-                const uint32_t me = rank0 + i, dst = (me + r) % n_shards, src = (me + n_shards - r) % n_shards;
-                const uint64_t n_out = counts(me, dst), n_in = counts(src, me);
-                CK(cudaSetDevice(ctx->device));
-                if (cm) {
-                    if (!n_out && !n_in) continue;      // both ends know the counts: neither posts a transfer
-                    NK(ctx, nccl().GroupStart());
-                    if (n_out) NK(ctx, nccl().Send(ctx->kmer.d_send.as<KmerSlot>() + offsets[i][dst], 2 * n_out, ncclUint64, (int)dst, cm->comm, ctx->stream));
-                    if (n_in) NK(ctx, nccl().Recv(ctx->kmer.d_recv.p, 2 * n_in, ncclUint64, (int)src, cm->comm, ctx->stream));
-                    NK(ctx, nccl().GroupEnd());
-                } else if (n_in) {
-                    const fq_ctx *from = ctxs[src];
-                    CK(cudaMemcpyPeerAsync(ctx->kmer.d_recv.p, ctx->device, from->kmer.d_send.as<KmerSlot>() + offsets[src][me], from->device,
-                                           n_in * sizeof(KmerSlot), ctx->stream));
-                }
-                st = kmer_merge_received(ctx, n_in);
-                if (st != FQ_OK) return st;
-            }
-        }
     }
     // 5. summarise each shard; 6. combine
     const KmerSum S(n_shards);
@@ -1744,7 +1835,7 @@ fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
         if (st == FQ_OK) {
             for (uint32_t j = 0; j < n_shards; ++j)
                 if (sum[S.n_big + j] > kKmerBigCap) return fail(ctx0, FQ_ERR_ARG, "k-mer rarefaction: more than 2^20 k-mers with counts above 65535");
-            st = nccl_gather_big(ctx0, cm, sum.data() + S.n_big, &big);
+            st = nccl_gather_big(ctx0, cm, ctx0->kmer.d_big.p, sum.data() + S.n_big, &big);
         }
         if (st != FQ_OK) return st;
     }
@@ -1756,24 +1847,160 @@ fq_status kmer_end_pass_impl(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
     return FQ_OK;
 }
 
+// ---- duplication statistics: end of a pass, over one context or a table sharded over several -------------------------
+// The summary block of one shard: {histogram of counts below kKmerSmallCounts, distinct keys, per shard: keys with a larger
+// count (listed separately)}.
+constexpr size_t kDupDistinct = kKmerSmallCounts, kDupBig = kKmerSmallCounts + 1;
+
+fq_status dup_summarize(fq_ctx *ctx, uint32_t n_shards, uint32_t me, std::vector<uint64_t> *flat, std::vector<uint32_t> *big)
+{
+    fq_ctx::Dup &D = ctx->dup;
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaMemsetAsync(D.d_small.p, 0, (size_t)kKmerSmallCounts * 8, ctx->stream));
+    CK(cudaMemsetAsync(D.T.d_scalars.p, 0, 64, ctx->stream));
+    // no slot of this table has a first call (fq_dup.cuh), so the per-call array is never written
+    k_kmer_summarize<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(D.T), nullptr, D.d_small.as<unsigned long long>(), D.d_big.as<uint32_t>(), kKmerBigCap,
+                                                              reinterpret_cast<uint32_t *>(D.T.d_scalars.as<uint8_t>() + 16), D.T.d_scalars.as<unsigned long long>());
+    ctx->launches++;
+    flat->assign(kDupBig + n_shards, 0);
+    uint64_t *F = flat->data();
+    uint32_t n_big = 0;
+    CK(cudaMemcpyAsync(F, D.d_small.p, (size_t)kKmerSmallCounts * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(F + kDupDistinct, D.T.d_scalars.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(&n_big, D.T.d_scalars.as<uint8_t>() + 16, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    F[kDupBig + me] = n_big;
+    if (big) {
+        big->resize(std::min(n_big, kKmerBigCap));
+        if (!big->empty()) CK(cudaMemcpy(big->data(), D.d_big.p, big->size() * 4, cudaMemcpyDeviceToHost));
+    }
+    return FQ_OK;
+}
+
+// The pass's result on one context, then a cleared table for the next pass.
+fq_status dup_finish(fq_ctx *ctx, uint64_t units, const std::vector<uint64_t> &sum, const std::vector<uint32_t> &big)
+{
+    fq_ctx::Dup &D = ctx->dup;
+    std::map<uint64_t, uint64_t> levels;
+    for (uint32_t c = 1; c < kKmerSmallCounts; ++c)
+        if (sum[c]) levels[c] += sum[c];
+    for (uint32_t c : big) levels[c] += 1;
+    D.levels.clear();
+    for (const auto &kv : levels) { D.levels.push_back(kv.first); D.levels.push_back(kv.second); }
+    D.res_units = units;
+    D.res_distinct = sum[kDupDistinct];
+    D.units = 0;
+    D.n_mates = 0;
+    D.T.occupied_bound = 0;
+    CK(cudaSetDevice(ctx->device));
+    k_kmer_clear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(D.T));
+    ctx->launches++;
+    CK(cudaStreamSynchronize(ctx->stream));
+    D.T.d_send.release();
+    D.T.d_recv.release();
+    return FQ_OK;
+}
+
+fq_status dup_end_pass_impl(fq_ctx *const *ctxs, int n, const fq_comm *cm, uint32_t n_shards, uint32_t rank0)
+{
+    fq_ctx *const ctx0 = ctxs[0];
+    fq_status st = sync_all(ctxs, n);
+    if (st != FQ_OK) return st;
+    // 1. agree on the units; 2. occupied slots per owner: header {enabled, mates per unit (0: no batch), units, -, counts[n_shards]}
+    const size_t H = kHeadCounts + n_shards;
+    std::vector<uint64_t> head((size_t)n_shards * H, 0);
+    for (int i = 0; i < n; ++i) {
+        fq_ctx::Dup &D = ctxs[i]->dup;
+        uint64_t *h = head.data() + (size_t)(rank0 + i) * H;
+        h[0] = D.enabled; h[1] = D.n_mates; h[2] = D.units;
+        if (D.enabled && n_shards > 1) {
+            st = table_owner_counts(ctxs[i], D.T, n_shards, h + kHeadCounts);
+            if (st != FQ_OK) return st;
+        }
+    }
+    if (cm) {
+        const std::vector<uint64_t> mine(head.begin() + (size_t)rank0 * H, head.begin() + (size_t)(rank0 + 1) * H);
+        st = nccl_allgather_u64(ctx0, cm, mine, &head);
+        if (st != FQ_OK) return st;
+    }
+    uint64_t enabled = 0, n_mates = 0, units = 0;
+    for (uint32_t j = 0; j < n_shards; ++j) {
+        const uint64_t *h = head.data() + (size_t)j * H;
+        enabled += h[0];
+        if (h[1] && n_mates && h[1] != n_mates) return fail(ctx0, FQ_ERR_ARG, "fq_dup_end_pass_all: some contexts counted pairs, others single reads");
+        if (h[1]) n_mates = h[1];
+        units += h[2];
+    }
+    if (!enabled) return fail(ctx0, FQ_ERR_STATE, "fq_dup_end_pass_all: duplication statistics are not enabled (fq_dup_enable)");
+    if (enabled != n_shards) return fail(ctx0, FQ_ERR_ARG, "fq_dup_end_pass_all: duplication statistics are enabled on some contexts only");
+    // 3, 4. exchange the groups and merge
+    if (n_shards > 1) {
+        st = table_exchange(ctxs, n, cm, rank0, n_shards, [](fq_ctx *c) -> HashTable & { return c->dup.T; }, head, H);
+        if (st != FQ_OK) return st;
+    }
+    // 5. summarise each shard; 6. combine
+    std::vector<uint64_t> sum(kDupBig + n_shards, 0), flat;
+    std::vector<uint32_t> big, part;
+    for (int i = 0; i < n; ++i) {
+        st = dup_summarize(ctxs[i], n_shards, rank0 + i, &flat, cm ? nullptr : &part);
+        if (st != FQ_OK) return st;
+        for (size_t k = 0; k < sum.size(); ++k) sum[k] += flat[k];
+        big.insert(big.end(), part.begin(), part.end());
+    }
+    if (cm) {
+        st = nccl_sum_u64(ctx0, cm, &sum);
+        if (st != FQ_OK) return st;
+    }
+    for (uint32_t j = 0; j < n_shards; ++j)
+        if (sum[kDupBig + j] > kKmerBigCap) return fail(ctx0, FQ_ERR_ARG, "duplication statistics: more than 2^20 sequences with more than 65535 copies in one shard");
+    if (cm) {
+        st = nccl_gather_big(ctx0, cm, ctx0->dup.d_big.p, sum.data() + kDupBig, &big);
+        if (st != FQ_OK) return st;
+    }
+    // 7. the same result on every context
+    for (int i = 0; i < n; ++i) {
+        st = dup_finish(ctxs[i], units, sum, big);
+        if (st != FQ_OK) return st;
+    }
+    return FQ_OK;
+}
+
 }  // namespace
 
 fq_status fq_kmer_end_pass_all(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
 {
-    if (!ctxs || n < 1) return FQ_ERR_ARG;
-    for (int i = 0; i < n; ++i) {
-        if (!ctxs[i]) return FQ_ERR_ARG;
-        for (int j = 0; j < i; ++j)
-            if (ctxs[j] == ctxs[i]) return fail(ctxs[0], FQ_ERR_ARG, "fq_kmer_end_pass_all: a context is listed twice");
-    }
-    if (comm && !comm[0]) return fail(ctxs[0], FQ_ERR_ARG, "fq_kmer_end_pass_all: null communicator");
-    const fq_status st = kmer_end_pass_impl(ctxs, n, comm);
-    if (st != FQ_OK) {          // the verdict is the run's: every context reports it
-        std::string msg;
-        for (int i = 0; i < n && msg.empty(); ++i) msg = ctxs[i]->error;
-        for (int i = 0; i < n; ++i) ctxs[i]->error = msg;
-    }
+    return end_pass_entry(ctxs, n, comm, "fq_kmer_end_pass_all", kmer_end_pass_impl);
+}
+
+fq_status fq_dup_enable(fq_ctx *ctx)
+{
+    if (!ctx) return FQ_ERR_ARG;
+    fq_ctx::Dup &D = ctx->dup;
+    if (D.enabled) return D.units ? fail(ctx, FQ_ERR_STATE, "fq_dup_enable: a pass is under way") : FQ_OK;
+    CK(cudaSetDevice(ctx->device));
+    CK(D.T.d_scalars.ensure(64));
+    CK(D.d_small.ensure((size_t)kKmerSmallCounts * 8));
+    CK(D.d_big.ensure((size_t)kKmerBigCap * 4));
+    const fq_status st = table_resize(ctx, D.T, D.T.min_cap);
+    if (st == FQ_OK) D.enabled = true;
     return st;
+}
+
+fq_status fq_dup_end_pass_all(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
+{
+    return end_pass_entry(ctxs, n, comm, "fq_dup_end_pass_all", dup_end_pass_impl);
+}
+
+fq_status fq_dup_results(fq_ctx *ctx, fq_dup_view *view)
+{
+    if (!ctx || !view) return FQ_ERR_ARG;
+    const fq_ctx::Dup &D = ctx->dup;
+    if (!D.enabled) return fail(ctx, FQ_ERR_STATE, "fq_dup_results: duplication statistics are not enabled (fq_dup_enable)");
+    view->units = D.res_units;
+    view->distinct = D.res_distinct;
+    view->n_levels = D.levels.size() / 2;
+    view->levels = D.levels.data();
+    return FQ_OK;
 }
 
 }  // extern "C"

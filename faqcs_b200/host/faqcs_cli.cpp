@@ -61,6 +61,7 @@ struct Cli {
     int device = 0;
     size_t batch_mb = 64;
     bool gz_out = false;            // trimmed reads as blocked gzip (BGZF), deflated by several threads
+    bool dup_stats = false;         // sequence duplication of each input pass -> prefix.duplication.txt
     bool keep_unpaired = false;     // the -u pass appends to prefix.unpaired.trimmed.fastq instead of truncating it (the reference's Q11 quirk, fixed)
     vector<int> devices;            // --devices 0,1,...: consecutive batches go to consecutive GPUs, one NCCL all-reduce at the end
     bool has_paired() const { return !input_read1_file.empty(); }       // has_paired() tests read1 twice, FaQCs.h:135-138
@@ -146,7 +147,8 @@ static void usage()
     cerr << "GPU:\n\t--device\t\t<INT> CUDA device (default 0)\n\t--devices\t\t<INT,INT,..> several CUDA devices: batches are dealt out in order, statistics merged with one NCCL all-reduce\n"
             "\t--batch_mb\t\t<INT> MiB of FASTQ per mate per batch (default 64)\n"
             "Output (extensions):\n\t--gz_out\t\t<bool> write the trimmed reads as blocked gzip (prefix.*.trimmed.fastq.gz), deflated in parallel\n"
-            "\t--keep_unpaired\t\t<bool> with -1/-2 and -u: append the -u pass to prefix.unpaired.trimmed.fastq instead of overwriting it\n";
+            "\t--keep_unpaired\t\t<bool> with -1/-2 and -u: append the -u pass to prefix.unpaired.trimmed.fastq instead of overwriting it\n"
+            "\t--dup_stats\t\t<bool> count identical reads (-u) and read pairs (-1/-2) of each input: prefix.duplication.txt\n";
 }
 
 static void parse_options(int argc, char *argv[], Cli &o)
@@ -171,7 +173,7 @@ static void parse_options(int argc, char *argv[], Cli &o)
         {"qc_only", false, &config_opt, 17}, {"kmer_rarefaction", false, &config_opt, 18}, {"subset", true, &config_opt, 19},
         {"discard", false, &config_opt, 20}, {"substitute", false, &config_opt, 21}, {"trim_only", false, &config_opt, 22},
         {"5trim_off", false, &config_opt, 23}, {"debug", false, &config_opt, 24}, {"version", false, &config_opt, 25}, {"R1", true, &config_opt, 26},
-        {"R2", true, &config_opt, 27}, {"replace_to_N_q", true, &config_opt, 31}, {"device", true, &config_opt, 40}, {"batch_mb", true, &config_opt, 41}, {"devices", true, &config_opt, 42}, {"gz_out", false, &config_opt, 43}, {"keep_unpaired", false, &config_opt, 44},
+        {"R2", true, &config_opt, 27}, {"replace_to_N_q", true, &config_opt, 31}, {"device", true, &config_opt, 40}, {"batch_mb", true, &config_opt, 41}, {"devices", true, &config_opt, 42}, {"gz_out", false, &config_opt, 43}, {"keep_unpaired", false, &config_opt, 44}, {"dup_stats", false, &config_opt, 45},
         {0, 0, 0, 0}};
     int opt_code;
     opterr = 0;
@@ -237,6 +239,7 @@ static void parse_options(int argc, char *argv[], Cli &o)
                     }
                     case 43: o.gz_out = true; break;
                     case 44: o.keep_unpaired = true; break;
+                    case 45: o.dup_stats = true; break;
                     default: cerr << "Unknown flag!" << endl; break;
                 }
                 break;
@@ -754,10 +757,23 @@ struct Run {
             ctxs.push_back(c);
             if (pieces_mode) check(fq_set_output_pieces(c, 1), c);
             if (o.kmer_rarefaction) check(fq_kmer_enable(c, o.kmer, o.split_size, o.num_subsample), c);   // one shard of the pass's table
+            if (o.dup_stats) check(fq_dup_enable(c), c);
         }
     }
     // end of an input's pass: the contexts' k-mer tables merge into the run's curve and histogram (FaQCs.cpp:518-537, 737-756)
     void kmer_end_pass() { check(fq_kmer_end_pass_all(ctxs.data(), (int)ctxs.size(), nullptr)); }
+    // --dup_stats: the contexts' duplication tables merge into the pass's result, one block of prefix.duplication.txt
+    string dup_report;
+    void dup_end_pass(bool paired)
+    {
+        if (!o.dup_stats) return;
+        check(fq_dup_end_pass_all(ctxs.data(), (int)ctxs.size(), nullptr));
+        fq_dup_view v;
+        check(fq_dup_results(ctx, &v));
+        dup_report += string("pass\t") + (paired ? "paired" : "unpaired") + "\tunits\t" + to_string(v.units) + "\tdistinct\t" + to_string(v.distinct) +
+                      "\tduplicates\t" + to_string(v.units - v.distinct) + "\n";
+        for (uint64_t i = 0; i < v.n_levels; ++i) dup_report += to_string(v.levels[2 * i]) + "\t" + to_string(v.levels[2 * i + 1]) + "\n";
+    }
     void set_quality_everywhere(int q) { for (fq_ctx *c : ctxs) check(fq_set_quality(c, q), c); }
 };
 
@@ -1305,6 +1321,7 @@ int main(int argc, char *argv[])
         if (o.devices.empty()) o.devices.push_back(o.device);
         if (fq_create(&f, o.devices[0], &ctx) != FQ_OK) throw string(fq_last_error(nullptr));
         if (o.kmer_rarefaction && fq_kmer_enable(ctx, o.kmer, o.split_size, o.num_subsample) != FQ_OK) throw string(fq_last_error(ctx));
+        if (o.dup_stats && fq_dup_enable(ctx) != FQ_OK) throw string(fq_last_error(ctx));
         const double t_created = now_s();
         Run R(o);
         R.ctx = ctx;
@@ -1316,11 +1333,13 @@ int main(int argc, char *argv[])
         if (o.has_paired()) {
             process(R, true);
             R.kmer_end_pass();                     // FaQCs.cpp:518-537
+            R.dup_end_pass(true);
         }
         if (o.has_unpaired()) {
             R.first_batch = true;      // offset detection only if still unknown; the NextSeq check runs per input (FaQCs.cpp:586,673-683)
             process(R, false);
             R.kmer_end_pass();                     // FaQCs.cpp:737-756
+            R.dup_end_pass(false);
         }
         const double t_processed = now_s();
         if (R.ctxs.size() > 1) {
@@ -1345,6 +1364,13 @@ int main(int argc, char *argv[])
         fq_stats_view v;
         if (fq_stats(ctx, &v) != FQ_OK) throw string(fq_last_error(ctx));
         write_stats(v, o);
+        if (o.dup_stats) {
+            const string fn = o.output_dir + "/" + o.prefix + ".duplication.txt";
+            ofstream fout(fn.c_str());
+            fout << R.dup_report;
+            fout.close();
+            if (!fout) throw string("Unable to write the duplication statistics file: ") + fn;
+        }
         if (!o.trim_only && o.debug) {                           // the reference deletes these unless --debug (plot.cpp:517-537)
             write_debug_files(v, o);
             fq_kmer_view kv;

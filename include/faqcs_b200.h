@@ -374,6 +374,33 @@ fq_status fq_kmer_end_pass(fq_ctx *ctx);
 fq_status fq_kmer_end_pass_all(fq_ctx *const *ctx, int n, fq_comm *const *comm);
 fq_status fq_kmer_results(fq_ctx *ctx, fq_kmer_view *view);
 
+/*
+ * Sequence duplication statistics (not part of FaQCs; the figure FastQC and fastp report).  A unit is a pair (records i of
+ * r1 and r2) of a paired batch, a read of a single-end batch (r2 == NULL).  Every framed record counts, including reads that
+ * trimming or filtering discard: the count depends on no option.  Two units are copies when the bytes of their sequence
+ * lines -- up to the first '\r' or '\n', case-sensitive, before any masking, trimming or G -> N replacement -- are equal.
+ * Each unit is counted as a 64-bit fingerprint of those bytes (defined in fq_dup.cuh): n distinct units give about
+ * n^2 / 2^65 expected pairs of equal fingerprints (0.03 at 10^9 units).
+ *   fq_dup_enable        before the first batch of a pass; afterwards every batch path counts (fq_process_host,
+ *                        fq_submit_host / fq_run / fq_wait, fq_process_device, byte and pieces mode), in any order, on any
+ *                        context, from any first_record_index.  Nothing is allocated and no kernel runs without it.
+ *   fq_dup_end_pass_all  after the last batch of an input: merges the tables of n contexts (n == 1 and comm == NULL for one
+ *                        context; otherwise as for fq_kmer_end_pass_all), publishes the pass's result on every context and
+ *                        clears the tables for the next pass.
+ *   fq_dup_results       the last finished pass; `levels` belongs to the context and stays valid until its next fq_dup_* call.
+ * Duplicate units = units - distinct.  FQ_ERR_STATE for an end of pass or results on a context that never enabled the table;
+ * FQ_ERR_ARG when the contexts of one end of pass differ in whether the table is enabled or in paired versus single-end
+ * units, and for a batch whose kind differs from the earlier batches of the pass on the same context.
+ */
+typedef struct fq_dup_view {
+    uint64_t units, distinct;
+    uint64_t n_levels;                 /* pairs in `levels` */
+    const uint64_t *levels;            /* {multiplicity, distinct keys with that multiplicity}, ascending multiplicity */
+} fq_dup_view;
+fq_status fq_dup_enable(fq_ctx *ctx);
+fq_status fq_dup_end_pass_all(fq_ctx *const *ctx, int n, fq_comm *const *comm);
+fq_status fq_dup_results(fq_ctx *ctx, fq_dup_view *view);
+
 /* Zero the accumulators (new run on the same context). */
 fq_status fq_reset_stats(fq_ctx *ctx);
 
