@@ -108,6 +108,18 @@ class CDupView(C.Structure):
     _fields_ = [("units", C.c_uint64), ("distinct", C.c_uint64), ("n_levels", C.c_uint64), ("levels", C.POINTER(C.c_uint64))]
 
 
+class COverlapView(C.Structure):
+    _fields_ = [("pairs", C.c_uint64), ("too_short", C.c_uint64), ("overlapped", C.c_uint64), ("r1_adapter", C.c_uint64),
+                ("r2_adapter", C.c_uint64), ("overlap_bases", C.c_uint64), ("mismatch_bases", C.c_uint64),
+                ("n_insert", C.c_uint32), ("insert_hist", C.POINTER(C.c_uint64)),
+                ("n_cycles", C.c_uint32), ("r1_overlap", C.POINTER(C.c_uint64)), ("r1_mismatch", C.POINTER(C.c_uint64)),
+                ("r2_overlap", C.POINTER(C.c_uint64)), ("r2_mismatch", C.POINTER(C.c_uint64))]
+
+
+OVERLAP_SCALARS = ("pairs", "too_short", "overlapped", "r1_adapter", "r2_adapter", "overlap_bases", "mismatch_bases")
+OVERLAP_CYCLE_ARRAYS = ("r1_overlap", "r1_mismatch", "r2_overlap", "r2_mismatch")
+
+
 class CStatsView(C.Structure):
     _fields_ = [
         ("filter_stats", C.c_uint64 * NUM_STAT), ("n_adapters", C.c_uint32),
@@ -326,6 +338,9 @@ class Engine:
             L.fq_dup_enable.argtypes = [C.c_void_p]
             L.fq_dup_end_pass_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
             L.fq_dup_results.argtypes = [C.c_void_p, C.POINTER(CDupView)]
+            L.fq_overlap_enable.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]
+            L.fq_overlap_end_pass_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
+            L.fq_overlap_results.argtypes = [C.c_void_p, C.POINTER(COverlapView)]
             L.fq_last_allreduce_ms.argtypes = [C.c_void_p]
             L.fq_last_allreduce_ms.restype = C.c_float
             L.fq_device_outputs.argtypes = [C.c_void_p, C.POINTER(C.c_void_p * NUM_STREAM)]
@@ -404,6 +419,30 @@ class Engine:
         if v.n_levels:
             levels[:] = np.ctypeslib.as_array(v.levels, (v.n_levels, 2))
         return {"units": int(v.units), "distinct": int(v.distinct), "levels": levels}
+
+    def overlap_enable(self, min_overlap: int = 30, diff_limit: int = 5, diff_percent: int = 20):
+        """Insert size and overlap error profile (fq_overlap_enable): every pair of the following paired batches is searched for
+        the overlap of R1 with reverse-complemented R2.  Call before the first batch of a pass."""
+        self._check(self.lib.fq_overlap_enable(self.ctx, int(min_overlap), int(diff_limit), int(diff_percent)))
+
+    def overlap_end_pass(self):
+        """End of one input's pass on this context alone (fq_overlap_end_pass_all with n = 1); dist_stats has the other forms."""
+        ctxs = (C.c_void_p * 1)(self.ctx)
+        self._check(self.lib.fq_overlap_end_pass_all(ctxs, 1, None))
+
+    def overlap_results(self) -> dict:
+        """The last finished pass: the scalars of OVERLAP_SCALARS as ints, "insert_hist" (index = insert size) and the four
+        OVERLAP_CYCLE_ARRAYS (index = 0-based cycle) as uint64 arrays without trailing zeros."""
+        v = COverlapView()
+        self._check(self.lib.fq_overlap_results(self.ctx, C.byref(v)))
+        out = {k: int(getattr(v, k)) for k in OVERLAP_SCALARS}
+
+        def arr(p, n):
+            return np.ctypeslib.as_array(p, (n,)).copy() if n else np.zeros(0, np.uint64)
+        out["insert_hist"] = arr(v.insert_hist, v.n_insert)
+        for k in OVERLAP_CYCLE_ARRAYS:
+            out[k] = arr(getattr(v, k), v.n_cycles)
+        return out
 
     def set_quality(self, quality: int):
         """Options::quality for the following batches (the reference's NextSeq adjustment, FaQCs.cpp:272-277)."""

@@ -25,6 +25,7 @@
 #include "fq_emit.cuh"
 #include "fq_frame.cuh"
 #include "fq_kmer.cuh"
+#include "fq_overlap.cuh"
 #include "fq_trim.cuh"
 
 using namespace fq;
@@ -160,6 +161,18 @@ struct fq_ctx {
         uint64_t res_units = 0, res_distinct = 0;  // the last finished pass (fq_dup_view)
         std::vector<uint64_t> levels;
     } dup;
+
+    // insert size and overlap error profile (fq_overlap_*, fq_overlap.cuh): per-pair overlap of R1 with reverse-complemented R2
+    struct Overlap {
+        bool enabled = false;
+        uint32_t min_overlap = 30, diff_limit = 5, diff_percent = 20;
+        uint32_t cyc = 0;                          // cycle capacity of d_acc (OverlapLayout; 0: nothing allocated yet)
+        uint64_t pairs = 0;                        // pairs of the current pass counted here
+        DevBuf d_acc, d_scratch;
+        // the last finished pass (fq_overlap_view): scalars, insert-size histogram, per-cycle arrays
+        uint64_t res[kOvlPairs + 1] = {};
+        std::vector<uint64_t> ins, r1o, r1m, r2o, r2m;
+    } ovl;
 
     // host-side stats views handed out by fq_stats
     std::vector<uint64_t> v_adapter_reads, v_adapter_bases, v_pre_q, v_post_q, v_pre_b, v_post_b, v_hist[4], v_pre_comp,
@@ -605,6 +618,68 @@ fq_status dup_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint3
     return FQ_OK;
 }
 
+// Host copy of an accumulator block of capacity `from` added into one of capacity `to` >= from, section by section.
+void overlap_add_relaid(const uint64_t *src, uint32_t from, uint64_t *dst, uint32_t to)
+{
+    const OverlapLayout a = OverlapLayout::make(from), b = OverlapLayout::make(to);
+    const uint32_t so[6] = {0, a.ins, a.d1, a.d2, a.m1, a.m2}, dO[6] = {0, b.ins, b.d1, b.d2, b.m1, b.m2};
+    const uint32_t len[6] = {kOvlScalars, 2 * from, from + 1, from + 1, from, from};
+    for (int k = 0; k < 6; ++k)
+        for (uint32_t i = 0; i < len[k]; ++i) dst[dO[k] + i] += src[so[k] + i];
+}
+
+// One paired batch of the overlap profile: the accumulators grown (contents kept) to the batch's longest mate, then k_overlap.
+fq_status overlap_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint32_t n, uint32_t max_len)
+{
+    fq_ctx::Overlap &V = ctx->ovl;
+    if (!V.d_acc.p || max_len > V.cyc) {
+        const uint32_t C = std::max(64u, round_up(max_len, 64));
+        const OverlapLayout L = OverlapLayout::make(C);
+        std::vector<uint64_t> h(L.total, 0);
+        if (V.cyc) {
+            std::vector<uint64_t> old(OverlapLayout::make(V.cyc).total);
+            CK(cudaMemcpyAsync(old.data(), V.d_acc.p, old.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
+            overlap_add_relaid(old.data(), V.cyc, h.data(), C);
+        }
+        DevBuf nb;
+        CK(nb.ensure((size_t)L.total * 8));
+        CK(cudaMemcpy(nb.p, h.data(), h.size() * 8, cudaMemcpyHostToDevice));
+        V.d_acc = std::move(nb);
+        V.cyc = C;
+    }
+    OverlapArgs oa{};
+    oa.raw[0] = d_r1; oa.raw[1] = d_r2;
+    oa.rec[0] = ctx->d_rec[0].as<Rec>(); oa.rec[1] = ctx->d_rec[1].as<Rec>();
+    oa.n_rec = n;
+    oa.min_overlap = V.min_overlap; oa.diff_limit = V.diff_limit; oa.diff_percent = V.diff_percent;
+    oa.L = OverlapLayout::make(V.cyc);
+    oa.acc = V.d_acc.as<unsigned long long>();
+    oa.wa = (max_len + 31) / 32;
+    oa.plane_words = 2 * oa.wa + 2;                // b: one word of padding in front, one behind
+    const size_t per_warp = (size_t)oa.plane_words * sizeof(uint4), counters = (size_t)oa.L.total * 4;
+    const size_t budget = std::min<size_t>(ctx->smem_optin, 200 * 1024);
+    int warps = kOvlThreads / 32;
+    while (warps > 1 && counters + warps * per_warp > budget) warps >>= 1;
+    if (counters + warps * per_warp <= budget) {
+        const size_t smem = counters + warps * per_warp;
+        CK(allow_dynamic_smem(ctx, reinterpret_cast<const void *>(k_overlap<true>)));
+        int per_sm = 1;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_overlap<true>, warps * 32, smem));
+        const int grid = std::max(1, std::min<int>((n + warps - 1) / warps, ctx->sm_count * std::max(per_sm, 1)));
+        k_overlap<true><<<grid, warps * 32, smem, ctx->stream>>>(oa);
+    } else {
+        // mates too long for shared memory: planes in global scratch (at most 256 MiB of it), counters straight to the block
+        const uint32_t total_warps = (uint32_t)std::max<size_t>(1, std::min<size_t>({(size_t)n, (size_t)ctx->sm_count * 32, ((size_t)256 << 20) / per_warp}));
+        CK(V.d_scratch.ensure(total_warps * per_warp));
+        oa.scratch = V.d_scratch.as<uint4>();
+        k_overlap<false><<<total_warps, 32, 0, ctx->stream>>>(oa);
+    }
+    ctx->launches++;
+    V.pairs += n;
+    return FQ_OK;
+}
+
 // Outputs go to the d_out / h_out set `slot`.  With async_copy the D2H runs on s_out and the caller waits on ev_out.
 fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint8_t *d_r2, size_t n2, bool paired,
                          uint64_t first_record_index, int is_final, int copy_out, int slot, bool async_copy, fq_batch_out *out)
@@ -785,6 +860,11 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
     // ---- duplication statistics: the sequence lines as framed
     if (ctx->dup.enabled) {
         st = dup_batch(ctx, d_r1, d_r2, n, n_mates);
+        if (st != FQ_OK) return st;
+    }
+    // ---- insert size and overlap error profile: paired batches, the sequence lines as framed
+    if (ctx->ovl.enabled && paired) {
+        st = overlap_batch(ctx, d_r1, d_r2, n, max_len);
         if (st != FQ_OK) return st;
     }
 
@@ -1965,6 +2045,88 @@ fq_status dup_end_pass_impl(fq_ctx *const *ctxs, int n, const fq_comm *cm, uint3
     return FQ_OK;
 }
 
+// ---- insert size and overlap error profile: end of a pass, over one context or several ---------------------------------
+// Every context's block, laid out for the largest capacity of any of them, is summed (on the host, or one ncclAllReduce
+// across ranks); the sum is published on every context and the accumulators are cleared.
+fq_status overlap_end_pass_impl(fq_ctx *const *ctxs, int n, const fq_comm *cm, uint32_t n_shards, uint32_t rank0)
+{
+    fq_ctx *const ctx0 = ctxs[0];
+    fq_status st = sync_all(ctxs, n);
+    if (st != FQ_OK) return st;
+    // 1. agree on the parameters and the capacity: header {enabled, min_overlap, diff_limit, diff_percent, capacity}
+    const size_t H = 5;
+    std::vector<uint64_t> head((size_t)n_shards * H, 0);
+    for (int i = 0; i < n; ++i) {
+        const fq_ctx::Overlap &V = ctxs[i]->ovl;
+        uint64_t *h = head.data() + (size_t)(rank0 + i) * H;
+        h[0] = V.enabled; h[1] = V.min_overlap; h[2] = V.diff_limit; h[3] = V.diff_percent; h[4] = V.cyc;
+    }
+    if (cm) {
+        const std::vector<uint64_t> mine(head.begin() + (size_t)rank0 * H, head.begin() + (size_t)(rank0 + 1) * H);
+        st = nccl_allgather_u64(ctx0, cm, mine, &head);
+        if (st != FQ_OK) return st;
+    }
+    uint64_t enabled = 0, cap = 0;
+    for (uint32_t j = 0; j < n_shards; ++j) {
+        const uint64_t *h = head.data() + (size_t)j * H;
+        enabled += h[0];
+        cap = std::max(cap, h[4]);
+    }
+    if (!enabled) return fail(ctx0, FQ_ERR_STATE, "fq_overlap_end_pass_all: the overlap profile is not enabled (fq_overlap_enable)");
+    if (enabled != n_shards) return fail(ctx0, FQ_ERR_ARG, "fq_overlap_end_pass_all: the overlap profile is enabled on some contexts only");
+    for (uint32_t j = 1; j < n_shards; ++j) {
+        const uint64_t *a = head.data(), *b = head.data() + (size_t)j * H;
+        if (a[1] != b[1] || a[2] != b[2] || a[3] != b[3]) {
+            char msg[240];
+            snprintf(msg, sizeof msg, "fq_overlap_end_pass_all: context %u has min_overlap = %llu, diff_limit = %llu, diff_percent = %llu; context 0 "
+                     "min_overlap = %llu, diff_limit = %llu, diff_percent = %llu", j, (unsigned long long)b[1], (unsigned long long)b[2],
+                     (unsigned long long)b[3], (unsigned long long)a[1], (unsigned long long)a[2], (unsigned long long)a[3]);
+            return fail(ctx0, FQ_ERR_ARG, msg);
+        }
+    }
+    // 2. sum the blocks
+    const uint32_t C = (uint32_t)cap;
+    const OverlapLayout L = OverlapLayout::make(C);
+    std::vector<uint64_t> sum(L.total, 0), blk;
+    for (int i = 0; i < n; ++i) {
+        fq_ctx *const ctx = ctxs[i];
+        fq_ctx::Overlap &V = ctx->ovl;
+        sum[kOvlPairs] += V.pairs;
+        if (!V.cyc) continue;
+        blk.assign(OverlapLayout::make(V.cyc).total, 0);
+        CK(cudaSetDevice(ctx->device));
+        CK(cudaMemcpy(blk.data(), V.d_acc.p, blk.size() * 8, cudaMemcpyDeviceToHost));
+        overlap_add_relaid(blk.data(), V.cyc, sum.data(), C);
+    }
+    if (cm) {
+        st = nccl_sum_u64(ctx0, cm, &sum);
+        if (st != FQ_OK) return st;
+    }
+    // 3. the result: difference arrays prefix-summed, trailing zero entries dropped; the same on every context
+    std::vector<uint64_t> ins(sum.begin() + L.ins, sum.begin() + L.ins + 2 * C), r1o(C), r2o(C), r1m(sum.begin() + L.m1, sum.begin() + L.m1 + C),
+        r2m(sum.begin() + L.m2, sum.begin() + L.m2 + C);
+    for (uint32_t x = 0; x < C; ++x) {
+        r1o[x] = (x ? r1o[x - 1] : 0) + sum[L.d1 + x];
+        r2o[x] = (x ? r2o[x - 1] : 0) + sum[L.d2 + x];
+    }
+    auto trimmed = [](std::vector<uint64_t> &v) { while (!v.empty() && !v.back()) v.pop_back(); return v.size(); };
+    trimmed(ins);
+    const size_t n_cyc = std::max({trimmed(r1o), trimmed(r2o), trimmed(r1m), trimmed(r2m)});
+    for (auto *v : {&r1o, &r2o, &r1m, &r2m}) v->resize(n_cyc, 0);
+    for (int i = 0; i < n; ++i) {
+        fq_ctx *const ctx = ctxs[i];
+        fq_ctx::Overlap &V = ctx->ovl;
+        std::copy(sum.begin(), sum.begin() + kOvlPairs + 1, V.res);
+        V.ins = ins; V.r1o = r1o; V.r1m = r1m; V.r2o = r2o; V.r2m = r2m;
+        V.pairs = 0;
+        if (V.cyc) {
+            CK(cudaSetDevice(ctx->device));
+            CK(cudaMemset(V.d_acc.p, 0, (size_t)OverlapLayout::make(V.cyc).total * 8));
+        }
+    }
+    return FQ_OK;
+}
+
 }  // namespace
 
 fq_status fq_kmer_end_pass_all(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
@@ -2000,6 +2162,45 @@ fq_status fq_dup_results(fq_ctx *ctx, fq_dup_view *view)
     view->distinct = D.res_distinct;
     view->n_levels = D.levels.size() / 2;
     view->levels = D.levels.data();
+    return FQ_OK;
+}
+
+fq_status fq_overlap_enable(fq_ctx *ctx, uint32_t min_overlap, uint32_t diff_limit, uint32_t diff_percent)
+{
+    if (!ctx) return FQ_ERR_ARG;
+    if (min_overlap == 0 || diff_percent > 100)
+        return fail(ctx, FQ_ERR_ARG, "fq_overlap_enable: min_overlap must be at least 1 and diff_percent at most 100");
+    fq_ctx::Overlap &V = ctx->ovl;
+    if (V.enabled && V.pairs) return fail(ctx, FQ_ERR_STATE, "fq_overlap_enable: a pass is under way");
+    V.enabled = true;
+    V.min_overlap = min_overlap; V.diff_limit = diff_limit; V.diff_percent = diff_percent;
+    return FQ_OK;
+}
+
+fq_status fq_overlap_end_pass_all(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
+{
+    return end_pass_entry(ctxs, n, comm, "fq_overlap_end_pass_all", overlap_end_pass_impl);
+}
+
+fq_status fq_overlap_results(fq_ctx *ctx, fq_overlap_view *view)
+{
+    if (!ctx || !view) return FQ_ERR_ARG;
+    const fq_ctx::Overlap &V = ctx->ovl;
+    if (!V.enabled) return fail(ctx, FQ_ERR_STATE, "fq_overlap_results: the overlap profile is not enabled (fq_overlap_enable)");
+    view->pairs = V.res[kOvlPairs];
+    view->too_short = V.res[kOvlTooShort];
+    view->overlapped = V.res[kOvlOverlapped];
+    view->r1_adapter = V.res[kOvlR1Adapter];
+    view->r2_adapter = V.res[kOvlR2Adapter];
+    view->overlap_bases = V.res[kOvlOverlapBases];
+    view->mismatch_bases = V.res[kOvlMismatchBases];
+    view->n_insert = (uint32_t)V.ins.size();
+    view->insert_hist = V.ins.data();
+    view->n_cycles = (uint32_t)V.r1o.size();
+    view->r1_overlap = V.r1o.data();
+    view->r1_mismatch = V.r1m.data();
+    view->r2_overlap = V.r2o.data();
+    view->r2_mismatch = V.r2m.data();
     return FQ_OK;
 }
 

@@ -62,6 +62,9 @@ struct Cli {
     size_t batch_mb = 64;
     bool gz_out = false;            // trimmed reads as blocked gzip (BGZF), deflated by several threads
     bool dup_stats = false;         // sequence duplication of each input pass -> prefix.duplication.txt
+    bool insert_size = false;       // insert size and overlap error profile of the paired pass -> prefix.insert_size.txt
+    long long insert_min_overlap = 30, insert_diff_limit = 5, insert_diff_pct = 20;    // checked after parsing
+    bool insert_bad_number = false;
     bool keep_unpaired = false;     // the -u pass appends to prefix.unpaired.trimmed.fastq instead of truncating it (the reference's Q11 quirk, fixed)
     vector<int> devices;            // --devices 0,1,...: consecutive batches go to consecutive GPUs, one NCCL all-reduce at the end
     bool has_paired() const { return !input_read1_file.empty(); }       // has_paired() tests read1 twice, FaQCs.h:135-138
@@ -148,7 +151,12 @@ static void usage()
             "\t--batch_mb\t\t<INT> MiB of FASTQ per mate per batch (default 64)\n"
             "Output (extensions):\n\t--gz_out\t\t<bool> write the trimmed reads as blocked gzip (prefix.*.trimmed.fastq.gz), deflated in parallel\n"
             "\t--keep_unpaired\t\t<bool> with -1/-2 and -u: append the -u pass to prefix.unpaired.trimmed.fastq instead of overwriting it\n"
-            "\t--dup_stats\t\t<bool> count identical reads (-u) and read pairs (-1/-2) of each input: prefix.duplication.txt\n";
+            "\t--dup_stats\t\t<bool> count identical reads (-u) and read pairs (-1/-2) of each input: prefix.duplication.txt\n"
+            "\t--insert_size\t\t<bool> with -1/-2: insert size of each pair from the overlap of R1 with reverse-complemented R2,\n"
+            "\t\t\t\tadapter read-through and mismatches per cycle in the overlap: prefix.insert_size.txt\n"
+            "\t--insert_min_overlap\t<INT> shortest overlap tested (default 30, at least 1)\n"
+            "\t--insert_diff_limit\t<INT> most mismatches in an accepted overlap (default 5)\n"
+            "\t--insert_diff_pct\t<INT> most mismatches in an accepted overlap, in percent of its length (default 20, 0-100)\n";
 }
 
 static void parse_options(int argc, char *argv[], Cli &o)
@@ -174,6 +182,8 @@ static void parse_options(int argc, char *argv[], Cli &o)
         {"discard", false, &config_opt, 20}, {"substitute", false, &config_opt, 21}, {"trim_only", false, &config_opt, 22},
         {"5trim_off", false, &config_opt, 23}, {"debug", false, &config_opt, 24}, {"version", false, &config_opt, 25}, {"R1", true, &config_opt, 26},
         {"R2", true, &config_opt, 27}, {"replace_to_N_q", true, &config_opt, 31}, {"device", true, &config_opt, 40}, {"batch_mb", true, &config_opt, 41}, {"devices", true, &config_opt, 42}, {"gz_out", false, &config_opt, 43}, {"keep_unpaired", false, &config_opt, 44}, {"dup_stats", false, &config_opt, 45},
+        {"insert_size", false, &config_opt, 46}, {"insert_min_overlap", true, &config_opt, 47}, {"insert_diff_limit", true, &config_opt, 48},
+        {"insert_diff_pct", true, &config_opt, 49},
         {0, 0, 0, 0}};
     int opt_code;
     opterr = 0;
@@ -240,6 +250,15 @@ static void parse_options(int argc, char *argv[], Cli &o)
                     case 43: o.gz_out = true; break;
                     case 44: o.keep_unpaired = true; break;
                     case 45: o.dup_stats = true; break;
+                    case 46: o.insert_size = true; break;
+                    case 47: case 48: case 49: {
+                        char *end = nullptr;
+                        errno = 0;
+                        const long long v = strtoll(optarg, &end, 10);
+                        if (end == optarg || *end || errno) o.insert_bad_number = true;
+                        (config_opt == 47 ? o.insert_min_overlap : config_opt == 48 ? o.insert_diff_limit : o.insert_diff_pct) = v;
+                        break;
+                    }
                     default: cerr << "Unknown flag!" << endl; break;
                 }
                 break;
@@ -290,6 +309,18 @@ static void parse_options(int argc, char *argv[], Cli &o)
     }
     if (o.num_subsample == 0) {
         cerr << "Please specify a subset (--subset) value greater than 0" << endl;
+        o.print_usage = true;
+        return;
+    }
+    if (o.insert_size && !o.has_paired()) {
+        cerr << "--insert_size needs paired reads (-1 <file> -2 <file>): the insert size is measured on the overlap of the two mates" << endl;
+        o.print_usage = true;
+        return;
+    }
+    if (o.insert_bad_number || o.insert_min_overlap < 1 || o.insert_min_overlap > UINT_MAX || o.insert_diff_limit < 0 || o.insert_diff_limit > UINT_MAX ||
+        o.insert_diff_pct < 0 || o.insert_diff_pct > 100) {
+        cerr << "Please specify --insert_min_overlap as an integer >= 1, --insert_diff_limit as an integer >= 0 and --insert_diff_pct as an integer "
+                "in the range 0 <= percent <= 100" << endl;
         o.print_usage = true;
         return;
     }
@@ -758,6 +789,7 @@ struct Run {
             if (pieces_mode) check(fq_set_output_pieces(c, 1), c);
             if (o.kmer_rarefaction) check(fq_kmer_enable(c, o.kmer, o.split_size, o.num_subsample), c);   // one shard of the pass's table
             if (o.dup_stats) check(fq_dup_enable(c), c);
+            if (o.insert_size) check(fq_overlap_enable(c, (uint32_t)o.insert_min_overlap, (uint32_t)o.insert_diff_limit, (uint32_t)o.insert_diff_pct), c);
         }
     }
     // end of an input's pass: the contexts' k-mer tables merge into the run's curve and histogram (FaQCs.cpp:518-537, 737-756)
@@ -773,6 +805,26 @@ struct Run {
         dup_report += string("pass\t") + (paired ? "paired" : "unpaired") + "\tunits\t" + to_string(v.units) + "\tdistinct\t" + to_string(v.distinct) +
                       "\tduplicates\t" + to_string(v.units - v.distinct) + "\n";
         for (uint64_t i = 0; i < v.n_levels; ++i) dup_report += to_string(v.levels[2 * i]) + "\t" + to_string(v.levels[2 * i + 1]) + "\n";
+    }
+    // --insert_size: the contexts' overlap accumulators summed after the paired pass, the text of prefix.insert_size.txt
+    string insert_report;
+    void overlap_end_pass()
+    {
+        if (!o.insert_size) return;
+        check(fq_overlap_end_pass_all(ctxs.data(), (int)ctxs.size(), nullptr));
+        fq_overlap_view v;
+        check(fq_overlap_results(ctx, &v));
+        const pair<const char *, uint64_t> totals[] = {{"pairs", v.pairs}, {"too_short", v.too_short}, {"overlapped", v.overlapped},
+                                                       {"r1_adapter", v.r1_adapter}, {"r2_adapter", v.r2_adapter},
+                                                       {"overlap_bases", v.overlap_bases}, {"mismatch_bases", v.mismatch_bases}};
+        for (const auto &t : totals) insert_report += string(t.first) + "\t" + to_string(t.second) + "\n";
+        insert_report += "#insert_size\tpairs\n";
+        for (uint32_t s = 0; s < v.n_insert; ++s)
+            if (v.insert_hist[s]) insert_report += to_string(s) + "\t" + to_string(v.insert_hist[s]) + "\n";
+        insert_report += "#cycle\tr1_overlap\tr1_mismatch\tr2_overlap\tr2_mismatch\n";
+        for (uint32_t c = 0; c < v.n_cycles; ++c)
+            insert_report += to_string(c + 1) + "\t" + to_string(v.r1_overlap[c]) + "\t" + to_string(v.r1_mismatch[c]) + "\t" +
+                             to_string(v.r2_overlap[c]) + "\t" + to_string(v.r2_mismatch[c]) + "\n";
     }
     void set_quality_everywhere(int q) { for (fq_ctx *c : ctxs) check(fq_set_quality(c, q), c); }
 };
@@ -1322,6 +1374,8 @@ int main(int argc, char *argv[])
         if (fq_create(&f, o.devices[0], &ctx) != FQ_OK) throw string(fq_last_error(nullptr));
         if (o.kmer_rarefaction && fq_kmer_enable(ctx, o.kmer, o.split_size, o.num_subsample) != FQ_OK) throw string(fq_last_error(ctx));
         if (o.dup_stats && fq_dup_enable(ctx) != FQ_OK) throw string(fq_last_error(ctx));
+        if (o.insert_size && fq_overlap_enable(ctx, (uint32_t)o.insert_min_overlap, (uint32_t)o.insert_diff_limit, (uint32_t)o.insert_diff_pct) != FQ_OK)
+            throw string(fq_last_error(ctx));
         const double t_created = now_s();
         Run R(o);
         R.ctx = ctx;
@@ -1334,6 +1388,7 @@ int main(int argc, char *argv[])
             process(R, true);
             R.kmer_end_pass();                     // FaQCs.cpp:518-537
             R.dup_end_pass(true);
+            R.overlap_end_pass();
         }
         if (o.has_unpaired()) {
             R.first_batch = true;      // offset detection only if still unknown; the NextSeq check runs per input (FaQCs.cpp:586,673-683)
@@ -1370,6 +1425,13 @@ int main(int argc, char *argv[])
             fout << R.dup_report;
             fout.close();
             if (!fout) throw string("Unable to write the duplication statistics file: ") + fn;
+        }
+        if (o.insert_size) {
+            const string fn = o.output_dir + "/" + o.prefix + ".insert_size.txt";
+            ofstream fout(fn.c_str());
+            fout << R.insert_report;
+            fout.close();
+            if (!fout) throw string("Unable to write the insert size file: ") + fn;
         }
         if (!o.trim_only && o.debug) {                           // the reference deletes these unless --debug (plot.cpp:517-537)
             write_debug_files(v, o);

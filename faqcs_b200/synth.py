@@ -229,6 +229,43 @@ def shotgun(n_pairs: int, genome_len: int = 60000, seed: int = 77, start: int = 
     return Workload("shotgun", mates[0], mates[1] if paired else None, ["--kmer_rarefaction"])
 
 
+def fragments(n_pairs: int, seed: int = 91, start: int = 0, L: int = 150, mean: float = 200.0, sd: float = 50.0) -> Workload:
+    """Paired reads sequenced from both ends of fragments, the workload of --insert_size: R1 is the fragment's start, R2 the
+    reverse complement of its end.  Insert sizes: 70 % normal(mean, sd), 15 % shorter than the read (both mates run into
+    their Nextera adapter, then random bases), 10 % between L and 2L, 5 % too long for the mates to overlap.  Then 0.5 %
+    substitutions and 0.2 % N per mate, 2 % lowercase mates, and 5 % of the pairs with one mate cut to 1..L bases."""
+    rng = np.random.default_rng(seed + start)
+    kind = rng.random(n_pairs)
+    f = np.rint(rng.normal(mean, sd, size=n_pairs)).astype(np.int64)
+    f = np.where(kind >= 0.70, rng.integers(10, L, size=n_pairs), f)
+    f = np.where(kind >= 0.85, rng.integers(L, 2 * L, size=n_pairs), f)
+    f = np.where(kind >= 0.95, rng.integers(2 * L, 3 * L, size=n_pairs), f)
+    f = np.clip(f, 10, 3 * L)
+    W = 3 * L
+    frag = _BASES[rng.integers(0, 4, size=(n_pairs, W))]
+    comp = np.zeros(256, dtype=np.uint8)
+    comp[list(b"ACGT")] = list(b"TGCA")
+    col = np.arange(L)[None, :]
+    rows = np.arange(n_pairs)[:, None]
+    mates = []
+    for mate in (1, 2):
+        ad = np.frombuffer(dict(BUILTIN_ADAPTERS)[f"Nextera-primer-adapter-{mate}"].encode(), dtype=np.uint8)
+        tail = np.concatenate([np.broadcast_to(ad, (n_pairs, ad.size)), _BASES[rng.integers(0, 4, size=(n_pairs, L))]], 1)
+        inside = col < f[:, None]
+        if mate == 1:
+            body = frag[rows, np.minimum(col, W - 1)]
+        else:
+            body = comp[frag[rows, np.clip(f[:, None] - 1 - col, 0, W - 1)]]
+        s = np.where(inside, body, tail[rows, np.clip(col - f[:, None], 0, tail.shape[1] - 1)])
+        s = np.where(rng.random((n_pairs, L)) < 0.005, _BASES[rng.integers(0, 4, size=(n_pairs, L))], s)
+        s = np.where(rng.random((n_pairs, L)) < 0.002, np.uint8(ord("N")), s)
+        s = np.where((rng.random(n_pairs) < 0.02)[:, None], s | 0x20, s)
+        lengths = np.where((rng.random(n_pairs) < 0.025), rng.integers(1, L + 1, size=n_pairs), L)
+        q = _qualities(rng, n_pairs, L, 30, 40, 0.12, 3.0, 2, 41, 0.10, 59)
+        mates.append(_assemble(_headers(n_pairs, "FR", mate, start), s, q + 33, lengths))
+    return Workload("fragments", mates[0], mates[1], [])
+
+
 def fastq_bytes(records: List[Tuple[str, str, str]], eol: str = "\n") -> bytes:
     """Hand-written records -> FASTQ bytes (micro-cases)."""
     return "".join(f"{h}{eol}{s}{eol}+{eol}{q}{eol}" for h, s, q in records).encode()

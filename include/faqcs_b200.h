@@ -401,6 +401,38 @@ fq_status fq_dup_enable(fq_ctx *ctx);
 fq_status fq_dup_end_pass_all(fq_ctx *const *ctx, int n, fq_comm *const *comm);
 fq_status fq_dup_results(fq_ctx *ctx, fq_dup_view *view);
 
+/*
+ * Paired-end insert size and overlap error profile (not part of FaQCs).  For every pair of a paired batch (records i of r1
+ * and r2, including pairs that trimming or filtering discard: the result depends on no option) the library looks for the
+ * overlap of R1 with the reverse complement of R2, both as framed (up to the first '\r' or '\n').  A, C, G, T in either case
+ * are known bases; every other byte is unknown, and a position matches only when both bases are known and equal.  A
+ * candidate insert size s puts R1 on fragment positions [0, L1) and reverse-complemented R2 on [s - L2, s); candidates have
+ * an overlap o(s) of at least min_overlap positions, and s is accepted when its mismatches m(s) <= min(diff_limit,
+ * floor(o(s) * diff_percent / 100)).  The pair's insert size is the accepted s with the fewest mismatches, then the longest
+ * overlap, then the smallest s (this selection rule is the library's own; the defaults 30 / 5 / 20 are fastp's).  Per
+ * overlapped pair: insert_hist[s] += 1; r1_adapter += s < L1, r2_adapter += s < L2 (the mate reads into adapter);
+ * overlap_bases += o(s), mismatch_bases += m(s); overlap position x is R1 cycle x and R2 cycle s - 1 - x (0-based), each
+ * counted in r*_overlap and, where the bases disagree, in r*_mismatch.  too_short counts pairs with a mate shorter than
+ * min_overlap.  Arrays end at their last non-zero entry (n_cycles: the longest of the four).
+ *   fq_overlap_enable        before the first batch of a pass (FQ_ERR_STATE in the middle of one); FQ_ERR_ARG for
+ *                            min_overlap == 0 or diff_percent > 100.  Afterwards every batch path counts paired batches;
+ *                            single-end batches are neither counted nor refused.  Nothing is allocated and no kernel runs
+ *                            without it.
+ *   fq_overlap_end_pass_all  after the last batch of an input: sums the accumulators of n contexts (n == 1 and comm == NULL
+ *                            for one context; one context per rank with comm), publishes the pass's result on every context
+ *                            and clears the accumulators.  FQ_ERR_ARG when the contexts differ in enablement or parameters.
+ *   fq_overlap_results       the last finished pass; the pointers belong to the context and stay valid until its next
+ *                            fq_overlap_* call.  FQ_ERR_STATE (also for an end of pass) on a context that never enabled it.
+ */
+typedef struct fq_overlap_view {
+    uint64_t pairs, too_short, overlapped, r1_adapter, r2_adapter, overlap_bases, mismatch_bases;
+    uint32_t n_insert;   const uint64_t *insert_hist;           /* index = insert size */
+    uint32_t n_cycles;   const uint64_t *r1_overlap, *r1_mismatch, *r2_overlap, *r2_mismatch;   /* index = 0-based cycle */
+} fq_overlap_view;
+fq_status fq_overlap_enable(fq_ctx *ctx, uint32_t min_overlap, uint32_t diff_limit, uint32_t diff_percent);
+fq_status fq_overlap_end_pass_all(fq_ctx *const *ctx, int n, fq_comm *const *comm);
+fq_status fq_overlap_results(fq_ctx *ctx, fq_overlap_view *view);
+
 /* Zero the accumulators (new run on the same context). */
 fq_status fq_reset_stats(fq_ctx *ctx);
 
