@@ -116,6 +116,15 @@ class COverlapView(C.Structure):
                 ("r2_overlap", C.POINTER(C.c_uint64)), ("r2_mismatch", C.POINTER(C.c_uint64))]
 
 
+class COverrepSeq(C.Structure):
+    _fields_ = [("count", C.c_uint64), ("mate", C.c_uint32), ("len", C.c_uint32), ("offset", C.c_uint64)]
+
+
+class COverrepView(C.Structure):
+    _fields_ = [("prefix_len", C.c_uint32), ("min_ppm", C.c_uint32), ("reads", C.c_uint64 * 2), ("min_count", C.c_uint64 * 2),
+                ("n_seqs", C.c_uint64), ("seqs", C.POINTER(COverrepSeq)), ("bytes", C.POINTER(C.c_uint8))]
+
+
 OVERLAP_SCALARS = ("pairs", "too_short", "overlapped", "r1_adapter", "r2_adapter", "overlap_bases", "mismatch_bases")
 OVERLAP_CYCLE_ARRAYS = ("r1_overlap", "r1_mismatch", "r2_overlap", "r2_mismatch")
 
@@ -341,6 +350,9 @@ class Engine:
             L.fq_overlap_enable.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]
             L.fq_overlap_end_pass_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
             L.fq_overlap_results.argtypes = [C.c_void_p, C.POINTER(COverlapView)]
+            L.fq_overrep_enable.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32]
+            L.fq_overrep_end_pass_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
+            L.fq_overrep_results.argtypes = [C.c_void_p, C.POINTER(COverrepView)]
             L.fq_last_allreduce_ms.argtypes = [C.c_void_p]
             L.fq_last_allreduce_ms.restype = C.c_float
             L.fq_device_outputs.argtypes = [C.c_void_p, C.POINTER(C.c_void_p * NUM_STREAM)]
@@ -443,6 +455,28 @@ class Engine:
         for k in OVERLAP_CYCLE_ARRAYS:
             out[k] = arr(getattr(v, k), v.n_cycles)
         return out
+
+    def overrep_enable(self, prefix_len: int = 50, min_ppm: int = 1000):
+        """Overrepresented sequences (fq_overrep_enable): the first prefix_len bytes of every read of the following batches are
+        counted, each mate on its own.  Call before the first batch of a pass."""
+        self._check(self.lib.fq_overrep_enable(self.ctx, int(prefix_len), int(min_ppm)))
+
+    def overrep_end_pass(self):
+        """End of one input's pass on this context alone (fq_overrep_end_pass_all with n = 1); dist_stats has the sharded forms."""
+        ctxs = (C.c_void_p * 1)(self.ctx)
+        self._check(self.lib.fq_overrep_end_pass_all(ctxs, 1, None))
+
+    def overrep_results(self) -> dict:
+        """The last finished pass: {"prefix_len", "min_ppm", "reads": [mate 1, mate 2], "min_count": [mate 1, mate 2],
+        "seqs": [(mate, bytes, count)] in the library's order (count descending, mate, bytes)}."""
+        v = COverrepView()
+        self._check(self.lib.fq_overrep_results(self.ctx, C.byref(v)))
+        seqs = []
+        for i in range(v.n_seqs):
+            e = v.seqs[i]
+            seqs.append((int(e.mate), C.string_at(C.addressof(v.bytes.contents) + e.offset, e.len), int(e.count)))
+        return {"prefix_len": int(v.prefix_len), "min_ppm": int(v.min_ppm), "reads": [int(x) for x in v.reads],
+                "min_count": [int(x) for x in v.min_count], "seqs": seqs}
 
     def set_quality(self, quality: int):
         """Options::quality for the following batches (the reference's NextSeq adjustment, FaQCs.cpp:272-277)."""

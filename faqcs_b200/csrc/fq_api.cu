@@ -26,6 +26,7 @@
 #include "fq_frame.cuh"
 #include "fq_kmer.cuh"
 #include "fq_overlap.cuh"
+#include "fq_overrep.cuh"
 #include "fq_trim.cuh"
 
 using namespace fq;
@@ -81,7 +82,7 @@ using DevBuf = Buf<false>;
 using HostBuf = Buf<true>;
 
 // An open-addressing table of KmerSlot in device memory (fq_kmer.cuh) with the buffers of its end-of-pass exchange: the k-mer
-// table and the duplication table of a context.
+// table, the duplication table and the overrepresented-sequence count table of a context.
 struct HashTable {
     unsigned long long min_cap = 1ull << 20;       // slots of a new table (a power of two)
     unsigned long long cap = 0, occupied_bound = 0;
@@ -173,6 +174,21 @@ struct fq_ctx {
         uint64_t res[kOvlPairs + 1] = {};
         std::vector<uint64_t> ins, r1o, r1m, r2o, r2m;
     } ovl;
+
+    // overrepresented sequences (fq_overrep_*, fq_overrep.cuh): one key per read's prefix, the bytes in a capture store
+    struct Overrep {
+        bool enabled = false;
+        uint32_t prefix_len = 50, min_ppm = 1000;
+        uint64_t reads[2] = {0, 0};                // mate-m reads of the current pass counted here
+        HashTable T{1ull << 16};
+        DevBuf d_store, d_sel;                     // capture store (OverrepStore); end of a pass: the selected slots
+        uint64_t store_cap = 0, store_bound = 0;   // entries, and a bound on the occupied ones
+        // the last finished pass (fq_overrep_view)
+        uint32_t res_prefix_len = 50, res_min_ppm = 1000;
+        uint64_t res_reads[2] = {0, 0}, res_min_count[2] = {2, 2};
+        std::vector<fq_overrep_seq> seqs;
+        std::vector<uint8_t> bytes;
+    } ovr;
 
     // host-side stats views handed out by fq_stats
     std::vector<uint64_t> v_adapter_reads, v_adapter_bases, v_pre_q, v_post_q, v_pre_b, v_post_b, v_hist[4], v_pre_comp,
@@ -465,7 +481,7 @@ fq_status map_device_error(fq_ctx *ctx, const BatchInfo &hi)
     return fail(ctx, FQ_ERR_STATE, "unknown device error");
 }
 
-// ---- the hash tables (k-mer rarefaction, duplication statistics): host side of fq_kmer.cuh -------------------------
+// ---- the hash tables (k-mer rarefaction, duplication statistics, overrepresented sequences): host side of fq_kmer.cuh ----
 KmerTable table_of(const HashTable &T)
 {
     return KmerTable{T.d_slots.as<KmerSlot>(), T.cap - 1};
@@ -680,6 +696,69 @@ fq_status overlap_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, u
     return FQ_OK;
 }
 
+size_t overrep_stride(uint32_t prefix_len) { return 16 + ((size_t)prefix_len + 7) / 8 * 8; }
+
+OverrepStore overrep_store_of(fq_ctx::Overrep &R)
+{
+    return OverrepStore{R.d_store.as<uint8_t>() + 64, R.store_cap - 1, (uint32_t)overrep_stride(R.prefix_len), R.d_store.as<unsigned long long>()};
+}
+
+// Room for `adding` more entries in the capture store at a load factor <= 1/2, contents kept (as table_reserve does).  The
+// store's first 64 bytes hold its exact occupancy.
+fq_status overrep_store_reserve(fq_ctx *ctx, fq_ctx::Overrep &R, uint64_t adding)
+{
+    uint64_t need = R.store_bound + adding;
+    if (2 * need > R.store_cap && R.store_cap) {
+        uint64_t occ = 0;
+        CK(cudaMemcpyAsync(&occ, R.d_store.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        need = occ + adding;
+    }
+    if (2 * need > R.store_cap) {
+        uint64_t cap = 1024;
+        while (cap < 4 * need) cap <<= 1;           // headroom: the exact occupancy is read back rarely
+        const size_t stride = overrep_stride(R.prefix_len);
+        DevBuf nb;
+        CK(nb.ensure(64 + cap * stride));
+        OverrepStore to{nb.as<uint8_t>() + 64, cap - 1, (uint32_t)stride, nb.as<unsigned long long>()};
+        if (R.store_cap) CK(cudaMemcpyAsync(nb.p, R.d_store.p, 8, cudaMemcpyDeviceToDevice, ctx->stream));
+        else CK(cudaMemsetAsync(nb.p, 0, 8, ctx->stream));
+        k_overrep_store_clear<<<ctx->sm_count * 4, 256, 0, ctx->stream>>>(to);
+        if (R.store_cap) k_overrep_store_rehash<<<ctx->sm_count * 4, 256, 0, ctx->stream>>>(overrep_store_of(R), to);
+        ctx->launches += R.store_cap ? 2 : 1;
+        CK(cudaStreamSynchronize(ctx->stream));
+        R.d_store = std::move(nb);
+        R.store_cap = cap;
+    }
+    R.store_bound = need;
+    return FQ_OK;
+}
+
+// One batch of overrepresented sequences: room for one key per read in the count table and, per mate, for the keys that can
+// meet the capture condition in this batch (at most floor(10^6 / ppm), and at most the batch's reads), then k_overrep.
+fq_status overrep_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint32_t n, int n_mates)
+{
+    fq_ctx::Overrep &R = ctx->ovr;
+    fq_status st = table_reserve(ctx, R.T, (uint64_t)n * n_mates);
+    if (st != FQ_OK) return st;
+    st = overrep_store_reserve(ctx, R, (uint64_t)n_mates * std::min<uint64_t>(n, 1000000u / R.min_ppm));
+    if (st != FQ_OK) return st;
+    OverrepArgs oa{};
+    oa.raw[0] = d_r1; oa.raw[1] = d_r2;
+    oa.rec[0] = ctx->d_rec[0].as<Rec>(); oa.rec[1] = ctx->d_rec[1].as<Rec>();
+    oa.n_rec = n; oa.n_mates = (uint32_t)n_mates; oa.prefix_len = R.prefix_len;
+    for (int m = 0; m < n_mates; ++m) {
+        R.reads[m] += n;
+        oa.thr[m] = (unsigned long long)R.min_ppm * R.reads[m];
+    }
+    oa.T = table_of(R.T);
+    oa.S = overrep_store_of(R);
+    const uint64_t warps = (uint64_t)(n + 31) / 32 * n_mates;
+    k_overrep<<<(unsigned)((warps + 7) / 8), 256, 0, ctx->stream>>>(oa);
+    ctx->launches++;
+    return FQ_OK;
+}
+
 // Outputs go to the d_out / h_out set `slot`.  With async_copy the D2H runs on s_out and the caller waits on ev_out.
 fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint8_t *d_r2, size_t n2, bool paired,
                          uint64_t first_record_index, int is_final, int copy_out, int slot, bool async_copy, fq_batch_out *out)
@@ -865,6 +944,11 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
     // ---- insert size and overlap error profile: paired batches, the sequence lines as framed
     if (ctx->ovl.enabled && paired) {
         st = overlap_batch(ctx, d_r1, d_r2, n, max_len);
+        if (st != FQ_OK) return st;
+    }
+    // ---- overrepresented sequences: the prefixes of the sequence lines as framed, each mate on its own
+    if (ctx->ovr.enabled) {
+        st = overrep_batch(ctx, d_r1, d_r2, n, n_mates);
         if (st != FQ_OK) return st;
     }
 
@@ -2127,6 +2211,195 @@ fq_status overlap_end_pass_impl(fq_ctx *const *ctxs, int n, const fq_comm *cm, u
     return FQ_OK;
 }
 
+// ---- overrepresented sequences: end of a pass, over one context or a table sharded over several ------------------------
+// Every rank's u64 list on every rank, concatenated in rank order: the sizes, then the lists padded to the longest.
+fq_status nccl_allgather_var(fq_ctx *ctx, const fq_comm *c, std::vector<uint64_t> mine, std::vector<uint64_t> *all)
+{
+    std::vector<uint64_t> sizes, padded;
+    fq_status st = nccl_allgather_u64(ctx, c, std::vector<uint64_t>{mine.size()}, &sizes);
+    if (st != FQ_OK) return st;
+    const uint64_t most = std::max<uint64_t>(1, *std::max_element(sizes.begin(), sizes.end()));
+    mine.resize(most, 0);
+    st = nccl_allgather_u64(ctx, c, mine, &padded);
+    if (st != FQ_OK) return st;
+    all->clear();
+    for (int j = 0; j < c->n_ranks; ++j) all->insert(all->end(), padded.begin() + (size_t)j * most, padded.begin() + (size_t)j * most + sizes[j]);
+    return FQ_OK;
+}
+
+// The owner shard's keys that pass the report rule, appended to `sel` as {key, count} word pairs.
+fq_status overrep_select(fq_ctx *ctx, const uint64_t min_count[2], std::vector<uint64_t> *sel)
+{
+    fq_ctx::Overrep &R = ctx->ovr;
+    const uint32_t cap = 2 * (1000000u / R.min_ppm);            // at most floor(10^6 / ppm) keys per mate pass
+    CK(cudaSetDevice(ctx->device));
+    CK(R.d_sel.ensure((size_t)cap * sizeof(KmerSlot)));
+    CK(cudaMemsetAsync(R.T.d_scalars.p, 0, 8, ctx->stream));
+    uint32_t *const d_n = R.T.d_scalars.as<uint32_t>();
+    k_overrep_select<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(R.T), min_count[0], min_count[1], R.d_sel.as<KmerSlot>(), cap, d_n);
+    ctx->launches++;
+    uint32_t n_sel = 0;
+    CK(cudaMemcpyAsync(&n_sel, d_n, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (n_sel > cap) return fail(ctx, FQ_ERR_STATE, "overrepresented sequences: more keys pass the threshold than the reads allow");
+    std::vector<KmerSlot> e(n_sel);
+    if (n_sel) CK(cudaMemcpy(e.data(), R.d_sel.p, (size_t)n_sel * sizeof(KmerSlot), cudaMemcpyDeviceToHost));
+    for (const KmerSlot &x : e) { sel->push_back(x.key); sel->push_back(x.count); }
+    return FQ_OK;
+}
+
+// The context's captured entries whose key is in `keys`, appended to `out` as whole store entries (stride / 8 words each).
+fq_status overrep_captured(fq_ctx *ctx, const std::map<uint64_t, uint64_t> &keys, std::vector<uint64_t> *out)
+{
+    fq_ctx::Overrep &R = ctx->ovr;
+    if (!R.store_cap || keys.empty()) return FQ_OK;
+    const size_t words = overrep_stride(R.prefix_len) / 8;
+    std::vector<uint64_t> h(R.store_cap * words);
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaMemcpy(h.data(), R.d_store.as<uint8_t>() + 64, h.size() * 8, cudaMemcpyDeviceToHost));
+    for (uint64_t i = 0; i < R.store_cap; ++i) {
+        const uint64_t *const e = h.data() + i * words;
+        if (e[0] != kKmerEmpty && keys.count(e[0])) out->insert(out->end(), e, e + words);
+    }
+    return FQ_OK;
+}
+
+// A cleared count table and capture store for the next pass.
+fq_status overrep_clear(fq_ctx *ctx)
+{
+    fq_ctx::Overrep &R = ctx->ovr;
+    R.reads[0] = R.reads[1] = 0;
+    R.T.occupied_bound = 0;
+    R.store_bound = 0;
+    CK(cudaSetDevice(ctx->device));
+    k_kmer_clear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(table_of(R.T));
+    ctx->launches++;
+    if (R.store_cap) {
+        CK(cudaMemsetAsync(R.d_store.p, 0, 8, ctx->stream));
+        k_overrep_store_clear<<<ctx->sm_count * 4, 256, 0, ctx->stream>>>(overrep_store_of(R));
+        ctx->launches++;
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    R.T.d_send.release();
+    R.T.d_recv.release();
+    return FQ_OK;
+}
+
+fq_status overrep_end_pass_impl(fq_ctx *const *ctxs, int n, const fq_comm *cm, uint32_t n_shards, uint32_t rank0)
+{
+    fq_ctx *const ctx0 = ctxs[0];
+    fq_status st = sync_all(ctxs, n);
+    if (st != FQ_OK) return st;
+    // 1. agree on the parameters; occupied slots per owner: header {enabled, prefix_len << 32 | min_ppm, reads of mate 1, of mate 2, counts[n_shards]}
+    const size_t H = kHeadCounts + n_shards;
+    std::vector<uint64_t> head((size_t)n_shards * H, 0);
+    for (int i = 0; i < n; ++i) {
+        fq_ctx::Overrep &R = ctxs[i]->ovr;
+        uint64_t *h = head.data() + (size_t)(rank0 + i) * H;
+        h[0] = R.enabled; h[1] = (uint64_t)R.prefix_len << 32 | R.min_ppm; h[2] = R.reads[0]; h[3] = R.reads[1];
+        if (R.enabled && n_shards > 1) {
+            st = table_owner_counts(ctxs[i], R.T, n_shards, h + kHeadCounts);
+            if (st != FQ_OK) return st;
+        }
+    }
+    if (cm) {
+        const std::vector<uint64_t> mine(head.begin() + (size_t)rank0 * H, head.begin() + (size_t)(rank0 + 1) * H);
+        st = nccl_allgather_u64(ctx0, cm, mine, &head);
+        if (st != FQ_OK) return st;
+    }
+    uint64_t enabled = 0, reads[2] = {0, 0};
+    for (uint32_t j = 0; j < n_shards; ++j) {
+        const uint64_t *h = head.data() + (size_t)j * H;
+        enabled += h[0];
+        reads[0] += h[2];
+        reads[1] += h[3];
+    }
+    if (!enabled) return fail(ctx0, FQ_ERR_STATE, "fq_overrep_end_pass_all: overrepresented sequences are not enabled (fq_overrep_enable)");
+    if (enabled != n_shards) return fail(ctx0, FQ_ERR_ARG, "fq_overrep_end_pass_all: overrepresented sequences are enabled on some contexts only");
+    for (uint32_t j = 1; j < n_shards; ++j) {
+        const uint64_t a = head[1], b = head[(size_t)j * H + 1];
+        if (a != b) {
+            char msg[200];
+            snprintf(msg, sizeof msg, "fq_overrep_end_pass_all: context %u has prefix_len = %llu, min_ppm = %llu; context 0 prefix_len = %llu, min_ppm = %llu", j,
+                     (unsigned long long)(b >> 32), (unsigned long long)(b & 0xffffffffu), (unsigned long long)(a >> 32), (unsigned long long)(a & 0xffffffffu));
+            return fail(ctx0, FQ_ERR_ARG, msg);
+        }
+    }
+    const uint32_t prefix_len = (uint32_t)(head[1] >> 32), ppm = (uint32_t)(head[1] & 0xffffffffu);
+    uint64_t min_count[2];
+    for (int m = 0; m < 2; ++m) min_count[m] = std::max<uint64_t>(2, (ppm * reads[m] + 999999) / 1000000);
+    // 2. exchange the groups and merge
+    if (n_shards > 1) {
+        st = table_exchange(ctxs, n, cm, rank0, n_shards, [](fq_ctx *c) -> HashTable & { return c->ovr.T; }, head, H);
+        if (st != FQ_OK) return st;
+    }
+    // 3. select on each owner; 4. the selected {key, count} and the captured entries of those keys, from every shard
+    std::vector<uint64_t> sel, all;
+    for (int i = 0; i < n; ++i) {
+        st = overrep_select(ctxs[i], min_count, &sel);
+        if (st != FQ_OK) return st;
+    }
+    if (cm) {
+        st = nccl_allgather_var(ctx0, cm, sel, &all);
+        if (st != FQ_OK) return st;
+        sel.swap(all);
+    }
+    std::map<uint64_t, uint64_t> count;
+    for (size_t k = 0; k < sel.size(); k += 2) count[sel[k]] = sel[k + 1];
+    std::vector<uint64_t> cap;
+    for (int i = 0; i < n; ++i) {
+        st = overrep_captured(ctxs[i], count, &cap);
+        if (st != FQ_OK) return st;
+    }
+    if (cm) {
+        st = nccl_allgather_var(ctx0, cm, cap, &all);
+        if (st != FQ_OK) return st;
+        cap.swap(all);
+    }
+    // 5. join and order: count descending, mate ascending, bytes ascending (memcmp on the common length, shorter first)
+    const size_t words = overrep_stride(prefix_len) / 8;
+    std::map<uint64_t, const uint8_t *> entry;
+    for (size_t k = 0; k < cap.size(); k += words) entry.emplace(cap[k], reinterpret_cast<const uint8_t *>(cap.data() + k));
+    struct Seq { uint64_t count; uint32_t mate, len; const uint8_t *s; };
+    std::vector<Seq> seqs;
+    for (const auto &kv : count) {
+        const auto it = entry.find(kv.first);
+        if (it == entry.end()) {
+            char msg[200];
+            snprintf(msg, sizeof msg, "fq_overrep_end_pass_all: key %016llx (mate %llu, %llu reads) passed the threshold, but no context captured its bytes",
+                     (unsigned long long)kv.first, (unsigned long long)(kv.first & 1) + 1, (unsigned long long)kv.second);
+            return fail(ctx0, FQ_ERR_STATE, msg);
+        }
+        uint32_t hdr[2];
+        memcpy(hdr, it->second + 8, 8);
+        seqs.push_back(Seq{kv.second, (uint32_t)(kv.first & 1) + 1, hdr[0], it->second + 16});
+    }
+    std::sort(seqs.begin(), seqs.end(), [](const Seq &a, const Seq &b) {
+        if (a.count != b.count) return a.count > b.count;
+        if (a.mate != b.mate) return a.mate < b.mate;
+        const int c = memcmp(a.s, b.s, std::min(a.len, b.len));
+        return c ? c < 0 : a.len < b.len;
+    });
+    std::vector<fq_overrep_seq> out;
+    std::vector<uint8_t> bytes;
+    for (const Seq &q : seqs) {
+        out.push_back(fq_overrep_seq{q.count, q.mate, q.len, bytes.size()});
+        bytes.insert(bytes.end(), q.s, q.s + q.len);
+    }
+    // 6. the same result on every context, then a cleared table and store
+    for (int i = 0; i < n; ++i) {
+        fq_ctx::Overrep &R = ctxs[i]->ovr;
+        R.res_prefix_len = prefix_len;
+        R.res_min_ppm = ppm;
+        for (int m = 0; m < 2; ++m) { R.res_reads[m] = reads[m]; R.res_min_count[m] = min_count[m]; }
+        R.seqs = out;
+        R.bytes = bytes;
+        st = overrep_clear(ctxs[i]);
+        if (st != FQ_OK) return st;
+    }
+    return FQ_OK;
+}
+
 }  // namespace
 
 fq_status fq_kmer_end_pass_all(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
@@ -2201,6 +2474,47 @@ fq_status fq_overlap_results(fq_ctx *ctx, fq_overlap_view *view)
     view->r1_mismatch = V.r1m.data();
     view->r2_overlap = V.r2o.data();
     view->r2_mismatch = V.r2m.data();
+    return FQ_OK;
+}
+
+fq_status fq_overrep_enable(fq_ctx *ctx, uint32_t prefix_len, uint32_t min_ppm)
+{
+    if (!ctx) return FQ_ERR_ARG;
+    if (prefix_len < 1 || prefix_len > kOverrepMaxPrefix || min_ppm < 10 || min_ppm > 1000000)
+        return fail(ctx, FQ_ERR_ARG, "fq_overrep_enable: prefix_len must be in 1..256 and min_ppm in 10..1000000");
+    fq_ctx::Overrep &R = ctx->ovr;
+    if (R.enabled && (R.reads[0] || R.reads[1])) return fail(ctx, FQ_ERR_STATE, "fq_overrep_enable: a pass is under way");
+    CK(cudaSetDevice(ctx->device));
+    CK(R.T.d_scalars.ensure(64));
+    fq_status st = table_resize(ctx, R.T, R.T.min_cap);
+    if (st != FQ_OK) return st;
+    if (prefix_len != R.prefix_len) {              // the store's entries have another size: a new one at the first batch
+        R.d_store.release();
+        R.store_cap = R.store_bound = 0;
+    }
+    R.prefix_len = prefix_len;
+    R.min_ppm = min_ppm;
+    if (!R.enabled) { R.res_prefix_len = prefix_len; R.res_min_ppm = min_ppm; }
+    R.enabled = true;
+    return FQ_OK;
+}
+
+fq_status fq_overrep_end_pass_all(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
+{
+    return end_pass_entry(ctxs, n, comm, "fq_overrep_end_pass_all", overrep_end_pass_impl);
+}
+
+fq_status fq_overrep_results(fq_ctx *ctx, fq_overrep_view *view)
+{
+    if (!ctx || !view) return FQ_ERR_ARG;
+    const fq_ctx::Overrep &R = ctx->ovr;
+    if (!R.enabled) return fail(ctx, FQ_ERR_STATE, "fq_overrep_results: overrepresented sequences are not enabled (fq_overrep_enable)");
+    view->prefix_len = R.res_prefix_len;
+    view->min_ppm = R.res_min_ppm;
+    for (int m = 0; m < 2; ++m) { view->reads[m] = R.res_reads[m]; view->min_count[m] = R.res_min_count[m]; }
+    view->n_seqs = R.seqs.size();
+    view->seqs = R.seqs.data();
+    view->bytes = R.bytes.data();
     return FQ_OK;
 }
 

@@ -68,6 +68,19 @@ __device__ __forceinline__ void kmer_insert(const KmerTable &T, unsigned long lo
     }
 }
 
+// kmer_insert adding `add` to the key's count (first_call untouched): returns the count right after this increment.
+__device__ __forceinline__ uint32_t kmer_insert_add(const KmerTable &T, unsigned long long key, uint32_t add)
+{
+    unsigned long long slot = kmer_hash(key) & T.cap_mask;
+    for (;;) {
+        KmerSlot *const p = &T.slots[slot];
+        unsigned long long prev = *reinterpret_cast<volatile unsigned long long *>(&p->key);
+        if (prev == kKmerEmpty) prev = atomicCAS(&p->key, kKmerEmpty, key);
+        if (prev == kKmerEmpty || prev == key) return atomicAdd(&p->count, add) + add;
+        slot = (slot + 1) & T.cap_mask;
+    }
+}
+
 // One thread per read (mate-major).  The reference's trim() call of record r of mate m (batches of 32768 records, mate 1's
 // call in front of mate 2's): first_call + (r / 32768) * n_mates + m.
 __global__ void __launch_bounds__(256) k_kmer(const KmerArgs a)

@@ -34,6 +34,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <unordered_map>
 #include <vector>
 
 #include "../../include/faqcs_b200.h"
@@ -46,6 +47,16 @@ static const char *kPhiXComplement = "__PhiX174_NC_001422_complement__";
 static const char *kPhiXSeq =
 #include "phix174.inc"
     ;
+static const char *kBuiltinAdapters[][2] = {              // options.cpp:576-618 (sequence data)
+    {"cre-loxp-forward", "TCGTATAACTTCGTATAATGTATGCTATACGAAGTTATTACG"},
+    {"cre-loxp-reverse", "AGCATATTGAAGCATATTACATACGATATGCTTCAATAATGC"},
+    {"TruSeq-adapter-1", "GGGGTAGTGTGGATCCTCCTCTAGGCAGTTGGGTTATTCTAGAAGCAGATGTGTTGGCTGTTTCTGAAACTCTGGAAAA"},
+    {"TruSeq-adapter-3", "CAACAGCCGGTCAAAACATCTGGAGGGTAAGCCATAAACACCTCAACAGAAAA"},
+    {"PCR-primer-1", "CGATAACTTCGTATAATGTATGCTATACGAAGTTATTACG"},
+    {"PCR-primer-2", "GCATAACTTCGTATAGCATACATTATACGAAGTTATACGA"},
+    {"Nextera-primer-adapter-1", "GATCGGAAGAGCACACGTCTGAACTCCAGTCAC"},
+    {"Nextera-primer-adapter-2", "GATCGGAAGAGCGTCGTGTAGGGAAAGAGTGT"},
+    {"Nextera-junction-adapter-1", "CTGTCTCTTATACACATCTAGATGTGTATAAGAGACAG"}};
 
 struct Cli {
     bool print_usage = false, protect_5 = false, replace_N = false, kmer_rarefaction = false, discard_output = false;
@@ -65,6 +76,10 @@ struct Cli {
     bool insert_size = false;       // insert size and overlap error profile of the paired pass -> prefix.insert_size.txt
     long long insert_min_overlap = 30, insert_diff_limit = 5, insert_diff_pct = 20;    // checked after parsing
     bool insert_bad_number = false;
+    bool overrep = false;           // overrepresented sequences of each input pass -> prefix.overrepresented.txt
+    long long overrep_len = 50, overrep_ppm = 1000;    // checked after parsing
+    bool overrep_bad_number = false;
+    vector<pair<string, string>> artifacts;            // --artifactFile entries (also in `adapter`)
     bool keep_unpaired = false;     // the -u pass appends to prefix.unpaired.trimmed.fastq instead of truncating it (the reference's Q11 quirk, fixed)
     vector<int> devices;            // --devices 0,1,...: consecutive batches go to consecutive GPUs, one NCCL all-reduce at the end
     bool has_paired() const { return !input_read1_file.empty(); }       // has_paired() tests read1 twice, FaQCs.h:135-138
@@ -156,7 +171,11 @@ static void usage()
             "\t\t\t\tadapter read-through and mismatches per cycle in the overlap: prefix.insert_size.txt\n"
             "\t--insert_min_overlap\t<INT> shortest overlap tested (default 30, at least 1)\n"
             "\t--insert_diff_limit\t<INT> most mismatches in an accepted overlap (default 5)\n"
-            "\t--insert_diff_pct\t<INT> most mismatches in an accepted overlap, in percent of its length (default 20, 0-100)\n";
+            "\t--insert_diff_pct\t<INT> most mismatches in an accepted overlap, in percent of its length (default 20, 0-100)\n"
+            "\t--overrep\t\t<bool> list the sequences (read prefixes, each mate on its own) above a share of the reads of each\n"
+            "\t\t\t\tinput, with the built-in adapter, PhiX or --artifactFile entry they match: prefix.overrepresented.txt\n"
+            "\t--overrep_len\t\t<INT> bases of each read's prefix compared (default 50, 1-256)\n"
+            "\t--overrep_ppm\t\t<INT> smallest listed share, in reads per million of the mate (default 1000 = 0.1 %, 10-1000000)\n";
 }
 
 static void parse_options(int argc, char *argv[], Cli &o)
@@ -183,7 +202,8 @@ static void parse_options(int argc, char *argv[], Cli &o)
         {"5trim_off", false, &config_opt, 23}, {"debug", false, &config_opt, 24}, {"version", false, &config_opt, 25}, {"R1", true, &config_opt, 26},
         {"R2", true, &config_opt, 27}, {"replace_to_N_q", true, &config_opt, 31}, {"device", true, &config_opt, 40}, {"batch_mb", true, &config_opt, 41}, {"devices", true, &config_opt, 42}, {"gz_out", false, &config_opt, 43}, {"keep_unpaired", false, &config_opt, 44}, {"dup_stats", false, &config_opt, 45},
         {"insert_size", false, &config_opt, 46}, {"insert_min_overlap", true, &config_opt, 47}, {"insert_diff_limit", true, &config_opt, 48},
-        {"insert_diff_pct", true, &config_opt, 49},
+        {"insert_diff_pct", true, &config_opt, 49}, {"overrep", false, &config_opt, 50}, {"overrep_len", true, &config_opt, 51},
+        {"overrep_ppm", true, &config_opt, 52},
         {0, 0, 0, 0}};
     int opt_code;
     opterr = 0;
@@ -259,6 +279,15 @@ static void parse_options(int argc, char *argv[], Cli &o)
                         (config_opt == 47 ? o.insert_min_overlap : config_opt == 48 ? o.insert_diff_limit : o.insert_diff_pct) = v;
                         break;
                     }
+                    case 50: o.overrep = true; break;
+                    case 51: case 52: {
+                        char *end = nullptr;
+                        errno = 0;
+                        const long long v = strtoll(optarg, &end, 10);
+                        if (end == optarg || *end || errno) o.overrep_bad_number = true;
+                        (config_opt == 51 ? o.overrep_len : o.overrep_ppm) = v;
+                        break;
+                    }
                     default: cerr << "Unknown flag!" << endl; break;
                 }
                 break;
@@ -324,27 +353,25 @@ static void parse_options(int argc, char *argv[], Cli &o)
         o.print_usage = true;
         return;
     }
+    if (o.overrep_bad_number || o.overrep_len < 1 || o.overrep_len > 256 || o.overrep_ppm < 10 || o.overrep_ppm > 1000000) {
+        cerr << "Please specify --overrep_len as an integer in the range 1 <= length <= 256 and --overrep_ppm as an integer in the range "
+                "10 <= ppm <= 1000000" << endl;
+        o.print_usage = true;
+        return;
+    }
     o.num_subsample *= 2;      // options.cpp:519-523: doubled on every command line that gets this far, paired input or not
     if (o.replace_N) cerr << "**Warning** \"-substitue\" is not currently implemented" << endl;
-    if (o.filter_adapter) {                               // built-in adapters, options.cpp:576-618 (sequence data)
-        static const char *builtin[][2] = {
-            {"cre-loxp-forward", "TCGTATAACTTCGTATAATGTATGCTATACGAAGTTATTACG"},
-            {"cre-loxp-reverse", "AGCATATTGAAGCATATTACATACGATATGCTTCAATAATGC"},
-            {"TruSeq-adapter-1", "GGGGTAGTGTGGATCCTCCTCTAGGCAGTTGGGTTATTCTAGAAGCAGATGTGTTGGCTGTTTCTGAAACTCTGGAAAA"},
-            {"TruSeq-adapter-3", "CAACAGCCGGTCAAAACATCTGGAGGGTAAGCCATAAACACCTCAACAGAAAA"},
-            {"PCR-primer-1", "CGATAACTTCGTATAATGTATGCTATACGAAGTTATTACG"},
-            {"PCR-primer-2", "GCATAACTTCGTATAGCATACATTATACGAAGTTATACGA"},
-            {"Nextera-primer-adapter-1", "GATCGGAAGAGCACACGTCTGAACTCCAGTCAC"},
-            {"Nextera-primer-adapter-2", "GATCGGAAGAGCGTCGTGTAGGGAAAGAGTGT"},
-            {"Nextera-junction-adapter-1", "CTGTCTCTTATACACATCTAGATGTGTATAAGAGACAG"}};
-        for (auto &b : builtin) o.adapter.push_back(make_pair(string(b[0]), string(b[1])));
-    }
+    if (o.filter_adapter)                                 // built-in adapters, options.cpp:576-618
+        for (auto &b : kBuiltinAdapters) o.adapter.push_back(make_pair(string(b[0]), string(b[1])));
     if (trim_polyA) o.adapter.push_back(make_pair(string("polyA"), string(20, 'A')));
     if (o.filter_phiX) {
         o.adapter.push_back(make_pair(string(kPhiX), string(kPhiXSeq)));
         o.adapter.push_back(make_pair(string(kPhiXComplement), reverse_complement(kPhiXSeq)));
     }
-    if (!o.artifact_file.empty()) parse_artifact_file(o.artifact_file, o.adapter);
+    if (!o.artifact_file.empty()) {
+        parse_artifact_file(o.artifact_file, o.artifacts);
+        o.adapter.insert(o.adapter.end(), o.artifacts.begin(), o.artifacts.end());
+    }
     const string base = o.output_dir + "/" + o.prefix;    // options.cpp:696-741
     if (!o.input_read1_file.empty() && !o.input_read2_file.empty()) {
         o.trimmed_read1_file = base + ".1.trimmed.fastq";
@@ -790,6 +817,7 @@ struct Run {
             if (o.kmer_rarefaction) check(fq_kmer_enable(c, o.kmer, o.split_size, o.num_subsample), c);   // one shard of the pass's table
             if (o.dup_stats) check(fq_dup_enable(c), c);
             if (o.insert_size) check(fq_overlap_enable(c, (uint32_t)o.insert_min_overlap, (uint32_t)o.insert_diff_limit, (uint32_t)o.insert_diff_pct), c);
+            if (o.overrep) check(fq_overrep_enable(c, (uint32_t)o.overrep_len, (uint32_t)o.overrep_ppm), c);
         }
     }
     // end of an input's pass: the contexts' k-mer tables merge into the run's curve and histogram (FaQCs.cpp:518-537, 737-756)
@@ -825,6 +853,59 @@ struct Run {
         for (uint32_t c = 0; c < v.n_cycles; ++c)
             insert_report += to_string(c + 1) + "\t" + to_string(v.r1_overlap[c]) + "\t" + to_string(v.r1_mismatch[c]) + "\t" +
                              to_string(v.r2_overlap[c]) + "\t" + to_string(v.r2_mismatch[c]) + "\n";
+    }
+    // --overrep: the contexts' count tables merged after each input pass, one block of prefix.overrepresented.txt
+    string overrep_report;
+    void overrep_end_pass(bool paired)
+    {
+        if (!o.overrep) return;
+        check(fq_overrep_end_pass_all(ctxs.data(), (int)ctxs.size(), nullptr));
+        fq_overrep_view v;
+        check(fq_overrep_results(ctx, &v));
+        overrep_report += string("pass\t") + (paired ? "paired" : "unpaired") + "\tprefix_len\t" + to_string(v.prefix_len) + "\tppm\t" + to_string(v.min_ppm) + "\n";
+        overrep_report += "#mate\treads\tmin_count\n";
+        for (int m = 0; m < (paired ? 2 : 1); ++m) overrep_report += to_string(m + 1) + "\t" + to_string(v.reads[m]) + "\t" + to_string(v.min_count[m]) + "\n";
+        overrep_report += "#mate\tcount\tpercent\tsequence\tsource\n";
+        for (uint64_t i = 0; i < v.n_seqs; ++i) {
+            const fq_overrep_seq &q = v.seqs[i];
+            const string seq(reinterpret_cast<const char *>(v.bytes + q.offset), q.len);
+            char pct[32];
+            snprintf(pct, sizeof pct, "%.4f", 100.0 * (double)q.count / (double)v.reads[q.mate - 1]);
+            overrep_report += to_string(q.mate) + "\t" + to_string(q.count) + "\t" + pct + "\t" + seq + "\t" + overrep_source(seq) + "\n";
+        }
+    }
+    // The first of the nine built-in adapters, PhiX174 and the --artifactFile entries (in that order) that holds some 20-base
+    // window of the upper-cased sequence (the whole sequence if it is shorter), on either strand; "No Hit" otherwise.
+    vector<pair<string, string>> sources;      // name, upper-cased entry + '\n' + its reverse complement
+    unordered_map<string, size_t> source_of;   // 20-base window -> first entry holding it
+    string overrep_source(string s)
+    {
+        const size_t W = 20;
+        if (sources.empty()) {
+            vector<pair<string, string>> list;
+            for (auto &b : kBuiltinAdapters) list.push_back(make_pair(string(b[0]), string(b[1])));
+            list.push_back(make_pair(string("PhiX174"), string(kPhiXSeq)));
+            list.insert(list.end(), o.artifacts.begin(), o.artifacts.end());
+            for (size_t k = 0; k < list.size(); ++k) {
+                string e = list[k].second;
+                for (char &c : e) c = (char)toupper((unsigned char)c);
+                e += "\n" + reverse_complement(e);
+                for (size_t p = 0; p + W <= e.size(); ++p) source_of.emplace(e.substr(p, W), k);
+                sources.push_back(make_pair(list[k].first, e));
+            }
+        }
+        for (char &c : s) c = (char)toupper((unsigned char)c);
+        size_t best = sources.size();
+        if (s.size() < W) {
+            for (size_t k = 0; k < sources.size() && best == sources.size(); ++k)
+                if (sources[k].second.find(s) != string::npos) best = k;
+        } else {
+            for (size_t p = 0; p + W <= s.size(); ++p) {
+                const auto it = source_of.find(s.substr(p, W));
+                if (it != source_of.end()) best = min(best, it->second);
+            }
+        }
+        return best < sources.size() ? sources[best].first : string("No Hit");
     }
     void set_quality_everywhere(int q) { for (fq_ctx *c : ctxs) check(fq_set_quality(c, q), c); }
 };
@@ -1376,6 +1457,7 @@ int main(int argc, char *argv[])
         if (o.dup_stats && fq_dup_enable(ctx) != FQ_OK) throw string(fq_last_error(ctx));
         if (o.insert_size && fq_overlap_enable(ctx, (uint32_t)o.insert_min_overlap, (uint32_t)o.insert_diff_limit, (uint32_t)o.insert_diff_pct) != FQ_OK)
             throw string(fq_last_error(ctx));
+        if (o.overrep && fq_overrep_enable(ctx, (uint32_t)o.overrep_len, (uint32_t)o.overrep_ppm) != FQ_OK) throw string(fq_last_error(ctx));
         const double t_created = now_s();
         Run R(o);
         R.ctx = ctx;
@@ -1389,12 +1471,14 @@ int main(int argc, char *argv[])
             R.kmer_end_pass();                     // FaQCs.cpp:518-537
             R.dup_end_pass(true);
             R.overlap_end_pass();
+            R.overrep_end_pass(true);
         }
         if (o.has_unpaired()) {
             R.first_batch = true;      // offset detection only if still unknown; the NextSeq check runs per input (FaQCs.cpp:586,673-683)
             process(R, false);
             R.kmer_end_pass();                     // FaQCs.cpp:737-756
             R.dup_end_pass(false);
+            R.overrep_end_pass(false);
         }
         const double t_processed = now_s();
         if (R.ctxs.size() > 1) {
@@ -1432,6 +1516,13 @@ int main(int argc, char *argv[])
             fout << R.insert_report;
             fout.close();
             if (!fout) throw string("Unable to write the insert size file: ") + fn;
+        }
+        if (o.overrep) {
+            const string fn = o.output_dir + "/" + o.prefix + ".overrepresented.txt";
+            ofstream fout(fn.c_str());
+            fout << R.overrep_report;
+            fout.close();
+            if (!fout) throw string("Unable to write the overrepresented sequences file: ") + fn;
         }
         if (!o.trim_only && o.debug) {                           // the reference deletes these unless --debug (plot.cpp:517-537)
             write_debug_files(v, o);

@@ -266,6 +266,54 @@ def fragments(n_pairs: int, seed: int = 91, start: int = 0, L: int = 150, mean: 
     return Workload("fragments", mates[0], mates[1], [])
 
 
+def phix174() -> str:
+    """The PhiX174 genome the command-line driver carries (faqcs_b200/host/phix174.inc)."""
+    import os
+    import re
+    txt = open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "host", "phix174.inc")).read()
+    return "".join(re.findall(r'"([^"]*)"', txt))
+
+
+TRUSEQ_FRAGMENT = dict(BUILTIN_ADAPTERS)["TruSeq-adapter-1"][:60]
+
+
+def overrepresented(n_pairs: int, plants=None, seed: int = 93, start: int = 0, paired: bool = True, L: int = 150) -> Workload:
+    """C2-like reads with planted sequences, the workload of --overrep.  A plant is (sequence, copies, mate, whole): `copies`
+    reads of `mate` (1, 2, or 0 for both mates of the same pairs) start with `sequence`; with whole=True the read is exactly
+    the sequence (a read shorter than the prefix when the sequence is), otherwise the rest of the read stays random (reads
+    equal in their first len(sequence) bases only).  Plants take disjoint reads of a mate.  The default plants a 60-base
+    TruSeq-adapter fragment in 2 % of both mates, a 150-base PhiX fragment in 1 % of R1 and a 30-base primer dimer read in
+    0.5 % of R1."""
+    if plants is None:
+        plants = [(TRUSEQ_FRAGMENT, n_pairs // 50, 0, False), (phix174()[1000:1000 + L], n_pairs // 100, 1, True),
+                  ("ACACTCTTTCCCTACACGACGCTCTTCCGA", n_pairs // 200, 1, True)]
+    rng = np.random.default_rng(seed + start)
+    mates = []
+    rows_both = {}
+    for mate in (1, 2) if paired else (1,):
+        q = _qualities(rng, n_pairs, L, 30, 40, 0.12, 3.0, 2, 41, 0.10, 59)
+        s = _bases(rng, n_pairs, L, 0.002, 0.01)
+        lengths = np.full(n_pairs, L, dtype=np.int64)
+        free = np.ones(n_pairs, dtype=bool)
+        for k, (seq, copies, pm, whole) in enumerate(plants):
+            if pm not in (0, mate):
+                continue
+            b = np.frombuffer(seq.encode(), dtype=np.uint8)
+            assert b.size <= L, "a plant longer than the reads"
+            if pm == 0 and k in rows_both:
+                rows = rows_both[k]
+            else:
+                rows = rng.choice(np.flatnonzero(free), size=copies, replace=False)
+                rows_both[k] = rows
+            assert free[rows].all(), "plants overlap"
+            free[rows] = False
+            s[rows, :b.size] = b
+            if whole:
+                lengths[rows] = b.size
+        mates.append(_assemble(_headers(n_pairs, "OR", mate, start), s, q + 33, lengths))
+    return Workload("overrepresented", mates[0], mates[1] if paired else None, [])
+
+
 def fastq_bytes(records: List[Tuple[str, str, str]], eol: str = "\n") -> bytes:
     """Hand-written records -> FASTQ bytes (micro-cases)."""
     return "".join(f"{h}{eol}{s}{eol}+{eol}{q}{eol}" for h, s, q in records).encode()

@@ -433,6 +433,48 @@ fq_status fq_overlap_enable(fq_ctx *ctx, uint32_t min_overlap, uint32_t diff_lim
 fq_status fq_overlap_end_pass_all(fq_ctx *const *ctx, int n, fq_comm *const *comm);
 fq_status fq_overlap_results(fq_ctx *ctx, fq_overlap_view *view);
 
+/*
+ * Overrepresented sequences (not part of FaQCs; the list FastQC and fastp print, without FastQC's truncation of reads over
+ * 75 bases to 50 and without its contaminant list).  A unit is one read: the mates of a pair count separately (mate 1, 2;
+ * a single-end batch has mate 1 only), and every framed record counts, including reads that trimming or filtering discard,
+ * so no option changes the result.  A read's prefix is the first min(len, prefix_len) bytes of its sequence line as framed
+ * (up to the first '\r' or '\n', case-sensitive, before any masking, trimming or G -> N replacement); reads with equal
+ * prefixes are one sequence, and reads of length 0 count in reads[] but are never listed.  Each prefix is counted exactly
+ * as a 64-bit key (fq_overrep.cuh; n distinct prefixes of one mate give about n^2 / 2^64 expected pairs of equal keys).  A
+ * sequence of mate m with count c is listed when c * 10^6 >= min_ppm * reads[m - 1] and c >= 2, i.e. c >= min_count[m - 1].
+ * The bytes of every listed sequence are kept by a capture rule that needs no second pass (DESIGN.md section 7).
+ *   fq_overrep_enable        before the first batch of a pass (FQ_ERR_STATE in the middle of one): prefix_len 1..256
+ *                            (default 50), min_ppm 10..1000000 (default 1000 = 0.1 %); FQ_ERR_ARG otherwise.  Afterwards every
+ *                            batch path counts.  Nothing is allocated and no kernel runs without it.  Memory: a count table of
+ *                            16-byte slots at load <= 1/2 (about 8.6 GB for 100 M pairs of mostly distinct reads) and a capture
+ *                            store of (16 + prefix_len) bytes per entry that grows by at most 2 x floor(10^6 / min_ppm)
+ *                            entries per batch.
+ *   fq_overrep_end_pass_all  after the last batch of an input: merges the count tables of n contexts (n == 1 and comm == NULL
+ *                            for one context; otherwise as for fq_kmer_end_pass_all), gathers the captured bytes, publishes the
+ *                            pass's list on every context and clears the table and store.  FQ_ERR_ARG when the contexts differ
+ *                            in enablement or parameters; FQ_ERR_STATE if a listed sequence has no captured bytes (a bug).
+ *   fq_overrep_results       the last finished pass; the pointers belong to the context and stay valid until its next
+ *                            fq_overrep_* call.  FQ_ERR_STATE (also for an end of pass) on a context that never enabled it.
+ * Order of seqs: count descending, then mate ascending, then bytes ascending (memcmp on the common length, shorter first).
+ */
+typedef struct fq_overrep_seq {
+    uint64_t count;
+    uint32_t mate;                     /* 1 or 2 */
+    uint32_t len;                      /* bytes of the sequence (its prefix) */
+    uint64_t offset;                   /* of its bytes in fq_overrep_view::bytes */
+} fq_overrep_seq;
+typedef struct fq_overrep_view {
+    uint32_t prefix_len, min_ppm;
+    uint64_t reads[2];                 /* reads of mate 1 and mate 2 in the pass */
+    uint64_t min_count[2];             /* max(2, ceil(min_ppm * reads[m] / 10^6)) */
+    uint64_t n_seqs;
+    const fq_overrep_seq *seqs;
+    const uint8_t *bytes;
+} fq_overrep_view;
+fq_status fq_overrep_enable(fq_ctx *ctx, uint32_t prefix_len, uint32_t min_ppm);
+fq_status fq_overrep_end_pass_all(fq_ctx *const *ctx, int n, fq_comm *const *comm);
+fq_status fq_overrep_results(fq_ctx *ctx, fq_overrep_view *view);
+
 /* Zero the accumulators (new run on the same context). */
 fq_status fq_reset_stats(fq_ctx *ctx);
 
