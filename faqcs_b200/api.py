@@ -125,6 +125,14 @@ class COverrepView(C.Structure):
                 ("n_seqs", C.c_uint64), ("seqs", C.POINTER(COverrepSeq)), ("bytes", C.POINTER(C.c_uint8))]
 
 
+class CTileQualView(C.Structure):
+    _fields_ = [("n_mates", C.c_uint32), ("overflow", C.c_uint32), ("n_tiles", C.c_uint32), ("cycles", C.c_uint32),
+                ("reads", C.c_uint64 * 2), ("untiled", C.c_uint64 * 2),
+                ("lane", C.POINTER(C.c_uint32)), ("tile", C.POINTER(C.c_uint32)),
+                ("tile_reads", C.POINTER(C.c_uint64)), ("tile_bases", C.POINTER(C.c_uint64)), ("tile_qsum", C.POINTER(C.c_uint64)),
+                ("cycle_bases", C.POINTER(C.c_uint64)), ("cycle_qsum", C.POINTER(C.c_uint64))]
+
+
 OVERLAP_SCALARS = ("pairs", "too_short", "overlapped", "r1_adapter", "r2_adapter", "overlap_bases", "mismatch_bases")
 OVERLAP_CYCLE_ARRAYS = ("r1_overlap", "r1_mismatch", "r2_overlap", "r2_mismatch")
 
@@ -353,6 +361,9 @@ class Engine:
             L.fq_overrep_enable.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32]
             L.fq_overrep_end_pass_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
             L.fq_overrep_results.argtypes = [C.c_void_p, C.POINTER(COverrepView)]
+            L.fq_tile_qual_enable.argtypes = [C.c_void_p]
+            L.fq_tile_qual_end_pass_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_void_p)]
+            L.fq_tile_qual_results.argtypes = [C.c_void_p, C.POINTER(CTileQualView)]
             L.fq_last_allreduce_ms.argtypes = [C.c_void_p]
             L.fq_last_allreduce_ms.restype = C.c_float
             L.fq_device_outputs.argtypes = [C.c_void_p, C.POINTER(C.c_void_p * NUM_STREAM)]
@@ -477,6 +488,36 @@ class Engine:
             seqs.append((int(e.mate), C.string_at(C.addressof(v.bytes.contents) + e.offset, e.len), int(e.count)))
         return {"prefix_len": int(v.prefix_len), "min_ppm": int(v.min_ppm), "reads": [int(x) for x in v.reads],
                 "min_count": [int(x) for x in v.min_count], "seqs": seqs}
+
+    def tile_qual_enable(self):
+        """Per flowcell tile quality (fq_tile_qual_enable): every read of the following batches is counted under the (lane,
+        tile) of its header, each mate on its own.  Call before the first batch of a pass."""
+        self._check(self.lib.fq_tile_qual_enable(self.ctx))
+
+    def tile_qual_end_pass(self):
+        """End of one input's pass on this context alone (fq_tile_qual_end_pass_all with n = 1); dist_stats has the other forms."""
+        ctxs = (C.c_void_p * 1)(self.ctx)
+        self._check(self.lib.fq_tile_qual_end_pass_all(ctxs, 1, None))
+
+    def tile_qual_results(self) -> dict:
+        """The last finished pass: ints "n_mates", "overflow", "n_tiles", "cycles"; uint64 arrays "reads" and "untiled" [2];
+        uint32 arrays "lane" and "tile" [n_tiles] ascending; uint64 arrays "tile_reads", "tile_bases", "tile_qsum"
+        [n_tiles, n_mates] and "cycle_bases", "cycle_qsum" [n_tiles, n_mates, cycles]."""
+        v = CTileQualView()
+        self._check(self.lib.fq_tile_qual_results(self.ctx, C.byref(v)))
+        T, M, Cy = int(v.n_tiles), int(v.n_mates), int(v.cycles)
+
+        def arr(p, shape, dt=np.uint64):
+            n = int(np.prod(shape))
+            return np.ctypeslib.as_array(p, (n,)).copy().reshape(shape) if n else np.zeros(shape, dt)
+        out = {"n_mates": M, "overflow": int(v.overflow), "n_tiles": T, "cycles": Cy,
+               "reads": np.array(list(v.reads), np.uint64), "untiled": np.array(list(v.untiled), np.uint64),
+               "lane": arr(v.lane, (T,), np.uint32), "tile": arr(v.tile, (T,), np.uint32)}
+        for k in ("tile_reads", "tile_bases", "tile_qsum"):
+            out[k] = arr(getattr(v, k), (T, M))
+        for k in ("cycle_bases", "cycle_qsum"):
+            out[k] = arr(getattr(v, k), (T, M, Cy))
+        return out
 
     def set_quality(self, quality: int):
         """Options::quality for the following batches (the reference's NextSeq adjustment, FaQCs.cpp:272-277)."""

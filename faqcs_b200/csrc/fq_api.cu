@@ -27,6 +27,7 @@
 #include "fq_kmer.cuh"
 #include "fq_overlap.cuh"
 #include "fq_overrep.cuh"
+#include "fq_tile_qual.cuh"
 #include "fq_trim.cuh"
 
 using namespace fq;
@@ -189,6 +190,26 @@ struct fq_ctx {
         std::vector<fq_overrep_seq> seqs;
         std::vector<uint8_t> bytes;
     } ovr;
+
+    // per flowcell tile quality (fq_tile_qual_*, fq_tile_qual.cuh): a key table and an accumulator block per context
+    struct TileQual {
+        bool enabled = false;
+        uint32_t n_mates = 0;                      // mates of the current pass's batches (0: no batch yet)
+        uint64_t reads[2] = {0, 0};                // reads of the current pass counted here
+        uint32_t longest = 0;                      // longest read of the current pass here
+        uint32_t claims = 0, overflow = 0;         // TileCounters after the last batch
+        // a batch counted its keys and has not returned FQ_OK yet; set when the next batch starts: a batch of this pass
+        // failed part-way (its keys are in the table, its reads only partly counted), so the pass has no result
+        bool batch_open = false, failed = false;
+        TileLayout L{0, 0};                        // of d_acc (D == 0: nothing allocated yet)
+        DevBuf d_slots, d_cnt, d_id[2], d_acc;
+        HostBuf h_cnt;                             // {claims, overflow}, read back with the batch's BatchInfo
+        // the last finished pass (fq_tile_qual_view)
+        uint32_t res_mates = 0, res_overflow = 0, res_cycles = 0;
+        uint64_t res_reads[2] = {0, 0}, res_untiled[2] = {0, 0};
+        std::vector<uint32_t> lane, tile;
+        std::vector<uint64_t> t_reads, t_bases, t_qsum, c_bases, c_qsum;
+    } tq;
 
     // host-side stats views handed out by fq_stats
     std::vector<uint64_t> v_adapter_reads, v_adapter_bases, v_pre_q, v_post_q, v_pre_b, v_post_b, v_hist[4], v_pre_comp,
@@ -759,6 +780,79 @@ fq_status overrep_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, u
     return FQ_OK;
 }
 
+KmerTable tile_table_of(fq_ctx::TileQual &Q) { return KmerTable{Q.d_slots.as<KmerSlot>(), kTileSlots - 1}; }
+
+// Per flowcell tile quality, first half of a batch (right after framing): every read's key into the table and its dense id
+// into d_id; {claims, overflow} travel back with the batch's BatchInfo, so the host knows the tiles without a sync of its own.
+fq_status tile_keys_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint32_t n, int n_mates)
+{
+    fq_ctx::TileQual &Q = ctx->tq;
+    Q.failed |= Q.batch_open;
+    Q.batch_open = true;
+    TileKeyArgs ka{};
+    ka.raw[0] = d_r1; ka.raw[1] = d_r2;
+    ka.rec[0] = ctx->d_rec[0].as<Rec>(); ka.rec[1] = ctx->d_rec[1].as<Rec>();
+    ka.n_rec = n; ka.n_mates = (uint32_t)n_mates;
+    ka.T = tile_table_of(Q);
+    ka.cnt = Q.d_cnt.as<TileCounters>();
+    for (int m = 0; m < n_mates; ++m) {
+        CK(Q.d_id[m].ensure((size_t)n * sizeof(uint16_t)));
+        ka.id[m] = Q.d_id[m].as<uint16_t>();
+        Q.reads[m] += n;
+    }
+    const uint64_t warps = (uint64_t)(n + 31) / 32 * n_mates;
+    k_tile_keys<<<(unsigned)((warps + kTileKeyThreads / 32 - 1) / (kTileKeyThreads / 32)), kTileKeyThreads, 0, ctx->stream>>>(ka);
+    ctx->launches++;
+    CK(cudaMemcpyAsync(Q.h_cnt.p, Q.d_cnt.p, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    Q.n_mates = (uint32_t)n_mates;
+    return FQ_OK;
+}
+
+// Second half, once the BatchInfo is back: the block grown to the tiles seen and the batch's longest read (contents relaid on
+// the device), then k_tile_qual.  A context that overflowed accumulates nothing more: its pass reports no table.
+fq_status tile_qual_batch(fq_ctx *ctx, const uint8_t *d_r1, const uint8_t *d_r2, uint32_t n, int n_mates, uint32_t max_len, int32_t in_off)
+{
+    fq_ctx::TileQual &Q = ctx->tq;
+    const uint32_t *h = Q.h_cnt.as<uint32_t>();
+    Q.claims = h[0];
+    Q.overflow |= h[1];
+    Q.longest = std::max(Q.longest, max_len);
+    if (Q.overflow || Q.claims == 0) return FQ_OK;
+    uint32_t D = 64;
+    while (D < (uint32_t)n_mates * Q.claims) D <<= 1;
+    const uint32_t C = std::min(kTileMaxCycles, round_up(std::max(Q.longest, 1u), 32));
+    if (D > Q.L.D || C > Q.L.C) {
+        const TileLayout nl{std::max(D, Q.L.D), std::max(C, Q.L.C)};
+        DevBuf nb;
+        CK(nb.ensure(nl.total() * 8));
+        CK(cudaMemsetAsync(nb.p, 0, nl.total() * 8, ctx->stream));
+        if (Q.L.D) {
+            k_tile_relay<<<ctx->sm_count * 4, 256, 0, ctx->stream>>>(Q.d_acc.as<unsigned long long>(), Q.L, nb.as<unsigned long long>(), nl);
+            ctx->launches++;
+        }
+        CK(cudaStreamSynchronize(ctx->stream));
+        Q.d_acc = std::move(nb);
+        Q.L = nl;
+    }
+    TileQualArgs qa{};
+    qa.raw[0] = d_r1; qa.raw[1] = d_r2;
+    qa.rec[0] = ctx->d_rec[0].as<Rec>(); qa.rec[1] = ctx->d_rec[1].as<Rec>();
+    qa.id[0] = Q.d_id[0].as<uint16_t>(); qa.id[1] = Q.d_id[1].as<uint16_t>();
+    qa.n_rec = n; qa.n_mates = (uint32_t)n_mates; qa.in_off = in_off;
+    // one wave of warps: runs as long as that allows, so that a run spans few id changes of sorted input
+    const size_t smem = (size_t)(kTileQualThreads / 32) * Q.L.C * 4;
+    int per_sm = 1;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_tile_qual, kTileQualThreads, smem));
+    const uint64_t wave = std::max<uint64_t>(1, (uint64_t)ctx->sm_count * std::max(per_sm, 1) * (kTileQualThreads / 32) / (uint64_t)n_mates);
+    qa.run = (uint32_t)std::max<uint64_t>(32, ((uint64_t)n + wave - 1) / wave);
+    qa.L = Q.L;
+    qa.acc = Q.d_acc.as<unsigned long long>();
+    const uint64_t warps = (uint64_t)((n + qa.run - 1) / qa.run) * n_mates;
+    k_tile_qual<<<(unsigned)((warps + kTileQualThreads / 32 - 1) / (kTileQualThreads / 32)), kTileQualThreads, smem, ctx->stream>>>(qa);
+    ctx->launches++;
+    return FQ_OK;
+}
+
 // Outputs go to the d_out / h_out set `slot`.  With async_copy the D2H runs on s_out and the caller waits on ev_out.
 fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint8_t *d_r2, size_t n2, bool paired,
                          uint64_t first_record_index, int is_final, int copy_out, int slot, bool async_copy, fq_batch_out *out)
@@ -774,6 +868,8 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
         return fail(ctx, FQ_ERR_ARG, "thread-count emulation needs batches that start on a 32768-record boundary");
     if (ctx->dup.enabled && ctx->dup.n_mates && ctx->dup.n_mates != (paired ? 2u : 1u))
         return fail(ctx, FQ_ERR_ARG, "duplication statistics: paired and single-end batches in one pass");
+    if (ctx->tq.enabled && ctx->tq.n_mates && ctx->tq.n_mates != (paired ? 2u : 1u))
+        return fail(ctx, FQ_ERR_ARG, "per flowcell tile quality: paired and single-end batches in one pass");
     BatchInfo *info = ctx->d_info.as<BatchInfo>();
     CK(reset_info(ctx));
     CK(cudaEventRecord(ctx->ev[0], ctx->stream));
@@ -794,6 +890,11 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
     if (n == 0) {
         CK(cudaStreamSynchronize(ctx->stream));
         return FQ_OK;
+    }
+    // ---- per flowcell tile quality, first half: the keys, while the host waits for the framing scalars anyway
+    if (ctx->tq.enabled) {
+        st = tile_keys_batch(ctx, d_r1, d_r2, n, n_mates);
+        if (st != FQ_OK) return st;
     }
     // second look at the framing scalars: max length, CR accounting, |seq| != |qual|
     BatchInfo hi;
@@ -951,6 +1052,11 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
         st = overrep_batch(ctx, d_r1, d_r2, n, n_mates);
         if (st != FQ_OK) return st;
     }
+    // ---- per flowcell tile quality, second half: the quality lines as framed, each mate on its own
+    if (ctx->tq.enabled) {
+        st = tile_qual_batch(ctx, d_r1, d_r2, n, n_mates, max_len, o.in_off);
+        if (st != FQ_OK) return st;
+    }
 
     // ---- route / scan / emit
     EmitArgs ea{};
@@ -1064,6 +1170,7 @@ fq_status process_common(fq_ctx *ctx, const uint8_t *d_r1, size_t n1, const uint
         }
     }
     CK(cudaStreamSynchronize(ctx->stream));
+    ctx->tq.batch_open = false;
     return FQ_OK;
 }
 
@@ -2400,6 +2507,153 @@ fq_status overrep_end_pass_impl(fq_ctx *const *ctxs, int n, const fq_comm *cm, u
     return FQ_OK;
 }
 
+// ---- per flowcell tile quality: end of a pass, over one context or several ---------------------------------------------
+// The contexts' key lists are united (gathered on the host, or NCCL all-gathers across ranks) and sorted by (lane, tile);
+// every context's block is laid out in union order for the largest cycle capacity of any, and the blocks are summed (on
+// the host, or one ncclAllReduce).  The same result goes to every context, then the tables and blocks are cleared.
+fq_status tile_qual_clear(fq_ctx *ctx)
+{
+    fq_ctx::TileQual &Q = ctx->tq;
+    CK(cudaSetDevice(ctx->device));
+    k_kmer_clear<<<ctx->sm_count * 2, 256, 0, ctx->stream>>>(tile_table_of(Q));
+    ctx->launches++;
+    CK(cudaMemsetAsync(Q.d_cnt.p, 0, sizeof(TileCounters), ctx->stream));
+    if (Q.L.D) CK(cudaMemsetAsync(Q.d_acc.p, 0, Q.L.total() * 8, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    Q.n_mates = 0;
+    Q.reads[0] = Q.reads[1] = 0;
+    Q.longest = Q.claims = Q.overflow = 0;
+    Q.batch_open = Q.failed = false;
+    return FQ_OK;
+}
+
+fq_status tile_qual_end_pass_impl(fq_ctx *const *ctxs, int n, const fq_comm *cm, uint32_t n_shards, uint32_t rank0)
+{
+    fq_ctx *const ctx0 = ctxs[0];
+    fq_status st = sync_all(ctxs, n);
+    if (st != FQ_OK) return st;
+    // 1. header {enabled, mates (0: no batch), overflow, longest, cycle capacity, reads[2], untiled[2], a batch failed};
+    //    each context's keys by dense id
+    const size_t H = 10;
+    std::vector<uint64_t> head((size_t)n_shards * H, 0), all_keys;
+    std::vector<std::vector<uint64_t>> key_of(n);
+    std::vector<KmerSlot> slots(kTileSlots);
+    for (int i = 0; i < n; ++i) {
+        fq_ctx *const ctx = ctxs[i];
+        fq_ctx::TileQual &Q = ctx->tq;
+        uint64_t *h = head.data() + (size_t)(rank0 + i) * H;
+        h[0] = Q.enabled;
+        if (!Q.enabled) continue;
+        TileCounters tc{};
+        CK(cudaSetDevice(ctx->device));
+        CK(cudaMemcpy(&tc, Q.d_cnt.p, sizeof tc, cudaMemcpyDeviceToHost));
+        CK(cudaMemcpy(slots.data(), Q.d_slots.p, slots.size() * sizeof(KmerSlot), cudaMemcpyDeviceToHost));
+        key_of[i].assign(tc.claims, kKmerEmpty);
+        for (const KmerSlot &e : slots)
+            if (e.key != kKmerEmpty && e.count >= 1 && e.count <= tc.claims) key_of[i][e.count - 1] = e.key;
+        h[1] = Q.n_mates; h[2] = tc.overflow; h[3] = Q.longest; h[4] = Q.L.C;
+        h[5] = Q.reads[0]; h[6] = Q.reads[1]; h[7] = tc.untiled[0]; h[8] = tc.untiled[1];
+        h[9] = Q.failed || Q.batch_open;
+        all_keys.insert(all_keys.end(), key_of[i].begin(), key_of[i].end());
+    }
+    if (cm) {
+        const std::vector<uint64_t> mine(head.begin() + (size_t)rank0 * H, head.begin() + (size_t)(rank0 + 1) * H);
+        st = nccl_allgather_u64(ctx0, cm, mine, &head);
+        if (st != FQ_OK) return st;
+        st = nccl_allgather_var(ctx0, cm, std::vector<uint64_t>(all_keys), &all_keys);
+        if (st != FQ_OK) return st;
+    }
+    uint64_t enabled = 0, n_mates = 0, overflow = 0, longest = 0, cap = 0, reads[2] = {0, 0}, untiled[2] = {0, 0}, failed = 0;
+    for (uint32_t j = 0; j < n_shards; ++j) {
+        const uint64_t *h = head.data() + (size_t)j * H;
+        enabled += h[0];
+        if (h[1] && n_mates && h[1] != n_mates) return fail(ctx0, FQ_ERR_ARG, "fq_tile_qual_end_pass_all: some contexts counted paired batches, others single-end ones");
+        if (h[1]) n_mates = h[1];
+        overflow |= h[2];
+        longest = std::max(longest, h[3]);
+        cap = std::max(cap, h[4]);
+        for (int m = 0; m < 2; ++m) { reads[m] += h[5 + m]; untiled[m] += h[7 + m]; }
+        failed |= h[9];
+    }
+    if (!enabled) return fail(ctx0, FQ_ERR_STATE, "fq_tile_qual_end_pass_all: per flowcell tile quality is not enabled (fq_tile_qual_enable)");
+    if (enabled != n_shards) return fail(ctx0, FQ_ERR_ARG, "fq_tile_qual_end_pass_all: per flowcell tile quality is enabled on some contexts only");
+    if (failed) {           // no partial result: the pass is dropped and the contexts are ready for the next one
+        for (int i = 0; i < n; ++i) {
+            st = tile_qual_clear(ctxs[i]);
+            if (st != FQ_OK) return st;
+        }
+        return fail(ctx0, FQ_ERR_STATE, "fq_tile_qual_end_pass_all: a batch of this pass failed, so the pass has no result");
+    }
+    // 2. the union, ascending by (lane, tile); more than kTileMaxKeys keys: no table
+    std::sort(all_keys.begin(), all_keys.end());
+    all_keys.erase(std::unique(all_keys.begin(), all_keys.end()), all_keys.end());
+    if (all_keys.size() > kTileMaxKeys) overflow = 1;
+    if (overflow) all_keys.clear();
+    const uint32_t U = (uint32_t)all_keys.size(), cycles = (uint32_t)std::min<uint64_t>(longest, kTileMaxCycles);
+    // 3. the blocks in union order, summed
+    const uint32_t M = (uint32_t)n_mates;
+    const TileLayout S{M * U, (uint32_t)cap};
+    std::vector<uint64_t> sum(U ? S.total() : 0, 0), blk;
+    for (int i = 0; i < n && U; ++i) {
+        fq_ctx *const ctx = ctxs[i];
+        const TileLayout L = ctx->tq.L;
+        if (!ctx->tq.n_mates) continue;                   // no batch here this pass
+        if ((uint64_t)M * key_of[i].size() > L.D) return fail(ctx0, FQ_ERR_STATE, "fq_tile_qual_end_pass_all: internal: a context's block is smaller than its keys");
+        blk.resize(L.total());
+        CK(cudaSetDevice(ctx->device));
+        CK(cudaMemcpy(blk.data(), ctx->tq.d_acc.p, blk.size() * 8, cudaMemcpyDeviceToHost));
+        for (uint32_t id = 0; id < key_of[i].size(); ++id) {
+            const uint32_t u = (uint32_t)(std::lower_bound(all_keys.begin(), all_keys.end(), key_of[i][id]) - all_keys.begin());
+            for (uint32_t m = 0; m < M; ++m) {
+                const uint32_t d = M * id + m, e = M * u + m;
+                sum[S.bases(e)] += blk[L.bases(d)];
+                sum[S.qual(e)] += blk[L.qual(d)];
+                for (uint32_t b = 0; b <= L.C; ++b) sum[S.hist(b, e)] += blk[L.hist(b, d)];
+                for (uint32_t c = 0; c < L.C; ++c) sum[S.cyc(c, e)] += blk[L.cyc(c, d)];
+            }
+        }
+    }
+    if (cm && U) {
+        st = nccl_sum_u64(ctx0, cm, &sum);
+        if (st != FQ_OK) return st;
+    }
+    // 4. the result, [tile][mate] and [tile][mate][cycle]; bases at cycle c are the reads longer than c
+    std::vector<uint32_t> lane(U), tile(U);
+    std::vector<uint64_t> t_reads((size_t)U * M), t_bases((size_t)U * M), t_qsum((size_t)U * M), c_bases((size_t)U * M * cycles),
+        c_qsum((size_t)U * M * cycles);
+    for (uint32_t u = 0; u < U; ++u) {
+        lane[u] = (uint32_t)(all_keys[u] >> 32);
+        tile[u] = (uint32_t)all_keys[u];
+        for (uint32_t m = 0; m < M; ++m) {
+            const uint32_t e = M * u + m;
+            const size_t k = (size_t)u * M + m;
+            uint64_t longer = 0;
+            for (uint32_t b = S.C + 1; b-- > 0;) {
+                if (b < cycles && b < S.C) {          // cycles past every tiled read stay 0
+                    c_bases[k * cycles + b] = longer;
+                    c_qsum[k * cycles + b] = sum[S.cyc(b, e)];
+                }
+                longer += sum[S.hist(b, e)];
+            }
+            t_reads[k] = longer;
+            t_bases[k] = sum[S.bases(e)];
+            t_qsum[k] = sum[S.qual(e)];
+        }
+    }
+    for (int i = 0; i < n; ++i) {
+        fq_ctx::TileQual &Q = ctxs[i]->tq;
+        Q.res_mates = M;
+        Q.res_overflow = (uint32_t)overflow;
+        Q.res_cycles = cycles;
+        for (int m = 0; m < 2; ++m) { Q.res_reads[m] = reads[m]; Q.res_untiled[m] = untiled[m]; }
+        Q.lane = lane; Q.tile = tile;
+        Q.t_reads = t_reads; Q.t_bases = t_bases; Q.t_qsum = t_qsum; Q.c_bases = c_bases; Q.c_qsum = c_qsum;
+        st = tile_qual_clear(ctxs[i]);
+        if (st != FQ_OK) return st;
+    }
+    return FQ_OK;
+}
+
 }  // namespace
 
 fq_status fq_kmer_end_pass_all(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
@@ -2515,6 +2769,45 @@ fq_status fq_overrep_results(fq_ctx *ctx, fq_overrep_view *view)
     view->n_seqs = R.seqs.size();
     view->seqs = R.seqs.data();
     view->bytes = R.bytes.data();
+    return FQ_OK;
+}
+
+fq_status fq_tile_qual_enable(fq_ctx *ctx)
+{
+    if (!ctx) return FQ_ERR_ARG;
+    fq_ctx::TileQual &Q = ctx->tq;
+    if (Q.enabled) return Q.reads[0] || Q.reads[1] ? fail(ctx, FQ_ERR_STATE, "fq_tile_qual_enable: a pass is under way") : FQ_OK;
+    CK(cudaSetDevice(ctx->device));
+    CK(Q.d_slots.ensure((size_t)kTileSlots * sizeof(KmerSlot)));
+    CK(Q.d_cnt.ensure(sizeof(TileCounters)));
+    CK(Q.h_cnt.ensure(8));
+    const fq_status st = tile_qual_clear(ctx);
+    if (st == FQ_OK) Q.enabled = true;
+    return st;
+}
+
+fq_status fq_tile_qual_end_pass_all(fq_ctx *const *ctxs, int n, fq_comm *const *comm)
+{
+    return end_pass_entry(ctxs, n, comm, "fq_tile_qual_end_pass_all", tile_qual_end_pass_impl);
+}
+
+fq_status fq_tile_qual_results(fq_ctx *ctx, fq_tile_qual_view *view)
+{
+    if (!ctx || !view) return FQ_ERR_ARG;
+    const fq_ctx::TileQual &Q = ctx->tq;
+    if (!Q.enabled) return fail(ctx, FQ_ERR_STATE, "fq_tile_qual_results: per flowcell tile quality is not enabled (fq_tile_qual_enable)");
+    view->n_mates = Q.res_mates;
+    view->overflow = Q.res_overflow;
+    view->n_tiles = (uint32_t)Q.lane.size();
+    view->cycles = Q.res_cycles;
+    for (int m = 0; m < 2; ++m) { view->reads[m] = Q.res_reads[m]; view->untiled[m] = Q.res_untiled[m]; }
+    view->lane = Q.lane.data();
+    view->tile = Q.tile.data();
+    view->tile_reads = Q.t_reads.data();
+    view->tile_bases = Q.t_bases.data();
+    view->tile_qsum = Q.t_qsum.data();
+    view->cycle_bases = Q.c_bases.data();
+    view->cycle_qsum = Q.c_qsum.data();
     return FQ_OK;
 }
 

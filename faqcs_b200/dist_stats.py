@@ -1,13 +1,14 @@
 """Multi-GPU merge of the statistics through the library's own collective (fq_allreduce_stats: one
 ncclAllReduce(u64, sum) over NVLink + a max of the row counters; include/faqcs_b200.h), and the end of a k-mer
 rarefaction, sequence duplication or overrepresented-sequence pass over a table sharded across contexts (fq_kmer_end_pass_all,
-fq_dup_end_pass_all, fq_overrep_end_pass_all), and of an insert-size pass (fq_overlap_end_pass_all).
+fq_dup_end_pass_all, fq_overrep_end_pass_all), and of an insert-size or per flowcell tile quality pass (fq_overlap_end_pass_all,
+fq_tile_qual_end_pass_all).
 
 Two launch shapes, both ending in the same C call:
   * one process per GPU (torchrun): rank 0 draws the NCCL id (fq_comm_unique_id), the launcher's process group
     broadcasts those 128 bytes, every rank joins (fq_comm_init_rank) and calls the library on its one context;
   * one process, several GPUs: fq_comm_init_all over the contexts (statistics) or no communicator at all (k-mer,
-    duplication, insert-size and overrepresented-sequence passes), one call for all of them.
+    duplication, insert-size, overrepresented-sequence and tile quality passes), one call for all of them.
 The reference's counterpart is the `omp critical` merge at the end of trim() (trim.cpp:120-154).
 """
 from __future__ import annotations
@@ -145,5 +146,25 @@ def overrep_end_pass_ranks(eng: Engine, dist, dev):
         ctxs = (C.c_void_p * 1)(eng.ctx)
         comms = (C.c_void_p * 1)(comm)
         _check(eng, eng.lib.fq_overrep_end_pass_all(ctxs, 1, comms))
+    finally:
+        eng.lib.fq_comm_destroy(comm)
+
+
+def tile_qual_end_pass_local(engines: Sequence[Engine]):
+    """End of a per flowcell tile quality pass whose batches ran on these contexts (one process, any devices, a device may
+    repeat): the key lists are united and the counts summed, and every engine's tile_qual_results() returns the whole pass."""
+    n = len(engines)
+    e0 = engines[0]
+    ctxs = (C.c_void_p * n)(*[e.ctx for e in engines])
+    _check(e0, e0.lib.fq_tile_qual_end_pass_all(ctxs, n, None))
+
+
+def tile_qual_end_pass_ranks(eng: Engine, dist, dev):
+    """The same with one context per process: keys and counts are merged over the ranks of `dist` (torch.distributed)."""
+    comm = _rank_comm(eng, dist, dev)
+    try:
+        ctxs = (C.c_void_p * 1)(eng.ctx)
+        comms = (C.c_void_p * 1)(comm)
+        _check(eng, eng.lib.fq_tile_qual_end_pass_all(ctxs, 1, comms))
     finally:
         eng.lib.fq_comm_destroy(comm)

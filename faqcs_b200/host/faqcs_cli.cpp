@@ -80,6 +80,7 @@ struct Cli {
     long long overrep_len = 50, overrep_ppm = 1000;    // checked after parsing
     bool overrep_bad_number = false;
     vector<pair<string, string>> artifacts;            // --artifactFile entries (also in `adapter`)
+    bool tile_quality = false;      // per flowcell tile quality of each input pass -> prefix.tile_quality.txt
     bool keep_unpaired = false;     // the -u pass appends to prefix.unpaired.trimmed.fastq instead of truncating it (the reference's Q11 quirk, fixed)
     vector<int> devices;            // --devices 0,1,...: consecutive batches go to consecutive GPUs, one NCCL all-reduce at the end
     bool has_paired() const { return !input_read1_file.empty(); }       // has_paired() tests read1 twice, FaQCs.h:135-138
@@ -175,7 +176,9 @@ static void usage()
             "\t--overrep\t\t<bool> list the sequences (read prefixes, each mate on its own) above a share of the reads of each\n"
             "\t\t\t\tinput, with the built-in adapter, PhiX or --artifactFile entry they match: prefix.overrepresented.txt\n"
             "\t--overrep_len\t\t<INT> bases of each read's prefix compared (default 50, 1-256)\n"
-            "\t--overrep_ppm\t\t<INT> smallest listed share, in reads per million of the mate (default 1000 = 0.1 %, 10-1000000)\n";
+            "\t--overrep_ppm\t\t<INT> smallest listed share, in reads per million of the mate (default 1000 = 0.1 %, 10-1000000)\n"
+            "\t--tile_quality\t\t<bool> mean quality per cycle of each flowcell tile (lane and tile from the read names) against\n"
+            "\t\t\t\tall tiles, each mate on its own, for each input: prefix.tile_quality.txt\n";
 }
 
 static void parse_options(int argc, char *argv[], Cli &o)
@@ -203,7 +206,7 @@ static void parse_options(int argc, char *argv[], Cli &o)
         {"R2", true, &config_opt, 27}, {"replace_to_N_q", true, &config_opt, 31}, {"device", true, &config_opt, 40}, {"batch_mb", true, &config_opt, 41}, {"devices", true, &config_opt, 42}, {"gz_out", false, &config_opt, 43}, {"keep_unpaired", false, &config_opt, 44}, {"dup_stats", false, &config_opt, 45},
         {"insert_size", false, &config_opt, 46}, {"insert_min_overlap", true, &config_opt, 47}, {"insert_diff_limit", true, &config_opt, 48},
         {"insert_diff_pct", true, &config_opt, 49}, {"overrep", false, &config_opt, 50}, {"overrep_len", true, &config_opt, 51},
-        {"overrep_ppm", true, &config_opt, 52},
+        {"overrep_ppm", true, &config_opt, 52}, {"tile_quality", false, &config_opt, 53},
         {0, 0, 0, 0}};
     int opt_code;
     opterr = 0;
@@ -280,6 +283,7 @@ static void parse_options(int argc, char *argv[], Cli &o)
                         break;
                     }
                     case 50: o.overrep = true; break;
+                    case 53: o.tile_quality = true; break;
                     case 51: case 52: {
                         char *end = nullptr;
                         errno = 0;
@@ -818,6 +822,7 @@ struct Run {
             if (o.dup_stats) check(fq_dup_enable(c), c);
             if (o.insert_size) check(fq_overlap_enable(c, (uint32_t)o.insert_min_overlap, (uint32_t)o.insert_diff_limit, (uint32_t)o.insert_diff_pct), c);
             if (o.overrep) check(fq_overrep_enable(c, (uint32_t)o.overrep_len, (uint32_t)o.overrep_ppm), c);
+            if (o.tile_quality) check(fq_tile_qual_enable(c), c);
         }
     }
     // end of an input's pass: the contexts' k-mer tables merge into the run's curve and histogram (FaQCs.cpp:518-537, 737-756)
@@ -873,6 +878,65 @@ struct Run {
             snprintf(pct, sizeof pct, "%.4f", 100.0 * (double)q.count / (double)v.reads[q.mate - 1]);
             overrep_report += to_string(q.mate) + "\t" + to_string(q.count) + "\t" + pct + "\t" + seq + "\t" + overrep_source(seq) + "\n";
         }
+    }
+    // --tile_quality: the contexts' tile tables united after each input pass, one block of prefix.tile_quality.txt.  Means
+    // and deltas are double arithmetic on the exact sums, printed %.2f; NA where there is no base.
+    string tile_report;
+    static string fixed2(double x)
+    {
+        char b[64];
+        snprintf(b, sizeof b, "%.2f", x);
+        return b;
+    }
+    void tile_qual_end_pass(bool paired)
+    {
+        if (!o.tile_quality) return;
+        check(fq_tile_qual_end_pass_all(ctxs.data(), (int)ctxs.size(), nullptr));
+        fq_tile_qual_view v;
+        check(fq_tile_qual_results(ctx, &v));
+        const uint32_t M = paired ? 2 : 1, C = v.cycles, T = v.n_tiles;
+        tile_report += string("pass\t") + (paired ? "paired" : "unpaired") + "\ttiles\t" + to_string(T) + "\tcycles\t" + to_string(C) +
+                       "\toverflow\t" + to_string(v.overflow) + "\n";
+        tile_report += "#mate\treads\ttiled\tuntiled\n";
+        for (uint32_t m = 0; m < M; ++m)
+            tile_report += to_string(m + 1) + "\t" + to_string(v.reads[m]) + "\t" + to_string(v.reads[m] - v.untiled[m]) + "\t" + to_string(v.untiled[m]) + "\n";
+        if (v.overflow) return;
+        // v.n_mates is 0 for a pass without batches: every row then has no reads
+        auto at = [&](const uint64_t *a, uint32_t t, uint32_t m, uint32_t c) { return m < v.n_mates ? a[((size_t)t * v.n_mates + m) * C + c] : 0ull; };
+        auto tot = [&](const uint64_t *a, uint32_t t, uint32_t m) { return m < v.n_mates ? a[(size_t)t * v.n_mates + m] : 0ull; };
+        vector<double> all((size_t)M * C, 0.0);
+        vector<bool> has((size_t)M * C, false);
+        tile_report += "#mate\tmean_by_cycle\n";
+        for (uint32_t m = 0; m < M; ++m) {
+            tile_report += to_string(m + 1);
+            for (uint32_t c = 0; c < C; ++c) {
+                uint64_t b = 0, q = 0;
+                for (uint32_t t = 0; t < T; ++t) { b += at(v.cycle_bases, t, m, c); q += at(v.cycle_qsum, t, m, c); }
+                has[(size_t)m * C + c] = b != 0;
+                if (b) all[(size_t)m * C + c] = (double)q / (double)b;
+                tile_report += "\t" + (b ? fixed2(all[(size_t)m * C + c]) : string("NA"));
+            }
+            tile_report += "\n";
+        }
+        tile_report += "#lane\ttile\tmate\treads\tbases\tmean\tworst_cycle\tworst_delta\tdelta_by_cycle\n";
+        for (uint32_t t = 0; t < T; ++t)
+            for (uint32_t m = 0; m < M; ++m) {
+                const uint64_t bases = tot(v.tile_bases, t, m);
+                string row = to_string(v.lane[t]) + "\t" + to_string(v.tile[t]) + "\t" + to_string(m + 1) + "\t" + to_string(tot(v.tile_reads, t, m)) + "\t" +
+                             to_string(bases) + "\t" + (bases ? fixed2((double)tot(v.tile_qsum, t, m) / (double)bases) : string("NA"));
+                string deltas;
+                uint32_t worst = C;
+                double worst_d = 0.0;
+                for (uint32_t c = 0; c < C; ++c) {
+                    const uint64_t b = at(v.cycle_bases, t, m, c);
+                    if (!b) { deltas += "\tNA"; continue; }
+                    const double d = (double)at(v.cycle_qsum, t, m, c) / (double)b - all[(size_t)m * C + c];
+                    if (worst == C || d < worst_d) { worst = c; worst_d = d; }
+                    deltas += "\t" + fixed2(d);
+                }
+                row += worst < C ? "\t" + to_string(worst + 1) + "\t" + fixed2(worst_d) : string("\tNA\tNA");
+                tile_report += row + deltas + "\n";
+            }
     }
     // The first of the nine built-in adapters, PhiX174 and the --artifactFile entries (in that order) that holds some 20-base
     // window of the upper-cased sequence (the whole sequence if it is shorter), on either strand; "No Hit" otherwise.
@@ -1458,6 +1522,7 @@ int main(int argc, char *argv[])
         if (o.insert_size && fq_overlap_enable(ctx, (uint32_t)o.insert_min_overlap, (uint32_t)o.insert_diff_limit, (uint32_t)o.insert_diff_pct) != FQ_OK)
             throw string(fq_last_error(ctx));
         if (o.overrep && fq_overrep_enable(ctx, (uint32_t)o.overrep_len, (uint32_t)o.overrep_ppm) != FQ_OK) throw string(fq_last_error(ctx));
+        if (o.tile_quality && fq_tile_qual_enable(ctx) != FQ_OK) throw string(fq_last_error(ctx));
         const double t_created = now_s();
         Run R(o);
         R.ctx = ctx;
@@ -1472,6 +1537,7 @@ int main(int argc, char *argv[])
             R.dup_end_pass(true);
             R.overlap_end_pass();
             R.overrep_end_pass(true);
+            R.tile_qual_end_pass(true);
         }
         if (o.has_unpaired()) {
             R.first_batch = true;      // offset detection only if still unknown; the NextSeq check runs per input (FaQCs.cpp:586,673-683)
@@ -1479,6 +1545,7 @@ int main(int argc, char *argv[])
             R.kmer_end_pass();                     // FaQCs.cpp:737-756
             R.dup_end_pass(false);
             R.overrep_end_pass(false);
+            R.tile_qual_end_pass(false);
         }
         const double t_processed = now_s();
         if (R.ctxs.size() > 1) {
@@ -1523,6 +1590,13 @@ int main(int argc, char *argv[])
             fout << R.overrep_report;
             fout.close();
             if (!fout) throw string("Unable to write the overrepresented sequences file: ") + fn;
+        }
+        if (o.tile_quality) {
+            const string fn = o.output_dir + "/" + o.prefix + ".tile_quality.txt";
+            ofstream fout(fn.c_str());
+            fout << R.tile_report;
+            fout.close();
+            if (!fout) throw string("Unable to write the tile quality file: ") + fn;
         }
         if (!o.trim_only && o.debug) {                           // the reference deletes these unless --debug (plot.cpp:517-537)
             write_debug_files(v, o);

@@ -314,6 +314,57 @@ def overrepresented(n_pairs: int, plants=None, seed: int = 93, start: int = 0, p
     return Workload("overrepresented", mates[0], mates[1] if paired else None, [])
 
 
+def _digits(v: np.ndarray, k: int) -> np.ndarray:
+    out = np.empty((v.size, k), dtype=np.uint8)
+    for d in range(k):
+        out[:, k - 1 - d] = 48 + (v // (10 ** d)) % 10
+    return out
+
+
+def tile_numbers(tiles_per_lane: int) -> List[int]:
+    """Flowcell tile numbers in the NovaSeq style: 1101, 1102, ..., 64 tiles per swath, then the next swath (1201, ...)."""
+    return [1101 + 100 * (k // 64) + k % 64 for k in range(tiles_per_lane)]
+
+
+def tiled(n_pairs: int, lanes: int = 2, tiles_per_lane: int = 16, order: str = "sorted", bad_tiles=None, seed: int = 95,
+          paired: bool = True, L: int = 150) -> Workload:
+    """C2-like reads under Casava 1.8 names '@B200SIM:1:FC:{lane}:{tile}:{x}:{y} {mate}:N:0:ACGT', the workload of
+    --tile_quality.  The pairs are spread evenly over lanes x tiles_per_lane flowcell tiles (tile_numbers(), zero-padded to
+    one width when they need more than 4 digits; lanes <= 9), in (lane, tile) order as a sequencer writes them
+    (order="sorted") or in random order ("shuffled").  bad_tiles = [(lane, tile, first_cycle, last_cycle, drop)]: the
+    scores of cycles first..last (1-based, inclusive) of both mates of that tile's reads drop by `drop` (at least 2 stays).
+    Default: one bubble on lane 1's second tile, cycles 50-80, 15 lower."""
+    assert 1 <= lanes <= 9 and tiles_per_lane >= 1 and order in ("sorted", "shuffled")
+    tnum = np.array(tile_numbers(tiles_per_lane), dtype=np.int64)
+    if bad_tiles is None:
+        bad_tiles = [(1, int(tnum[1]), 50, 80, 15)] if tiles_per_lane > 1 else []
+    rng = np.random.default_rng(seed)
+    n_keys = lanes * tiles_per_lane
+    key = np.arange(n_pairs, dtype=np.int64) * n_keys // max(n_pairs, 1)
+    if order == "shuffled":
+        key = key[rng.permutation(n_pairs)]
+    lane = 1 + key // tiles_per_lane
+    tile = tnum[key % tiles_per_lane]
+    x = rng.integers(10000, 100000, size=n_pairs)
+    y = rng.integers(10000, 100000, size=n_pairs)
+    tw = max(4, len(str(int(tnum.max()))))
+    mates = []
+    for mate in (1, 2) if paired else (1,):
+        q = _qualities(rng, n_pairs, L, 30, 40, 0.12, 3.0, 2, 41, 0.10, 59).astype(np.int16)
+        for bl, bt, c0, c1, drop in bad_tiles:
+            rows = np.flatnonzero((lane == bl) & (tile == bt))
+            q[rows[:, None], np.arange(c0 - 1, min(c1, L))[None, :]] -= drop
+        q = np.clip(q, 2, 41).astype(np.uint8)
+        s = _bases(rng, n_pairs, L, 0.002, 0.01)
+        head = np.frombuffer(b"@B200SIM:1:FC:", dtype=np.uint8)
+        tail = np.frombuffer(f" {mate}:N:0:ACGT".encode(), dtype=np.uint8)
+        colon = np.full((n_pairs, 1), ord(":"), dtype=np.uint8)
+        hdr = np.concatenate([np.broadcast_to(head, (n_pairs, head.size)), _digits(lane, 1), colon, _digits(tile, tw), colon,
+                              _digits(x, 5), colon, _digits(y, 5), np.broadcast_to(tail, (n_pairs, tail.size))], 1)
+        mates.append(_assemble(np.ascontiguousarray(hdr), s, q + 33))
+    return Workload("tiled", mates[0], mates[1] if paired else None, [])
+
+
 def fastq_bytes(records: List[Tuple[str, str, str]], eol: str = "\n") -> bytes:
     """Hand-written records -> FASTQ bytes (micro-cases)."""
     return "".join(f"{h}{eol}{s}{eol}+{eol}{q}{eol}" for h, s, q in records).encode()

@@ -475,6 +475,53 @@ fq_status fq_overrep_enable(fq_ctx *ctx, uint32_t prefix_len, uint32_t min_ppm);
 fq_status fq_overrep_end_pass_all(fq_ctx *const *ctx, int n, fq_comm *const *comm);
 fq_status fq_overrep_results(fq_ctx *ctx, fq_overrep_view *view);
 
+/*
+ * Per flowcell tile sequence quality (not part of FaQCs; the per-tile plot FastQC draws, used to find bubbles, a bad swath or
+ * a smeared tile).  Every framed record counts, whatever trimming, filtering or --qc_only do later; the mates of a pair count
+ * separately (mate 1, 2; a single-end pass has mate 1 only).
+ * A read's (lane, tile): its name is the header-line bytes after '@' up to the first ' ', '\t', '\r' or '\n', split at ':'
+ * into n fields f[0..n-1].  n >= 7 (Casava 1.8 / bcl-convert, with or without a UMI field): lane = f[3], tile = f[4]; n = 5
+ * or 6 (@inst:lane:tile:x:y#idx/1): lane = f[1], tile = f[2]; otherwise, or when lane or tile is not 1 to 9 ASCII digits, the
+ * read is untiled.  Lane and tile compare as values (01101 and 1101 are one tile).  No parity with FastQC is claimed: it
+ * splits the whole line rather than the name and ignores the lane.
+ * A base's score is max(0, byte - input_quality_offset) on the quality line as framed, before terminal-N masking, with no
+ * upper clamp.  A score above 41 fails the batch with FQ_ERR_QUALITY, with or without qc_only, unless the base lies in a
+ * leading or trailing run of 'N' (which the masking covers); such a base counts here with its score as read.
+ * Per (tile, mate): reads, bases and score sum of whole reads, and at each cycle 1..cycles the bases (the reads at least
+ * that long) and their score sum; cycles = min(longest read of the pass, 1024), and bases past cycle 1024 count in
+ * the whole-read totals only.  Per mate: reads and untiled reads of the pass.
+ * At most 16384 distinct (lane, tile) keys per pass: when the union of the keys of all contexts is larger, overflow = 1 and
+ * the pass reports reads[] and untiled[] but no table (n_tiles = 0), however the batches were dealt to the contexts.
+ *   fq_tile_qual_enable        before the first batch of a pass (FQ_ERR_STATE in the middle of one).  Afterwards every batch
+ *                              path counts.  Nothing is allocated and no kernel runs without it.  Memory: a 512 KiB key table,
+ *                              2 bytes per read and mate of the largest batch, and 8 x mates x (3 + 2 x cycle capacity)
+ *                              bytes per tile (tiles seen rounded up to a power of two, at least 64 / mates; cycle capacity:
+ *                              the longest read rounded up to 32, at most 1024): 537 MB at the extreme of 16 384 tiles,
+ *                              2 mates and 1024 cycles, a few MB for a real flowcell.  The end of a pass holds the summed
+ *                              counts on the host and hands every context its own copy of the result.
+ *   fq_tile_qual_end_pass_all  after the last batch of an input: unites the keys of n contexts (n == 1 and comm == NULL for
+ *                              one context; otherwise as for fq_kmer_end_pass_all), sums their counts, publishes the pass on
+ *                              every context and clears the tables.  FQ_ERR_ARG when the profile is enabled on some contexts
+ *                              only, or when some counted paired batches and others single-end ones (a batch of the other
+ *                              kind in a pass is refused with FQ_ERR_ARG too).  FQ_ERR_STATE when a batch of the pass
+ *                              failed part-way (its error was returned by the batch call): the pass is dropped, the
+ *                              contexts are cleared for the next one, and the results stay those of the last finished pass.
+ *   fq_tile_qual_results       the last finished pass; the pointers belong to the context and stay valid until its next
+ *                              fq_tile_qual_* call.  FQ_ERR_STATE (also for an end of pass) on a context that never enabled it.
+ */
+typedef struct fq_tile_qual_view {
+    uint32_t n_mates;                  /* 2 paired, 1 single-end, 0 no batch in the pass */
+    uint32_t overflow;                 /* 1: more than 16384 keys, no table */
+    uint32_t n_tiles, cycles;
+    uint64_t reads[2], untiled[2];     /* per mate */
+    const uint32_t *lane, *tile;       /* [n_tiles], ascending by (lane, tile) */
+    const uint64_t *tile_reads, *tile_bases, *tile_qsum;        /* [n_tiles][n_mates] */
+    const uint64_t *cycle_bases, *cycle_qsum;                   /* [n_tiles][n_mates][cycles] */
+} fq_tile_qual_view;
+fq_status fq_tile_qual_enable(fq_ctx *ctx);
+fq_status fq_tile_qual_end_pass_all(fq_ctx *const *ctx, int n, fq_comm *const *comm);
+fq_status fq_tile_qual_results(fq_ctx *ctx, fq_tile_qual_view *view);
+
 /* Zero the accumulators (new run on the same context). */
 fq_status fq_reset_stats(fq_ctx *ctx);
 
